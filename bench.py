@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the keypoint-voting hot path (BASELINE.json metric: keypoint-voting frames/s).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (ransac_voting_layer_all_masks: mask compaction -> hypothesis
 generation -> inlier scoring -> refinement) over one batch of synthetic LM-O-shaped frames.
@@ -62,7 +62,15 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="ransac", choices=["ransac", "ls", "pose"],
                     help="ransac: BASELINE config 2 (the headline); ls: CoordLSVotingWeighted on config-1-shaped tensors")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the keypoints of the last timed step as DIR/keypoints.npy (float32 [b,oc,9,2]; all ranks' "
+                         "frames with --gpus > 1), so that two builds can be compared on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "ransac" or args.impl != "ours"):
+        ap.error("--dump-outputs writes the keypoints of the voting workload (--workload ransac --impl ours)")
+    return args
 
 
 class ClockSampler(threading.Thread):
@@ -487,6 +495,11 @@ def main():
                     units=st[0], exact_units=st[1], last=last, clocks=clk)
 
     main_pass = timed_pass(lanes if lanes >= 2 else 1, 0 if lanes >= 2 else 1, True)
+    if args.dump_outputs and rank == 0:
+        # written now: the k_score pass below reuses the result buffers
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "keypoints.npy"), main_pass["last"].cpu().numpy())
+
     def kernel_pass():
         smp = ClockSampler(local)
         smp.start()
@@ -536,7 +549,7 @@ def main():
     # --- end to end through the host-buffer C-ABI entry point (pinned host buffers)
     e2e = None
     if not args.no_e2e:
-        e2e_steps = max(3, min(args.steps, int(2.0e10 / max(in_bytes, 1))))  # about 20 GB over PCIe at most
+        e2e_steps = max(1, min(args.steps, int(2.0e10 / max(in_bytes, 1))))  # about 20 GB over PCIe at most
         outs_h = [torch.empty((B, oc, vn, 2), dtype=torch.float32).pin_memory() for _ in range(args.host_calls + 1)]
 
         def e2e_pass(in_flight):

@@ -5,14 +5,15 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 
 
-def _run(args, timeout=300):
+def _run(args, timeout=300, env=None):
     return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True,
-                          timeout=timeout, cwd=ROOT)
+                          timeout=timeout, cwd=ROOT, env=env)
 
 
 def test_reference_arm_prints_the_contract_line():
@@ -29,10 +30,29 @@ def test_reference_arm_prints_the_contract_line():
 
 
 def test_product_arm_needs_a_gpu():
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    res = _run(["--steps", "1", "--warmup", "1", "--no-cpu-baseline", "--no-e2e"], timeout=120)
+    # the benchmark runs with every device hidden, so that this holds on a machine with GPUs too
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    res = _run(["--steps", "1", "--warmup", "1", "--no-cpu-baseline", "--no-e2e"], timeout=120, env=env)
     assert res.returncode != 0  # no CPU or PyTorch fallback of the product path
     assert not any(ln.startswith("{") for ln in res.stdout.splitlines())
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_are_the_keypoints_of_the_last_timed_step(cuda_lib, tmp_path):
+    """--dump-outputs writes what the timed path computed in its last step: the same call, made directly on the same
+    seeded frames, gives those keypoints bit for bit."""
+    import torch
+
+    from casapose_b200 import synthetic
+    from casapose_b200.pose_estimation import ransac_voting_layer_all_masks
+
+    steps = 3
+    res = _run(["--steps", str(steps), "--warmup", "1", "--no-cpu-baseline", "--no-e2e", "--dump-outputs", str(tmp_path)])
+    assert res.returncode == 0, res.stderr[-2000:]
+    assert json.loads(res.stdout.strip().splitlines()[-1])["steps"] == steps
+    got = np.load(tmp_path / "keypoints.npy")
+    d = synthetic.make_frames(16, 480, 640, synthetic.CONFIG_8_IDS, seed=synthetic.SEED_BASE)
+    want = ransac_voting_layer_all_masks(torch.from_numpy(d["mask"]).cuda(), torch.from_numpy(d["vertex"]).cuda(), 512,
+                                         seed=1000 + steps - 1).cpu().numpy()
+    assert got.dtype == np.float32 and got.shape == (16, 8, 9, 2)
+    assert np.array_equal(got, want, equal_nan=True)

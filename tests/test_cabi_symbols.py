@@ -43,20 +43,39 @@ def test_version_and_error_without_gpu(cuda_lib):
     assert b"oc=40" in cuda_lib.casa_last_error()
 
 
+NO_DEVICE_SCRIPT = r'''
+import sys
+sys.path.insert(0, %(root)r)
+import torch
+from casapose_b200 import _lib
+from casapose_b200.pose_estimation import ransac_voting_layer_all_masks
+
+assert not torch.cuda.is_available()
+try:
+    _lib.handle(0)
+    raise SystemExit("a handle was created without a device")
+except _lib.CasaError:
+    pass
+try:
+    ransac_voting_layer_all_masks(torch.zeros(1, 8, 8, 2), torch.zeros(1, 8, 8, 9, 2), 16)
+    raise SystemExit("host tensors were accepted by the device entry point")
+except ValueError:
+    pass
+print("no fallback ok")
+'''
+
+
 def test_product_path_fails_loudly_without_cuda(cuda_lib):
-    """No CPU fallback: without a device the handle cannot be created and the Python layer raises."""
-    import torch
+    """No CPU fallback: without a device the handle cannot be created and the Python layer raises.  Runs in a
+    subprocess that sees no device, so that it checks the same on a machine with GPUs."""
+    import subprocess
+    import sys
 
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    from casapose_b200 import _lib
-
-    with pytest.raises(_lib.CasaError):
-        _lib.handle(0)
-    from casapose_b200.pose_estimation import ransac_voting_layer_all_masks
-
-    with pytest.raises(ValueError):
-        ransac_voting_layer_all_masks(torch.zeros(1, 8, 8, 2), torch.zeros(1, 8, 8, 9, 2), 16)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    res = subprocess.run([sys.executable, "-c", NO_DEVICE_SCRIPT % {"root": ROOT}], capture_output=True, text=True,
+                         timeout=300, env=env)
+    assert res.returncode == 0, res.stdout + res.stderr
+    assert "no fallback ok" in res.stdout
 
 
 def test_pipelined_host_entry_rejects_bad_arguments_without_gpu(cuda_lib):
