@@ -245,6 +245,7 @@ struct casa_handle {
   unsigned long long* pinned_stats = nullptr;  // 4 words, page-locked
   int score_occ = 0, score_occ_narrow = 0;  // resident k_score blocks per SM (8 / 4 hypotheses per lane)
   int fused_occ = 0;              // resident k_ls_fused blocks per SM (persistent grid of the LS forward call)
+  int classify_static_smem[2] = {-1, -1};  // static shared memory of k_ls_classify<9> / <0> (queried once)
   int use_graph = 1;
   // keypoint all-gather (NCCL, resolved with dlopen: the library itself does not link against it)
   void* comm = nullptr;           // ncclComm_t
@@ -1756,7 +1757,15 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
   {
     const size_t sm = (size_t)kCountTile * ld.nc * 4;
     const void* classify = ld.nc == 9 ? (const void*)k_ls_classify<9> : (const void*)k_ls_classify<0>;
-    if (sm > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(classify, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    // Without the opt-in, static plus dynamic shared memory of a block may not exceed 48 KB: the kernel's own counters
+    // (scnt) count too, so nc = 12 (exactly 48 KB of staged logits) needs the attribute as well.
+    int& static_sm = h->classify_static_smem[ld.nc == 9 ? 0 : 1];
+    if (static_sm < 0) {
+      cudaFuncAttributes fa;
+      CUDA_TRY(cudaFuncGetAttributes(&fa, classify));
+      static_sm = (int)fa.sharedSizeBytes;
+    }
+    if (sm + (size_t)static_sm > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(classify, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
     steps.push_back(kstep(classify, dim3(d.nct, d.b), 256, sm).arg(seg).arg(ws).arg(d).arg(lw).arg(ld).arg((int)(runs_cc ? 1 : 0)));
   }
   steps.push_back(kstep((const void*)k_place<0>, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg((const float*)nullptr).arg(ws).arg(d).arg((int)0));
@@ -1780,11 +1789,13 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
     steps.push_back(kstep((const void*)k_ls_reduce, dim3(grid_x, d.vn), 256).arg(ws).arg(d).arg(lw).arg(ld));
   } else {
     if (h->fused_occ == 0) {
-      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->fused_occ, k_ls_fused, 32 * d.vn, 0));
+      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->fused_occ, k_ls_fused<true>, 32 * d.vn, 0));
       if (h->fused_occ < 1) h->fused_occ = 1;
     }
     const int fused_gx = d.max_rtiles < h->sm_count * h->fused_occ ? d.max_rtiles : h->sm_count * h->fused_occ;
-    steps.push_back(kstep((const void*)k_ls_fused, fused_gx, 32 * d.vn).arg(ws).arg(d).arg(lw).arg(ld).arg(seg).arg(direct).arg(conf)
+    // float2 loads of a pixel's (dy, dx) need an 8-byte aligned `direct`; callers may pass any 4-byte aligned buffer
+    const void* fused = (((uintptr_t)direct) & 7) == 0 ? (const void*)k_ls_fused<true> : (const void*)k_ls_fused<false>;
+    steps.push_back(kstep(fused, fused_gx, 32 * d.vn).arg(ws).arg(d).arg(lw).arg(ld).arg(seg).arg(direct).arg(conf)
                         .arg((int)(runs_cc ? 1 : 0)).joins());
   }
   if (!out_points) out_points = (float*)(base + off_tmp_out);
@@ -1794,7 +1805,8 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
     CUDA_TRY(cudaMemsetAsync(grad->grad_direct, 0, npx * 2 * d.vn * sizeof(float), st));
     CUDA_TRY(cudaMemsetAsync(grad->grad_conf, 0, npx * d.vn * sizeof(float), st));
     steps.push_back(kstep((const void*)k_ls_adjoint, d.J, 32).arg(ws).arg(d).arg(ld).arg(grad->grad_points).arg(adj));
-    steps.push_back(kstep((const void*)k_ls_backward, grid_x, 256).arg(ws).arg(d).arg(lw).arg(ld).arg(adj).arg(grad->grad_direct).arg(grad->grad_conf));
+    const void* bwd = (((uintptr_t)grad->grad_direct) & 7) == 0 ? (const void*)k_ls_backward<true> : (const void*)k_ls_backward<false>;
+    steps.push_back(kstep(bwd, grid_x, 256).arg(ws).arg(d).arg(lw).arg(ld).arg(adj).arg(grad->grad_direct).arg(grad->grad_conf));
   }
   for (const Step& s2 : steps) launches += s2.kind == STEP_KERNEL;
   rc = (h->use_graph && !debug) ? run_graph(h, steps, ws, st) : run_direct(h, steps, ws, st);

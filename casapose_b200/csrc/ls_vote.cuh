@@ -685,7 +685,10 @@ __global__ void __launch_bounds__(256) k_ls_reduce(WS ws, Dims d, LsWS lw, LsDim
 //                          go through the reference's float32 element-wise sequence (:89-108) into float64 sums.
 // Replaces k_gather_dirs + k_ls_weights + k_ls_reduce (102 us of launches and 140 MB of intermediates per 16 frames)
 // for the forward call; the backward pass still uses the gathered arrays.
+// VEC (chosen on the host from the pointer): `direct` is 8-byte aligned and a pixel's (dy, dx) is one float2 load;
+// otherwise (e.g. a view 4 bytes into an allocation) two scalar loads of the same floats.
 constexpr int kFusedTile = 512;  // list entries per tile of k_ls_fused (d.rtile of the forward call)
+template <bool VEC>
 __global__ void __launch_bounds__(512, 2) k_ls_fused(WS ws, Dims d, LsWS lw, LsDims ld, const float* __restrict__ seg,
                                                   const float* __restrict__ direct, const float* __restrict__ conf,
                                                   int use_keep) {
@@ -746,7 +749,12 @@ __global__ void __launch_bounds__(512, 2) k_ls_fused(WS ws, Dims d, LsWS lw, LsD
         bc[j] = 0.f;
         if (bw[j] != 0.f) {
           const size_t p = (size_t)img * ld.hw + (size_t)(bp[j] >> 16) * ld.w + (bp[j] & 0xFFFFu);
-          bd[j] = __ldg(reinterpret_cast<const float2*>(direct + p * (size_t)(2 * d.vn)) + v);  // (n0, n1) = (dy, dx)
+          if (VEC) {
+            bd[j] = __ldg(reinterpret_cast<const float2*>(direct + p * (size_t)(2 * d.vn)) + v);  // (n0, n1) = (dy, dx)
+          } else {
+            const float* dp = direct + p * (size_t)(2 * d.vn) + 2 * v;
+            bd[j] = make_float2(__ldg(dp), __ldg(dp + 1));
+          }
           bc[j] = __ldg(conf + p * (size_t)d.vn + v);
         }
       }
@@ -849,7 +857,8 @@ __global__ void __launch_bounds__(32) k_ls_solve(WS ws, Dims d, LsDims ld, float
     atomicOr(reinterpret_cast<unsigned*>(&ws.ctrl[CTRL_STATUS]), LS_STATUS_NONFINITE);
     if (sticky) atomicOr(sticky, LS_STATUS_NONFINITE);
   }
-  reinterpret_cast<float2*>(out)[(size_t)job * d.vn + v] = make_float2(o0, o1);  // (y, x) pixels
+  out[((size_t)job * d.vn + v) * 2] = o0;  // (y, x) pixels; scalar stores: out need only be 4-byte aligned
+  out[((size_t)job * d.vn + v) * 2 + 1] = o1;
   if (dbg_sums)
 #pragma unroll
     for (int k = 0; k < 5; ++k) dbg_sums[((size_t)job * d.vn + v) * 5 + k] = acc[k];
@@ -877,8 +886,8 @@ __global__ void __launch_bounds__(32) k_ls_adjoint(WS ws, Dims d, LsDims ld, con
   double P00, P10, P01, P11;
   pinv2x2_apply(a, b, c, 1.0, 0.0, P00, P10);
   pinv2x2_apply(a, b, c, 0.0, 1.0, P01, P11);
-  const float2 go = reinterpret_cast<const float2*>(grad_out)[(size_t)job * d.vn + v];
-  const double g0 = (double)__fmul_rn(go.x, (float)ld.h), g1 = (double)__fmul_rn(go.y, (float)ld.h);
+  const float* go = grad_out + ((size_t)job * d.vn + v) * 2;  // scalar loads: grad_out need only be 4-byte aligned
+  const double g0 = (double)__fmul_rn(go[0], (float)ld.h), g1 = (double)__fmul_rn(go[1], (float)ld.h);
   const double x0 = P00 * q0 + P01 * q1, x1 = P10 * q0 + P11 * q1;
   const double l0 = P00 * g0 + P10 * g1, l1 = P01 * g0 + P11 * g1;  // P^T g
   // I - A P (A symmetric)
@@ -899,7 +908,9 @@ __global__ void __launch_bounds__(32) k_ls_adjoint(WS ws, Dims d, LsDims ld, con
 
 // blockIdx.x strides over the refinement tiles (all keypoints per thread: 72 + 36 contiguous bytes per pixel).
 // grad_direct [b,h,w,2*vn] and grad_conf [b,h,w,vn] must be zero-filled; pixels listed for one class are
-// stored, pixels listed for several (near-tie logits) are accumulated atomically.
+// stored, pixels listed for several (near-tie logits) are accumulated atomically.  VEC (chosen on the host): grad_direct
+// is 8-byte aligned and a pixel's (dy, dx) gradient is one float2 store, otherwise two scalar stores.
+template <bool VEC>
 __global__ void __launch_bounds__(256) k_ls_backward(WS ws, Dims d, LsWS lw, LsDims ld, const float* __restrict__ adj,
                                                      float* __restrict__ grad_direct, float* __restrict__ grad_conf) {
   const int tid = threadIdx.x;
@@ -952,7 +963,12 @@ __global__ void __launch_bounds__(256) k_ls_backward(WS ws, Dims d, LsWS lw, LsD
           atomicAdd(gdp + 1, gd1);
           atomicAdd(gcp, gc);
         } else {
-          *reinterpret_cast<float2*>(gdp) = make_float2(gd0, gd1);
+          if (VEC) {
+            *reinterpret_cast<float2*>(gdp) = make_float2(gd0, gd1);
+          } else {
+            gdp[0] = gd0;
+            gdp[1] = gd1;
+          }
           *gcp = gc;
         }
       }

@@ -166,6 +166,10 @@ int casa_host_wait(casa_handle* h, int64_t ticket);
  *   out     device float32 [b,num_classes-1,vn,2]  (y,x) pixels            voting_layers_2d.py:122
  * Fully asynchronous on `stream` unless check_finite is set (one 32-byte read-back that stands in
  * for the reference's tf.Assert on non-finite R / q / p, :109-121 -> CASA_ERR_INPUT).
+ * casa_ls_vote and casa_ls_vote_backward accept any 4-byte-aligned float buffer for seg, direct, conf, out,
+ * grad_points, grad_direct and grad_conf (e.g. a contiguous view that starts one float into an allocation, or a
+ * DLPack export with a byte offset); wider vector loads are used only where the pointer allows them.  The
+ * debug buffers (casa_ls_debug) need their element type's natural alignment.
  */
 typedef struct casa_ls_params {
   int32_t b, h, w;

@@ -117,7 +117,11 @@ def test_tied_logits_list_a_pixel_for_every_class(Layer):
     """All-equal segmentation logits (a zero-initialised seg head): softmax(1e6 * seg) is 1/nc for EVERY class, so each
     pixel is listed oc times and the per-image lists need oc*h*w slots — the layer must give the reference's weighted
     solution (weights 1/nc), not zeros (the first attempt at h*w slots overflows and is retried with the measured need);
-    the backward pass must see the same lists."""
+    the backward pass must see the same lists and give the gradient oracle's result (every pixel's gradient sums the
+    four classes' terms with atomicAdd)."""
+    from oracle import ls_voting_grad as G
+    from tests.test_ls_backward import _check, _mask_singular
+
     rng = np.random.default_rng(11)
     b, h, w, nc, vn = 2, 24, 32, 5, 3
     seg = np.zeros((b, h, w, nc), np.float32)
@@ -128,8 +132,13 @@ def test_tied_logits_list_a_pixel_for_every_class(Layer):
     assert (dbg["tn"].cpu().numpy() == h * w).all()
     assert np.abs(ref).max() > 1.0  # a real solution, not the zeros of a gated class
     layer = Layer("ls", nc, num_points=vn)
-    g = torch.ones((b, nc - 1, vn, 2), device="cuda")
-    gd, gw = layer.backward([torch.from_numpy(seg).cuda(), torch.from_numpy(direct).cuda(), torch.from_numpy(conf).cuda()], g)
+    g = _mask_singular(rng.normal(size=(b, nc - 1, vn, 2)).astype(np.float32), seg, direct, conf, num_points=vn)
+    assert (g != 0).all()  # every job is regular
+    gd, gw = layer.backward([torch.from_numpy(seg).cuda(), torch.from_numpy(direct).cuda(), torch.from_numpy(conf).cuda()],
+                            torch.from_numpy(g).cuda())
+    _, rd, rw = G.ls_vote_with_grads(seg, direct, conf, g, num_points=vn)
+    _check(gd.cpu().numpy(), rd, "grad_direct")
+    _check(gw.cpu().numpy(), rw, "grad_conf")
     assert float(gd.abs().max()) > 0 and float(gw.abs().max()) > 0
 
 
