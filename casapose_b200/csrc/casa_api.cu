@@ -253,8 +253,6 @@ struct casa_handle {
   cudaStream_t gather_stream = nullptr;
   cudaEvent_t gather_after[8] = {}, gather_done[8] = {};
   void* deferred_list = nullptr;  // std::vector<DeferredDelete>*: consumed DLPack capsules whose deleters are pending
-  int vertex_mapped = 0;          // the current call's vector field is mapped host memory (casa_ransac_vote_host)
-  int host_not_binary = 0;        // the host packer saw a mask value other than 0 / 1 in the current call
   MaskPacker* packer = nullptr;   // host threads of casa_ransac_vote_host
   uint32_t* bits_host = nullptr;  // page-locked staging of the packed membership words
   size_t bits_host_bytes = 0;
@@ -322,7 +320,7 @@ NcclApi g_nccl;
 
 int nccl_load() {
   if (g_nccl.lib) return CASA_OK;
-  const char* names[] = {getenv("CASA_NCCL_LIB"), "libnccl.so.2", "libnccl.so"};
+  const char* names[] = {getenv("CASA_NCCL_LIB"), "libnccl.so.2", "libnccl.so"};  // an NCCL outside the loader's path
   void* lib = nullptr;
   for (const char* n : names)
     if (n && !lib) lib = dlopen(n, RTLD_NOW | RTLD_GLOBAL);
@@ -390,6 +388,7 @@ extern "C" int casa_create(int device, casa_handle** out) {
     CUDA_TRY(cudaEventCreate(&c.ev1));
     CUDA_TRY(cudaEventCreateWithFlags(&c.ev_round, cudaEventDisableTiming));
   }
+  // direct launches stay selectable: LS debug calls need run_direct anyway, and it is the form a debugger can step
   if (getenv("CASA_NO_GRAPH")) h->use_graph = 0;
   *out = h;
   return CASA_OK;
@@ -870,22 +869,34 @@ static void reset_totals(casa_handle* h) {
   for (int k = 0; k < 4; ++k) h->stats[k] = 0;
 }
 
-static int collect(casa_handle* h) {
+struct Collected {  // the calls one collect() took in (lanes included)
+  int64_t slots = 0;
+  int64_t launches = 0;
+  uint32_t status = 0;  // OR of their status words
+};
+
+static int collect(casa_handle* h, Collected* got = nullptr) {
+  Collected mine;
+  if (!got) got = &mine;
   int first_rc = CASA_OK;
   for (int i = 0; i < kMaxLanes; ++i) {  // lanes: their calls are this handle's calls
     casa_handle* s = h->lane[i];
     if (!s) continue;
-    const int rc = collect(s);
+    Collected lc;
+    const int rc = collect(s, &lc);
     if (first_rc == CASA_OK) first_rc = rc;
     h->score_ms += s->score_ms;
     h->score_launches += s->score_launches;
     h->rounds_total += s->rounds_total;
     h->launches_total += s->launches_total;
     for (int k = 0; k < 4; ++k) h->stats[k] += s->stats[k];
-    if (i == h->lane_last) {
+    if (lc.slots && i == h->lane_last) {  // the last vote; a pass that finds nothing new keeps what the handle reports
       h->last_status = s->last_status;
       h->last_launches = s->last_launches;
     }
+    got->slots += lc.slots;
+    got->launches += lc.launches;
+    got->status |= lc.status;
     reset_totals(s);
   }
   while (h->slot_tail < h->slot_head) {
@@ -897,6 +908,8 @@ static int collect(casa_handle* h) {
     h->rounds_total += rounds;
     h->last_launches = c.base_launches + (int64_t)(rounds > 1 ? rounds - 1 : 0) * c.round_launches;
     h->launches_total += h->last_launches;
+    ++got->slots;
+    got->launches += h->last_launches;
     if (c.timed) {
       float ms = 0.f;
       CUDA_TRY(cudaEventElapsedTime(&ms, c.ev0, c.ev1));
@@ -904,6 +917,7 @@ static int collect(casa_handle* h) {
     }
     for (int k = 0; k < 4; ++k) h->stats[k] += c.stats[k];
     h->last_status = (uint32_t)c.ctrl[CTRL_STATUS];
+    got->status |= h->last_status;
     if (first_rc == CASA_OK) {
       if (h->last_status & CASA_STATUS_PIX_OVERFLOW)
         first_rc = fail(CASA_ERR_WORKSPACE, "pixel lists exceed pix_capacity (mask is not one-hot?); retry with a larger pix_capacity");
@@ -914,11 +928,12 @@ static int collect(casa_handle* h) {
   return first_rc;
 }
 
-// Lanes (casa_set_async(h, n >= 2)): the next call runs on sub-handle `lane_next`, on that lane's own stream, behind an
-// event recorded on the caller's stream now (the lane sees what the caller queued so far).
-static int lane_begin(casa_handle* h, void* stream, casa_handle** sub_out, int* k_out) {
+// Lanes (casa_set_async(h, n >= 2), the image ranges of casa_ransac_vote_host): the next call runs on sub-handle
+// `lane_next` of `n`, on that lane's own stream, behind an event recorded on the caller's stream now (the lane sees
+// what the caller queued so far).
+static int lane_begin(casa_handle* h, int n, void* stream, casa_handle** sub_out, int* k_out) {
   CUDA_TRY(cudaSetDevice(h->device));
-  const int k = h->lane_next % h->async_mode;
+  const int k = h->lane_next % n;
   if (!h->lane[k]) {
     int rcl = casa_create(h->device, &h->lane[k]);
     if (rcl) return rcl;
@@ -929,8 +944,6 @@ static int lane_begin(casa_handle* h, void* stream, casa_handle** sub_out, int* 
   }
   casa_handle* sub = h->lane[k];
   sub->timing = h->timing;
-  sub->vertex_mapped = h->vertex_mapped;
-  sub->host_not_binary = h->host_not_binary;
   CUDA_TRY(cudaEventRecord(h->lane_fork[k], (cudaStream_t)stream));
   CUDA_TRY(cudaStreamWaitEvent(sub->own_stream, h->lane_fork[k], 0));
   *sub_out = sub;
@@ -942,25 +955,34 @@ static int lane_end(casa_handle* h, int k, void* stream) {
   CUDA_TRY(cudaEventRecord(h->lane_done[k], h->lane[k]->own_stream));
   h->lane_pending[k] = 1;
   h->lane_last = k;
-  h->lane_next = (k + 1) % h->async_mode;
+  h->lane_next = k + 1;
   h->last_stream = (cudaStream_t)stream;
   return CASA_OK;
 }
 
-static int ransac_vote_impl(casa_handle* h, const casa_ransac_params* p, const float* mask, int mask_is_seg,
-                            const float* vertex, const int32_t* idxs, const float* selection, float* out_points,
-                            const casa_ransac_debug* debug, void* stream) {
-  if (!h) return fail(CASA_ERR_INVALID, "handle is NULL");
-  if (!mask || !vertex || !out_points) return fail(CASA_ERR_INVALID, "mask / vertex / out_points must not be NULL");
-  if (h->async_mode >= 2 && !debug && !h->is_lane) {  // lanes: this vote runs on a sub-handle's own stream
-    casa_handle* sub = nullptr;
-    int k = 0;
-    int rcl = lane_begin(h, stream, &sub, &k);
-    if (rcl) return rcl;
-    rcl = ransac_vote_impl(sub, p, mask, mask_is_seg, vertex, idxs, selection, out_points, nullptr, (void*)sub->own_stream);
-    const int rce = lane_end(h, k, stream);
-    return rcl ? rcl : rce;
-  }
+// How a vote's mask arrives.
+enum class MaskForm {
+  kOneHot,     // float [b,h,w,oc] one-hot mask (casa_ransac_vote)
+  kSeg,        // float [b,h,w,1+oc] segmentation scores, arg-max on the device (casa_ransac_vote_seg)
+  kPackedBits  // u32 [b,h,w] membership words packed on the host (casa_ransac_vote_host)
+};
+
+// The inputs and outputs of one vote.
+struct VoteInput {
+  const void* mask = nullptr;
+  MaskForm form = MaskForm::kOneHot;
+  const float* vertex = nullptr;
+  bool vertex_mapped = false;  // the field is mapped host memory: k_gather_dirs reads it over PCIe, not k_place
+  int not_binary = 0;          // kPackedBits: the host packer saw a mask value other than 0 / 1
+  const int32_t* idxs = nullptr;
+  const float* selection = nullptr;
+  float* out = nullptr;
+};
+
+// Builds the launch list of one vote and launches it on `st` with `h`'s workspace, into the next read-back slot of
+// `h` (collect() reads the slot back).  Waits for the host only when that ring of slots is full.
+static int vote_enqueue(casa_handle* h, const casa_ransac_params* p, const VoteInput& in, const casa_ransac_debug* debug,
+                        cudaStream_t st) {
   Layout L;
   int rc = make_layout(p, L);
   if (rc) return rc;
@@ -968,12 +990,10 @@ static int ransac_vote_impl(casa_handle* h, const casa_ransac_params* p, const f
   if (h->ws_bytes < L.total) h->clean_ctrl = nullptr;
   rc = ensure(&h->ws_mem, &h->ws_bytes, L.total);
   if (rc) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
   if (h->slot_head - h->slot_tail >= kCallSlots) {  // the ring of read-back slots is full: collect the queued calls
     rc = collect(h);
     if (rc) return rc;
   }
-  if (!h->async_mode) reset_totals(h);  // synchronous calls report per-call statistics
   CallSlot* slot = &h->slots[h->slot_head % kCallSlots];
   h->last_stream = st;
   casa_ransac_debug dbg;
@@ -995,20 +1015,18 @@ static int ransac_vote_impl(casa_handle* h, const casa_ransac_params* p, const f
     CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->score_occ_narrow, k_score<kHypPerLaneNarrow>, kScoreThreads, 0));
     if (h->score_occ < 1 || h->score_occ_narrow < 1) return fail(CASA_ERR_INVALID, "scoring kernel does not fit");
     // The kernel is compiled for two resident blocks per SM (113 registers: ransac.cuh).  With the four-block build of
-    // the first half of round 2 (CASA_SCORE_MINB=4) votes on lanes ran three blocks per SM and left the fourth slot to
+    // the first half of round 2 (64 registers) votes on lanes ran three blocks per SM and left the fourth slot to
     // the neighbouring votes' short kernels (1-2 % per step: profiles/r02_lanes_overlap.txt).
-    int cap = h->is_lane ? 3 : h->score_occ;
-    const char* bps = getenv("CASA_SCORE_BPS");  // experiments
-    if (bps && atoi(bps) >= 1) cap = atoi(bps);
+    const int cap = h->is_lane ? 3 : h->score_occ;
     if (cap < h->score_occ) h->score_occ = cap;
     if (cap < h->score_occ_narrow) h->score_occ_narrow = cap;
   }
-  const bool narrow = score_hpl(d.hn) == kHypPerLaneNarrow && !getenv("CASA_SCORE_WIDE");
+  const bool narrow = score_hpl(d.hn) == kHypPerLaneNarrow;
   const void* score_fn = narrow ? (const void*)k_score<kHypPerLaneNarrow> : (const void*)k_score<kHypPerLaneWide>;
   const int score_occ = narrow ? h->score_occ_narrow : h->score_occ;
   const int refine_gx = d.max_rtiles < h->sm_count * 4 ? d.max_rtiles : h->sm_count * 4;
   const int gather_gx = (d.cap + 255) / 256 < 24 ? (d.cap + 255) / 256 : 24;
-  const int vec4 = ((((size_t)d.hw * d.oc) & 3) == 0) && ((((uintptr_t)mask) & 15) == 0);
+  const int vec4 = ((((size_t)d.hw * d.oc) & 3) == 0) && ((((uintptr_t)in.mask) & 15) == 0);
   const int plan_threads = d.J > 256 ? 1024 : 256;
 
   // The launch list of the whole call.  Round 0 is spelled out (it carries the timing events, which a WHILE body
@@ -1025,25 +1043,25 @@ static int ransac_vote_impl(casa_handle* h, const casa_ransac_params* p, const f
     CUDA_TRY(cudaMemsetAsync(ws.ctrl, 0, CTRL_WORDS * sizeof(int), st));
     CUDA_TRY(cudaMemsetAsync(ws.stats, 0, 4 * sizeof(unsigned long long), st));
   }
-  if (mask_is_seg == 2)  // membership words packed on the host (casa_ransac_vote_host); bit 30 of the flag: not binary
-    steps.push_back(kstep((const void*)k_bits_in, dim3(d.nct, d.b), 256).arg((const uint32_t*)mask).arg(ws).arg(d).arg(h->host_not_binary));
-  else if (mask_is_seg)
-    steps.push_back(kstep((const void*)k_seg_bits, dim3(d.nct, d.b), 256).arg(mask).arg(ws).arg(d));
+  if (in.form == MaskForm::kPackedBits)  // bit 30 of the flag: not binary
+    steps.push_back(kstep((const void*)k_bits_in, dim3(d.nct, d.b), 256).arg((const uint32_t*)in.mask).arg(ws).arg(d).arg(in.not_binary));
+  else if (in.form == MaskForm::kSeg)
+    steps.push_back(kstep((const void*)k_seg_bits, dim3(d.nct, d.b), 256).arg((const float*)in.mask).arg(ws).arg(d));
   else
-    steps.push_back(kstep((const void*)k_mask_bits, dim3(d.nct, d.b), 256).arg(mask).arg(ws).arg(d).arg(vec4));
+    steps.push_back(kstep((const void*)k_mask_bits, dim3(d.nct, d.b), 256).arg((const float*)in.mask).arg(ws).arg(d).arg(vec4));
   // k_place gathers the directions while it scatters the pixels, unless the field lives in mapped host memory (the
   // host entry point: k_gather_dirs reads full lines over PCIe) or is not 8-byte aligned; jobs above max_num are
   // gathered after the cap filter
-  const int fuse_gather = (!h->vertex_mapped && (((uintptr_t)vertex) & 7) == 0 && !getenv("CASA_NO_FUSED_GATHER")) ? 1 : 0;
+  const int fuse_gather = (!in.vertex_mapped && (((uintptr_t)in.vertex) & 7) == 0) ? 1 : 0;
   const bool may_cap = (float)d.hw > p->max_num;
-  steps.push_back(kstep(d.vn == 9 ? (const void*)k_place<9> : (const void*)k_place<0>, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg(vertex).arg(ws).arg(d).arg(fuse_gather));
-  if (may_cap) steps.push_back(kstep((const void*)k_cap_filter, d.J, 1024).arg(ws).arg(d).arg(selection));
+  steps.push_back(kstep(d.vn == 9 ? (const void*)k_place<9> : (const void*)k_place<0>, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg(in.vertex).arg(ws).arg(d).arg(fuse_gather));
+  if (may_cap) steps.push_back(kstep((const void*)k_cap_filter, d.J, 1024).arg(ws).arg(d).arg(in.selection));
   // round 0's plan (work items, refinement tiles) only needs the job table: it runs beside the direction gather and
   // k_hypgen (side branch in slot 1, joined by k_score)
   steps.push_back(kstep((const void*)k_plan, 1, plan_threads).arg(ws).arg(d).arg((int)0).on_side(1, 1));
   if (!fuse_gather || may_cap)
     steps.push_back(kstep(d.vn == 9 ? (const void*)k_gather_dirs<18> : (const void*)k_gather_dirs<0>, dim3(gather_gx, d.J), 256)
-                        .arg(vertex).arg(ws).arg(d).arg(fuse_gather));
+                        .arg(in.vertex).arg(ws).arg(d).arg(fuse_gather));
   for (int part = 0; part < 2; ++part) {  // part 0: round 0; part 1: the WHILE body (rnd = -1: read ctrl[CTRL_ROUND])
     const int rnd = part == 0 ? 0 : -1;
     if (part == 1) {
@@ -1052,7 +1070,7 @@ static int ransac_vote_impl(casa_handle* h, const casa_ransac_params* p, const f
       steps.push_back(kstep((const void*)k_plan, 1, plan_threads).arg(ws).arg(d).arg(rnd));
     }
     const size_t n0 = steps.size();
-    Step hg = kstep((const void*)k_hypgen, dim3((d.hn * d.vn + 255) / 256, d.J), 256).arg(ws).arg(d).arg(fc).arg(idxs).arg(rnd).arg(dbg.hyps);
+    Step hg = kstep((const void*)k_hypgen, dim3((d.hn * d.vn + 255) / 256, d.J), 256).arg(ws).arg(d).arg(fc).arg(in.idxs).arg(rnd).arg(dbg.hyps);
     steps.push_back(hg);
     // the timing events hang off the chain as leaves: ev0 fires when k_hypgen is done, ev1 when k_score is done
     if (part == 0 && h->timing) steps.push_back(special(STEP_EV0, 1));
@@ -1072,7 +1090,7 @@ static int ransac_vote_impl(casa_handle* h, const casa_ransac_params* p, const f
   // and solve do not wait for the copy engine
   steps.push_back(special(STEP_READBACK, 1));
   steps.push_back(special(STEP_CLEAR, 2));
-  steps.push_back(kstep((const void*)k_refine_solve, dim3(refine_gx, d.vn), kRefineThreads).arg(ws).arg(d).arg(fc).arg(out_points).arg(dbg));
+  steps.push_back(kstep((const void*)k_refine_solve, dim3(refine_gx, d.vn), kRefineThreads).arg(ws).arg(d).arg(fc).arg(in.out).arg(dbg));
   for (const Step& s2 : steps) base_launches += s2.kind == STEP_KERNEL;
   base_launches -= round_launches;  // the body's kernels are counted per executed round below
   slot->timed = h->timing;
@@ -1084,23 +1102,54 @@ static int ransac_vote_impl(casa_handle* h, const casa_ransac_params* p, const f
   h->clean_ctrl = ws.ctrl;
   CUDA_TRY(cudaGetLastError());
   if (dbg.pix) CUDA_TRY(cudaMemcpyAsync(dbg.pix, ws.pix, (size_t)d.b * d.cap * 4, cudaMemcpyDeviceToDevice, st));
-  if (h->async_mode && !dbg.stats) return CASA_OK;  // status, statistics and timing are collected by casa_sync()
+  return CASA_OK;
+}
+
+// A vote of the device entry points: on the next lane when the handle rotates over lanes (casa_set_async(h, n >= 2))
+// and no debug outputs are asked for, otherwise on `stream`, collected at once when the handle is synchronous.
+// *ran_on: the stream the vote's work went to.
+static int ransac_vote_route(casa_handle* h, const casa_ransac_params* p, const VoteInput& in,
+                             const casa_ransac_debug* debug, void* stream, cudaStream_t* ran_on) {
+  const cudaStream_t st = (cudaStream_t)stream;
+  *ran_on = st;
+  if (!h) return fail(CASA_ERR_INVALID, "handle is NULL");
+  if (!in.mask || !in.vertex || !in.out) return fail(CASA_ERR_INVALID, "mask / vertex / out_points must not be NULL");
+  if (h->async_mode >= 2 && !debug) {
+    casa_handle* sub = nullptr;
+    int k = 0;
+    int rc = lane_begin(h, h->async_mode, stream, &sub, &k);
+    if (rc) return rc;
+    *ran_on = sub->own_stream;
+    rc = vote_enqueue(sub, p, in, nullptr, sub->own_stream);
+    const int rce = lane_end(h, k, stream);
+    return rc ? rc : rce;
+  }
+  if (!h->async_mode) reset_totals(h);  // synchronous calls report per-call statistics
+  int rc = vote_enqueue(h, p, in, debug, st);
+  if (rc) return rc;
+  const bool want_stats = debug && debug->stats;
+  if (h->async_mode && !want_stats) return CASA_OK;  // status, statistics and timing are collected by casa_sync()
   rc = collect(h);
   // debug copy of the statistics: from the call's read-back slot (the workspace words are cleared by the graph)
-  if (dbg.stats) CUDA_TRY(cudaMemcpyAsync(dbg.stats, slot->stats, 4 * 8, cudaMemcpyHostToDevice, st));
+  if (want_stats)
+    CUDA_TRY(cudaMemcpyAsync(debug->stats, h->slots[(h->slot_head - 1) % kCallSlots].stats, 4 * 8, cudaMemcpyHostToDevice, st));
   return rc;
 }
 
 extern "C" int casa_ransac_vote(casa_handle* h, const casa_ransac_params* p, const float* mask, const float* vertex,
                                 const int32_t* idxs, const float* selection, float* out_points,
                                 const casa_ransac_debug* debug, void* stream) {
-  return ransac_vote_impl(h, p, mask, 0, vertex, idxs, selection, out_points, debug, stream);
+  const VoteInput in{mask, MaskForm::kOneHot, vertex, /*vertex_mapped=*/false, /*not_binary=*/0, idxs, selection, out_points};
+  cudaStream_t ran_on;
+  return ransac_vote_route(h, p, in, debug, stream, &ran_on);
 }
 
 extern "C" int casa_ransac_vote_seg(casa_handle* h, const casa_ransac_params* p, const float* seg, const float* vertex,
                                     const int32_t* idxs, const float* selection, float* out_points,
                                     const casa_ransac_debug* debug, void* stream) {
-  return ransac_vote_impl(h, p, seg, 1, vertex, idxs, selection, out_points, debug, stream);
+  const VoteInput in{seg, MaskForm::kSeg, vertex, /*vertex_mapped=*/false, /*not_binary=*/0, idxs, selection, out_points};
+  cudaStream_t ran_on;
+  return ransac_vote_route(h, p, in, debug, stream, &ran_on);
 }
 
 // ------------------------------------------------------------------------------------------------ DLPack shim
@@ -1212,16 +1261,18 @@ extern "C" int casa_ransac_vote_dlpack(casa_handle* h, const casa_ransac_params*
   if (vs[0] != ms[0] || vs[1] != ms[1] || vs[2] != ms[2] || vs[v->dl_tensor.ndim - 1] != 2 || (q.vertex_per_class && vs[3] != q.oc))
     return reject(fail(CASA_ERR_INVALID, "vertex must be [b,h,w,vn,2] or [b,h,w,oc,vn,2] matching the mask"));
   if (os[0] != q.b || os[1] != q.oc || os[2] != q.vn || os[3] != 2) return reject(fail(CASA_ERR_INVALID, "out must be [b,oc,vn,2]"));
-  rc = ransac_vote_impl(h, &q, dl_data(m), mask_is_seg, dl_data(v), nullptr, nullptr, (float*)dl_data(o), nullptr, stream);
-  // the capsules are consumed either way: their deleters run once the work queued so far on `stream` has finished
+  const VoteInput in{dl_data(m), mask_is_seg ? MaskForm::kSeg : MaskForm::kOneHot, dl_data(v), false, 0, nullptr, nullptr,
+                     (float*)dl_data(o)};
+  cudaStream_t ran_on;
+  rc = ransac_vote_route(h, &q, in, nullptr, stream, &ran_on);
+  // the capsules are consumed either way: their deleters run once the work queued so far where the vote ran has finished
   cudaEvent_t done = nullptr;
-  if (h->async_mode >= 2 && h->lane_last >= 0) stream = (void*)h->lane[h->lane_last]->own_stream;  // the vote ran on a lane
-  if (cudaEventCreateWithFlags(&done, cudaEventDisableTiming) == cudaSuccess && cudaEventRecord(done, (cudaStream_t)stream) == cudaSuccess) {
+  if (cudaEventCreateWithFlags(&done, cudaEventDisableTiming) == cudaSuccess && cudaEventRecord(done, ran_on) == cudaSuccess) {
     deferred(h).push_back({m, done});
     deferred(h).push_back({v, done});
     deferred(h).push_back({o, done});
   } else {
-    cudaStreamSynchronize((cudaStream_t)stream);
+    cudaStreamSynchronize(ran_on);
     if (m->deleter) m->deleter(m);
     if (v->deleter) v->deleter(v);
     if (o->deleter) o->deleter(o);
@@ -1241,7 +1292,8 @@ static bool host_pointer_is_mapped(const void* p, const void** dev_ptr) {
   return true;
 }
 
-// CASA_HOST_TRACE=1: host-side time stamps of the phases of casa_ransac_vote_host on stderr (microseconds)
+// CASA_HOST_TRACE=1: host-side time stamps of the phases of casa_ransac_vote_host on stderr (microseconds); it only
+// prints, so it stays for looking at the overlap of packing, copies and votes in a deployment
 static double host_now_us() {
   return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
@@ -1257,7 +1309,7 @@ static bool host_trace_on() {
 // Waits for `st`.  The driver threads of the pipelined host entry sleep on a blocking-sync event: a spinning
 // cudaStreamSynchronize would take a core from the packer threads for the two milliseconds of a call's GPU tail.
 static int host_wait_stream(casa_handle* h, cudaStream_t st) {
-  if (h->host_parent && !getenv("CASA_HOST_SPIN")) {
+  if (h->host_parent) {
     if (!h->ev_block) CUDA_TRY(cudaEventCreateWithFlags(&h->ev_block, cudaEventBlockingSync | cudaEventDisableTiming));
     CUDA_TRY(cudaEventRecord(h->ev_block, st));
     CUDA_TRY(cudaEventSynchronize(h->ev_block));
@@ -1280,23 +1332,12 @@ extern "C" int casa_ransac_vote_host(casa_handle* h, const casa_ransac_params* p
   const size_t mask_n = (size_t)p->b * hw * p->oc * 4, vert_n = (size_t)p->b * hw * vfields * p->vn * 2 * 4;
   const size_t out_b = (size_t)p->b * p->oc * p->vn * 2 * 4;
   cudaStream_t st = h->own_stream;
-  struct AsyncOff {  // the parts below are collected one by one
-    casa_handle* h;
-    int saved;
-    explicit AsyncOff(casa_handle* hh) : h(hh), saved(hh->async_mode) { h->async_mode = 0; }
-    ~AsyncOff() { h->async_mode = saved; }
-  } async_off(h);
-  struct MappedFlag {  // set while the vote reads the vector field from mapped host memory (k_gather_dirs, not k_place)
-    casa_handle* h;
-    explicit MappedFlag(casa_handle* hh) : h(hh) {}
-    ~MappedFlag() { h->vertex_mapped = 0; }
-  } mapped_flag(h);
   // Pinned (page-locked) host buffers: the mask is DMA-copied in up to 4 image ranges on a copy stream while the
   // previous range is being voted on, and the vector field is never copied — k_gather_dirs reads only the masked
   // pixels' rows straight from the mapped host buffer.  About 200 MB instead of 511 MB cross PCIe for a 16-frame
   // batch, and the voting hides behind the mask transfer.  Pageable buffers are staged in one piece.
   const void *dm = nullptr, *dv = nullptr;
-  const bool vertex_mapped = !getenv("CASA_NO_ZERO_COPY") && host_pointer_is_mapped(vertex_host, &dv);
+  const bool vertex_mapped = host_pointer_is_mapped(vertex_host, &dv);
   const bool mask_mapped = host_pointer_is_mapped(mask_host, &dm);
   // host-side packing of the mask (any host memory: the CPU reads it) needs the vector field to be readable in place
   // host threads a rank may use for packing: one process per GPU (torchrun exports LOCAL_WORLD_SIZE) shares the node's
@@ -1306,9 +1347,11 @@ extern "C" int casa_ransac_vote_host(casa_handle* h, const casa_ransac_params* p
   {
     const char* lws = getenv("LOCAL_WORLD_SIZE");
     if (lws && atoi(lws) > 1) pack_threads = ((int)std::thread::hardware_concurrency() - atoi(lws)) / atoi(lws);
+    // CASA_HOST_THREADS: a deployment knob for hosts whose cores are shared with more than the node's ranks
     if (getenv("CASA_HOST_THREADS")) pack_threads = atoi(getenv("CASA_HOST_THREADS"));
     pack_threads = pack_threads > 12 ? 12 : pack_threads;  // 15 of 16 cores lose to oversubscription (profiles/r02_e2e.txt)
   }
+  // CASA_NO_HOST_PACK=1: every range crosses PCIe as raw floats (bench.py reads it to count the bytes a step moves)
   const bool pack = vertex_mapped && !getenv("CASA_NO_HOST_PACK") && p->oc <= 32 && (pack_threads >= 4 || !mask_mapped);
   const bool zero_copy = vertex_mapped && (pack || mask_mapped);
   const size_t bits_n = (size_t)p->b * hw * sizeof(uint32_t);
@@ -1319,29 +1362,36 @@ extern "C" int casa_ransac_vote_host(casa_handle* h, const casa_ransac_params* p
   if (rc) return rc;
   float* dmask = (float*)h->io_mem;
   float* dout = (float*)((char*)h->io_mem + mask_b + vert_b);
+  // The votes of the image ranges run on lanes (own workspace and stream each): the direction gather of one range
+  // (mapped reads over PCIe) and the short kernels of another overlap the scoring of a third, instead of four votes
+  // one behind the other on one stream.  A single range runs on the handle's own stream.
+  const int parts = !zero_copy ? 1 : (p->b >= 8 ? 4 : (p->b >= 2 ? 2 : 1));
+  if (parts >= 2)
+    for (int i = 0; i < kMaxLanes; ++i)  // lanes a caller left busy
+      if (h->lane[i] && h->lane_pending[i]) {
+        CUDA_TRY(cudaStreamSynchronize(h->lane[i]->own_stream));
+        h->lane_pending[i] = 0;
+      }
+  rc = collect(h);  // the calls before this one: what is collected below is this call's alone
+  if (rc) return rc;
+  reset_totals(h);
   if (!zero_copy) {
     float* dvert = (float*)((char*)h->io_mem + mask_b);
     CUDA_TRY(cudaMemcpyAsync(dmask, mask_host, mask_n, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(dvert, vertex_host, vert_n, cudaMemcpyHostToDevice, st));
-    rc = casa_ransac_vote(h, p, dmask, dvert, nullptr, nullptr, dout, nullptr, (void*)st);
+    rc = vote_enqueue(h, p, VoteInput{dmask, MaskForm::kOneHot, dvert, false, 0, nullptr, nullptr, dout}, nullptr, st);
     if (rc) return rc;
   } else {
-    h->vertex_mapped = 1;
-    int parts = p->b >= 8 ? 4 : (p->b >= 2 ? 2 : 1);
-    if (getenv("CASA_HOST_PARTS")) parts = atoi(getenv("CASA_HOST_PARTS"));
-    if (parts < 1) parts = 1;
-    if (parts > 8) parts = 8;
-    if (parts > p->b) parts = p->b;
     const size_t mask_img = hw * p->oc, vert_img = hw * vfields * p->vn * 2, out_img = (size_t)p->oc * p->vn * 2;
-    int start[9];
+    int start[kMaxLanes + 1];
     for (int k = 0; k <= parts; ++k) start[k] = (int)((long long)p->b * k / parts);
     // The one-hot mask is 32 bytes per pixel for 4 bits of information.  Two engines move it in parallel: the copy
     // engine DMA-copies the raw floats of the even image ranges over PCIe, host threads (MaskPacker) turn the odd
     // ranges into u32 membership words — 1/oc of the bytes — while the GPU votes on the ranges before them.
     // (Packing everything on the host is no faster than the DMA on a 16-core host: profiles/r02_e2e.txt.)
     uint32_t* dbits = (uint32_t*)((char*)h->io_mem + mask_b - bits_b);
-    bool packed[9] = {false, false, false, false, false, false, false, false, false};
-    int pack_index[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+    bool packed[kMaxLanes] = {false, false, false, false};
+    int pack_index[kMaxLanes] = {0, 0, 0, 0};
     // pipelined calls (casa_ransac_vote_host_async) share the parent handle's packer threads: the gate is held from the
     // start of this call's packing until its last range is packed, then the next call's packing starts while this
     // call's last ranges are still being voted on
@@ -1366,7 +1416,7 @@ extern "C" int casa_ransac_vote_host(casa_handle* h, const casa_ransac_params* p
       // outruns the DMA of the raw floats: every range is packed and only 4 bytes per pixel cross PCIe (e2e 3.08 ms
       // against 3.76 ms per 16 frames with half of the ranges packed: profiles/r02_e2e.txt).  With 4 or 5 threads the
       // odd ranges are packed beside the DMA of the even ones.  A pageable mask cannot be DMA-copied in place.
-      const bool all = (pack_threads >= 6 && !getenv("CASA_HOST_PACK_HALF")) || getenv("CASA_HOST_PACK_ALL") != nullptr || !mask_mapped;
+      const bool all = pack_threads >= 6 || !mask_mapped;
       std::vector<size_t> bounds;
       for (int k = 0; k < parts; ++k) {
         packed[k] = all || (k & 1);
@@ -1385,46 +1435,40 @@ extern "C" int casa_ransac_vote_host(casa_handle* h, const casa_ransac_params* p
       CUDA_TRY(cudaMemcpyAsync(dmask + o, mask_host + o, n * 4, cudaMemcpyHostToDevice, h->copy_stream));
       CUDA_TRY(cudaEventRecord(h->part_ev[k], h->copy_stream));
     }
-    int64_t launches = 0;
-    double score_ms = 0.0;
-    int64_t score_launches = 0;
-    uint64_t stats[4] = {0, 0, 0, 0};
-    uint32_t status = 0;
-    // The votes of the image ranges run on lanes (own workspace and stream each, casa_set_async(h, n)): the direction
-    // gather of one range (mapped reads over PCIe) and the short kernels of another overlap the scoring of a third,
-    // instead of four votes one behind the other on one stream.
-    const bool use_lanes = parts >= 2 && !getenv("CASA_HOST_NO_LANES");
-    if (use_lanes) {
-      for (int i = 0; i < kMaxLanes; ++i)  // lanes a caller left busy
-        if (h->lane[i] && h->lane_pending[i]) {
-          CUDA_TRY(cudaStreamSynchronize(h->lane[i]->own_stream));
-          h->lane_pending[i] = 0;
-        }
-      rc = collect(h);
-      if (rc) return rc;
-      reset_totals(h);
-      h->async_mode = parts < kMaxLanes ? parts : kMaxLanes;  // restored by async_off
-    }
     for (int k = 0; k < parts; ++k) {
       casa_ransac_params pp = *p;
       pp.b = start[k + 1] - start[k];
       pp.image_offset = p->image_offset + start[k];
+      VoteInput in;
+      in.vertex = (const float*)dv + (size_t)start[k] * vert_img;
+      in.vertex_mapped = true;
+      in.out = dout + (size_t)start[k] * out_img;
       if (packed[k]) {
         po->packer->wait_part((size_t)pack_index[k]);
         HOST_TRACE(h, "packed", k);
-        h->host_not_binary = po->packer->not_binary();
+        in.mask = dbits + (size_t)start[k] * hw;
+        in.form = MaskForm::kPackedBits;
+        in.not_binary = po->packer->not_binary();
         if (k == last_packed && gate.owns_lock()) gate.unlock();  // the packer threads are free for the next call
         const size_t o = (size_t)start[k] * hw, n = (size_t)pp.b * hw;
         CUDA_TRY(cudaMemcpyAsync(dbits + o, h->bits_host + o, n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->copy_stream));
         CUDA_TRY(cudaEventRecord(h->part_ev[k], h->copy_stream));
+      } else {
+        in.mask = dmask + (size_t)start[k] * mask_img;
       }
       CUDA_TRY(cudaStreamWaitEvent(st, h->part_ev[k], 0));
-      if (packed[k])
-        rc = ransac_vote_impl(h, &pp, (const float*)(dbits + (size_t)start[k] * hw), 2, (const float*)dv + (size_t)start[k] * vert_img,
-                              nullptr, nullptr, dout + (size_t)start[k] * out_img, nullptr, (void*)st);
-      else
-        rc = casa_ransac_vote(h, &pp, dmask + (size_t)start[k] * mask_img, (const float*)dv + (size_t)start[k] * vert_img,
-                              nullptr, nullptr, dout + (size_t)start[k] * out_img, nullptr, (void*)st);
+      if (parts >= 2) {
+        casa_handle* sub = nullptr;
+        int lane = 0;
+        rc = lane_begin(h, parts, (void*)st, &sub, &lane);
+        if (!rc) {
+          rc = vote_enqueue(sub, &pp, in, nullptr, sub->own_stream);
+          const int rce = lane_end(h, lane, (void*)st);
+          if (!rc) rc = rce;
+        }
+      } else {
+        rc = vote_enqueue(h, &pp, in, nullptr, st);
+      }
       HOST_TRACE(h, "issued", k);
       if (rc) {
         if (pack)
@@ -1432,37 +1476,24 @@ extern "C" int casa_ransac_vote_host(casa_handle* h, const casa_ransac_params* p
             if (packed[j]) po->packer->wait_part((size_t)pack_index[j]);  // the workers still read the caller's buffer
         return rc;
       }
-      if (use_lanes) continue;  // collected below
-      launches += h->last_launches;
-      score_ms += h->score_ms;
-      score_launches += h->score_launches;
-      status |= h->last_status;
-      for (int j = 0; j < 4; ++j) stats[j] += h->stats[j];
     }
-    if (use_lanes) {
+    if (parts >= 2) {
       rc = casa_join(h, (void*)st);  // the result copy below waits for every lane
       if (rc) return rc;
-      CUDA_TRY(cudaMemcpyAsync(out_points_host, dout, out_b, cudaMemcpyDeviceToHost, st));
-      rc = host_wait_stream(h, st);
-      if (rc) return rc;
-      HOST_TRACE(h, "done", 0);
-      for (int i = 0; i < kMaxLanes; ++i) h->lane_pending[i] = 0;
-      rc = collect(h);  // loop states, statistics and the first error of the ranges' votes
-      h->last_launches = h->launches_total;
-      uint32_t st_all = 0;
-      for (int i = 0; i < kMaxLanes; ++i)
-        if (h->lane[i]) st_all |= h->lane[i]->last_status;
-      h->last_status = st_all;
-      return rc;
     }
-    h->last_launches = launches;
-    h->score_ms = score_ms;
-    h->score_launches = score_launches;
-    h->last_status = status;
-    for (int j = 0; j < 4; ++j) h->stats[j] = stats[j];
   }
   CUDA_TRY(cudaMemcpyAsync(out_points_host, dout, out_b, cudaMemcpyDeviceToHost, st));
-  return host_wait_stream(h, st);
+  rc = host_wait_stream(h, st);
+  if (rc) return rc;
+  HOST_TRACE(h, "done", 0);
+  if (parts >= 2)
+    for (int i = 0; i < kMaxLanes; ++i) h->lane_pending[i] = 0;
+  // loop states, statistics and the first error of this call's votes; the status is the OR over its image ranges
+  Collected got;
+  rc = collect(h, &got);
+  h->last_status = got.status;
+  h->last_launches = got.launches;
+  return rc;
 }
 
 extern "C" int casa_selftest_pack(const float* mask, uint32_t* bits, int64_t npx, int oc, int threads, int parts) {
@@ -1586,7 +1617,7 @@ extern "C" int casa_ransac_vote_host_async(casa_handle* h, const casa_ransac_par
   }
   if (!h->host_depth) {
     int depth = 2;
-    if (getenv("CASA_HOST_DEPTH")) depth = atoi(getenv("CASA_HOST_DEPTH"));
+    if (getenv("CASA_HOST_DEPTH")) depth = atoi(getenv("CASA_HOST_DEPTH"));  // documented in casapose_b200.h
     h->host_depth = depth < 1 ? 1 : (depth > 4 ? 4 : depth);
   }
   const int k = (int)(h->host_ticket % h->host_depth);
@@ -1661,7 +1692,7 @@ extern "C" int casa_ls_vote(casa_handle* h, const casa_ls_params* p, const float
   if (h->async_mode >= 2 && !debug && !p->check_finite && !h->is_lane) {  // lanes, as for the votes (check_finite waits for the host)
     casa_handle* sub = nullptr;
     int k = 0;
-    int rcl = lane_begin(h, stream, &sub, &k);
+    int rcl = lane_begin(h, h->async_mode, stream, &sub, &k);
     if (rcl) return rcl;
     rcl = ls_vote_impl(sub, p, seg, direct, conf, out_points, nullptr, (void*)sub->own_stream, nullptr);
     const int rce = lane_end(h, k, stream);
@@ -1700,7 +1731,7 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
   // The forward call reduces 512-entry tiles in one fused pass and finds the components over horizontal runs
   // (k_cc_runs); gradient and debug calls keep the pixel-level union-find, whose forest the backward pass and the
   // debug outputs read.
-  const bool runs_cc = !grad && !debug && !getenv("CASA_LS_PIXEL_CC");
+  const bool runs_cc = !grad && !debug;
   const int ls_tile = grad ? kRefineTile : kFusedTile;
   Layout L;
   int rc = make_layout(&rp, L, ls_tile);

@@ -10,10 +10,7 @@ namespace casa {
 constexpr int kCountTile = 1024;   // pixels per block in the mask / scatter kernels (256 thr x 4)
 constexpr int kScoreWarps = 8;     // warps per scoring block
 constexpr int kScoreThreads = kScoreWarps * 32;
-#ifndef CASA_CHUNK
-#define CASA_CHUNK 128
-#endif
-constexpr int kChunk = CASA_CHUNK;  // pixels per scoring work item (one warp); 256 is an A/B build (profiles/r02_ab.txt)
+constexpr int kChunk = 128;        // pixels per scoring work item (one warp); 256: no faster, 64: -5 % (profiles/r02_ab.txt)
 constexpr int kRefineTile = 1024;  // pixels per reduction tile of the LS layer (256 threads x 4)
 constexpr int kVoteTile = 2048;    // pixels per refinement tile of the voting path (256 threads x 8)
 

@@ -166,7 +166,7 @@ __device__ __forceinline__ unsigned prmt_sign2(float a, float b) {
   return r;
 }
 
-// Build-time knobs of k_score, chosen by same-box A/B runs (profiles/r02_ab.txt).  The kernel is bound by dispatch
+// Tuning constants of k_score, chosen by same-box A/B builds (profiles/r02_ab.txt).  The kernel is bound by dispatch
 // cycles, and the register allocation ptxas finds for the 440-instruction loop body moves the result by +-2 %:
 //   hypotheses per lane 8 (16: 128 registers, -8..-13 %), TWO resident blocks/SM at 113 registers (the kernel keeps its
 //   rate down to two blocks per SM — it is bound by issue slots, not occupancy — and without the 64-register squeeze
@@ -175,19 +175,10 @@ __device__ __forceinline__ unsigned prmt_sign2(float a, float b) {
 //   __maxnreg__ or a larger launch-bounds thread count: all slower, 0.723..0.783 ms), 8 pixels per trip (16: the same,
 //   4: -1 %), binary search over item_start (a 16-byte record per chunk removed the search but cost 2-4 % through a
 //   worse allocation of the loop).
-#ifndef CASA_HPL
-#define CASA_HPL 8
-#endif
-#ifndef CASA_SCORE_MINB
-#define CASA_SCORE_MINB 2
-#endif
-#ifndef CASA_PIX_UNROLL
-#define CASA_PIX_UNROLL 8
-#endif
-constexpr int kHypPerLaneWide = CASA_HPL;         // hypotheses (and private counters) per lane of a scoring warp
-constexpr int kHypPerLaneNarrow = 4;              // second instantiation for small hypothesis counts (see score_hpl())
-constexpr int kScoreMinBlocks = CASA_SCORE_MINB;  // resident 256-thread blocks per SM the kernel is compiled for
-constexpr int kPixUnroll = CASA_PIX_UNROLL;  // pixels per trip of the scoring loop
+constexpr int kHypPerLaneWide = 8;    // hypotheses (and private counters) per lane of a scoring warp
+constexpr int kHypPerLaneNarrow = 4;  // second instantiation for small hypothesis counts (see score_hpl())
+constexpr int kScoreMinBlocks = 2;    // resident 256-thread blocks per SM the kernel is compiled for
+constexpr int kPixUnroll = 8;         // pixels per trip of the scoring loop
 
 // Exact inlier count of one hypothesis over pixels [t0, t0+npx) of a job, whole warp cooperating.
 __device__ __noinline__ int exact_count(const uint32_t* __restrict__ pix, const float2* __restrict__ vd, int t0, int npx,
@@ -208,12 +199,11 @@ __device__ __noinline__ int exact_count(const uint32_t* __restrict__ pix, const 
 //     |t| < kappa |p| + E        (E = evaluation-error bound of that hypothesis in this chunk)
 // and only units inside it are decided by exact_inlier().  Returns the corrections to the two sign
 // counts.  A NaN hypothesis (no partner / not a filter hypothesis) never enters the band.
-#ifndef CASA_STAGE2_LOOP
 // All kChunk coefficient slots of the chunk are evaluated by one straight-line pass (4 pixels x 2 hypotheses per
 // lane, 8 independent FFMA chains, the shared-memory loads issued together; padding slots hold t = +1e30 and never
 // enter a band), the in-band units — found by 8 % of the passes — are handled afterwards, and the warp reductions
-// run only when some lane has a correction (3 % of the flagged pairs).  The previous form (-DCASA_STAGE2_LOOP)
-// looped over the pixels with a branch per iteration and was latency-bound: 9.5 % of the kernel's instructions but
+// run only when some lane has a correction (3 % of the flagged pairs).  The earlier form, a loop over the pixels
+// with a branch per iteration, was latency-bound: 9.5 % of the kernel's instructions but
 // 28 % of its warp-stall samples (profiles/r01_k_score_source_regions.txt).
 __device__ __forceinline__ int2 band_adjust2(const float4* __restrict__ cA, const float2* __restrict__ cB, int qb, int qe,
                                              float ax, float ay, float bx, float by, float ea, float eb, float kappa2,
@@ -265,43 +255,6 @@ __device__ __forceinline__ int2 band_adjust2(const float4* __restrict__ cA, cons
   if (!__any_sync(0xffffffffu, (da | db) != 0)) return make_int2(0, 0);
   return make_int2(__reduce_add_sync(0xffffffffu, da), __reduce_add_sync(0xffffffffu, db));
 }
-#else
-__device__ __forceinline__ int2 band_adjust2(const float4* __restrict__ cA, const float2* __restrict__ cB, int qb, int qe,
-                                             float ax, float ay, float bx, float by, float ea, float eb, float kappa2,
-                                             const float2* __restrict__ hfilt, int ha, int hb_ok,
-                                             const uint32_t* __restrict__ pix, const float2* __restrict__ vd, int t0,
-                                             float thr, unsigned& n_exact) {
-  const int lane = threadIdx.x & 31;
-  int da = 0, db = 0;
-  for (int q = qb + lane; q < qe; q += 32) {
-    const float4 A = cA[q];
-    const float2 B = cB[q];
-    float pa, pb;
-    const float ta = local_unit(A, B, ax, ay, pa);
-    const float tb = local_unit(A, B, bx, by, pb);
-    const bool ua = fabsf(ta) < fmaf(kappa2, fabsf(pa), ea);
-    const bool ub = fabsf(tb) < fmaf(kappa2, fabsf(pb), eb);
-    if (ua || ub) {  // ~1e-5 of the units
-      const uint32_t pk = pix[t0 + q];
-      const int x = pk & 0xFFFFu, y = pk >> 16;
-      const float2 dv = load_dir(vd, t0 + q);
-      const float nd = exact_norm(dv.x, dv.y);
-      if (ua) {
-        const float2 h = hfilt[ha];
-        da += (exact_inlier(h.x, h.y, (float)x + 0.5f, (float)y + 0.5f, dv.x, dv.y, nd, thr) ? 1 : 0) -
-              (int)(__float_as_uint(ta) >> 31);
-      }
-      if (ub && hb_ok) {
-        const float2 h = hfilt[ha + 32];
-        db += (exact_inlier(h.x, h.y, (float)x + 0.5f, (float)y + 0.5f, dv.x, dv.y, nd, thr) ? 1 : 0) -
-              (int)(__float_as_uint(tb) >> 31);
-      }
-      n_exact += (ua ? 1u : 0u) + (ub ? 1u : 0u);
-    }
-  }
-  return make_int2(__reduce_add_sync(0xffffffffu, da), __reduce_add_sync(0xffffffffu, db));
-}
-#endif
 
 // K3 — THE HOT KERNEL.  Persistent grid of independent warps; each warp pulls (job, keypoint,
 // 128-pixel chunk) items from a global counter.  No block barriers.

@@ -311,9 +311,10 @@ int casa_allgather_points_overlapped(casa_handle* h, const float* local, float* 
                                      void* after_stream, int slot);
 int casa_gather_wait(casa_handle* h, int slot, void* stream);
 
-/* Device status word of the last casa_ransac_vote on this handle (CASA_STATUS_* bits). */
+/* Device status word of the last casa_ransac_vote on this handle (CASA_STATUS_* bits); after casa_ransac_vote_host
+ * (or casa_host_wait) the OR over the image ranges of that call. */
 int casa_last_status(casa_handle* h, uint32_t* status);
-/* Number of kernels the last call launched on this handle. */
+/* Number of kernels the last call launched on this handle (casa_ransac_vote_host: all its image ranges). */
 int casa_last_launches(casa_handle* h, int64_t* launches);
 
 /*
