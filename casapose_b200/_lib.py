@@ -81,6 +81,8 @@ EXPORTS = {
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "casa_pnp": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                            C.c_void_p]),
+    "casa_pnp_backward": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                    C.c_void_p, C.c_void_p, C.c_void_p]),
     "casa_pose_errors": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
     "casa_set_async": (C.c_int, [C.c_void_p, C.c_int]),

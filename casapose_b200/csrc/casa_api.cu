@@ -1896,6 +1896,23 @@ extern "C" int casa_pnp(casa_handle* h, int32_t n, int32_t vn, const float* poin
   return CASA_OK;
 }
 
+extern "C" int casa_pnp_backward(casa_handle* h, int32_t n, int32_t vn, const float* points3d, const float* camera,
+                                 const float* poses, int32_t pose_form, const float* grad_poses, float* grad_points2d,
+                                 void* stream) {
+  if (!h) return fail(CASA_ERR_INVALID, "handle is NULL");
+  if (!points3d || !camera || !poses || !grad_poses || !grad_points2d)
+    return fail(CASA_ERR_INVALID, "points3d / camera / poses / grad_poses / grad_points2d must not be NULL");
+  if (n < 0 || vn < 6 || vn > 16) return fail(CASA_ERR_INVALID, "n=%d, vn=%d: need n >= 0 and 6 <= vn <= 16", n, vn);
+  if (pose_form != 6 && pose_form != 12) return fail(CASA_ERR_INVALID, "pose_form=%d: need 6 (rvec, tvec) or 12 ([R|t])", pose_form);
+  if (n == 0) return CASA_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  k_pnp_backward<<<(n + 3) / 4, 128, 0, (cudaStream_t)stream>>>(n, vn, pose_form, points3d, camera, poses, grad_poses,
+                                                                grad_points2d);
+  CUDA_TRY(cudaGetLastError());
+  h->last_launches = 1;
+  return CASA_OK;
+}
+
 extern "C" int casa_pose_errors(casa_handle* h, int32_t n, int32_t m, int32_t maxp, const float* poses, const float* poses_gt,
                                 const float* camera, const float* model_points, const int32_t* model_counts,
                                 const int32_t* obj_model, const float* diameters, const int32_t* valid,

@@ -502,4 +502,165 @@ __global__ void __launch_bounds__(128) k_pnp(PnpParams pp, const float* __restri
   }
 }
 
+// K10 — backward of PnP, BPnP_fast (Chen et al., CVPR 2020; the reference's bpnp_layers.py:138-277).
+// The pose y is differentiated through the stationarity condition f(x, y) = C^T (pi(y) - x) = 0 with
+// C = -2 dpi/dy detached at the forward pose, so that with J = dpi/dy (2vn x 6)
+//   dy/dx = (J^T J)^-1 J^T   and   grad_x = J (J^T J)^-1 grad_y.
+// J does not depend on the observed points x, and the result does not depend on how the rotation is parameterised:
+// y is taken as the left-multiplicative tangent of pnp_lm (R <- exp([w]x) R, t <- t + dt), and the incoming gradient
+// is mapped onto it.
+//   pose_form 12: poses [n,3,4] = [R|t] as written by k_pnp / poses_pnp.  A t_z < 0 flip (-[R|t], ransac_voting.py:53-55)
+//                 is recognised by det(R) < 0: the un-flipped pose is differentiated with the incoming gradient negated.
+//                 g_w = vee(A - A^T) with A = G_R R^T, g_t = G_t.
+//   pose_form 6:  poses [n,6] = (rvec, tvec) as returned by BPNP_fast; g_w = Jl(rvec)^-T g_rvec, where Jl is the left
+//                 Jacobian of SO(3) (exp(r + dr) = exp([Jl dr]x) exp(r)), and g_t = g_tvec.
+// Guards, each giving an exact zero gradient for the object instead of NaN / inf:
+//   * an all-zero pose (dead object, failed solve, available = 0);
+//   * a point at z <= 0 under the differentiated (un-flipped) pose, or any non-finite entry of J or of Jl^-T;
+//   * a Cholesky pivot of J^T J that is not above kPnpPivotRtol times its diagonal entry (rank-deficient J, e.g.
+//     collinear keypoints; the reference's torch.inverse would fail or return inf there).
+// One warp per object, one lane per row of J (point i = lane / 2, coordinate lane % 2); the 21 entries of J^T J are
+// warp-reduced and every lane factors the 6x6 system itself.  float64 inside, float32 in and out.
+constexpr double kPnpPivotRtol = 1e-10;  // pivot^2 / diagonal; collinear float32 keypoints give ~1e-14
+
+__global__ void __launch_bounds__(128) k_pnp_backward(int n, int vn, int pose_form, const float* __restrict__ pts3d,
+                                                     const float* __restrict__ cam, const float* __restrict__ poses,
+                                                     const float* __restrict__ grad_poses, float* __restrict__ grad2d) {
+  const int obj = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (obj >= n) return;
+  const int np = pose_form;  // floats per pose
+  const float* P = poses + (size_t)obj * np;
+  const float* Gp = grad_poses + (size_t)obj * np;
+  bool dead = true;
+  for (int k = 0; k < np; ++k) dead = dead && P[k] == 0.f;
+  bool ok = !dead;
+  double R[9], t[3], gw[3], gt[3];
+  if (pose_form == 12) {
+    for (int r = 0; r < 3; ++r) {
+      for (int c = 0; c < 3; ++c) R[3 * r + c] = P[4 * r + c];
+      t[r] = P[4 * r + 3];
+    }
+    const double sg = mat3_det(R) < 0 ? -1.0 : 1.0;
+    double G[9];
+    for (int r = 0; r < 3; ++r) {
+      for (int c = 0; c < 3; ++c) {
+        R[3 * r + c] *= sg;
+        G[3 * r + c] = sg * Gp[4 * r + c];
+      }
+      t[r] *= sg;
+      gt[r] = sg * Gp[4 * r + 3];
+    }
+    double A[9];  // A = G_R R^T
+    for (int r = 0; r < 3; ++r)
+      for (int c = 0; c < 3; ++c) A[3 * r + c] = G[3 * r] * R[3 * c] + G[3 * r + 1] * R[3 * c + 1] + G[3 * r + 2] * R[3 * c + 2];
+    gw[0] = A[7] - A[5];
+    gw[1] = A[2] - A[6];
+    gw[2] = A[3] - A[1];
+  } else {
+    const double rv[3] = {P[0], P[1], P[2]}, gr[3] = {Gp[0], Gp[1], Gp[2]};
+    for (int k = 0; k < 3; ++k) {
+      t[k] = P[3 + k];
+      gt[k] = Gp[3 + k];
+    }
+    // R = exp([r]x) = I + a K + b K^2 (Rodrigues, like so3_exp) from the half angle: a = 2 sh ch / th, b = 2 sh^2 / th^2.
+    // Jl^-1 = I - [r]x / 2 + c [r]x^2, so Jl^-T g = g + r x g / 2 + c r x (r x g), c = 1/th^2 - cot(th/2) / (2 th)
+    // (series below th = 1e-2; infinite at th = 2 pi, where the guard applies).  sincospi needs no argument-reduction
+    // scratch in local memory, unlike sin / cos.
+    const double th2 = rv[0] * rv[0] + rv[1] * rv[1] + rv[2] * rv[2], th = sqrt(th2);
+    double sh, ch;
+    sincospi(th * 0.15915494309189535, &sh, &ch);  // th / (2 pi)
+    const double a = th < 1e-12 ? 1.0 : 2.0 * sh * ch / th, b = th < 1e-12 ? 0.5 : 2.0 * sh * sh / th2;
+    const double x = rv[0], y = rv[1], z = rv[2];
+    R[0] = 1.0 - b * (y * y + z * z); R[1] = -a * z + b * x * y;       R[2] = a * y + b * x * z;
+    R[3] = a * z + b * x * y;         R[4] = 1.0 - b * (x * x + z * z); R[5] = -a * x + b * y * z;
+    R[6] = -a * y + b * x * z;        R[7] = a * x + b * y * z;         R[8] = 1.0 - b * (x * x + y * y);
+    const double cf = th2 < 1e-4 ? 1.0 / 12.0 + th2 * (1.0 / 720.0 + th2 / 30240.0) : 1.0 / th2 - ch / (2.0 * th * sh);
+    const double rg[3] = {rv[1] * gr[2] - rv[2] * gr[1], rv[2] * gr[0] - rv[0] * gr[2], rv[0] * gr[1] - rv[1] * gr[0]};
+    const double rrg[3] = {rv[1] * rg[2] - rv[2] * rg[1], rv[2] * rg[0] - rv[0] * rg[2], rv[0] * rg[1] - rv[1] * rg[0]};
+    for (int k = 0; k < 3; ++k) gw[k] = gr[k] + 0.5 * rg[k] + cf * rrg[k];
+    ok = ok && isfinite(cf);
+  }
+  // this lane's row of J
+  const int pt = lane >> 1, coord = lane & 1;
+  double Jr[6] = {0, 0, 0, 0, 0, 0};
+  if (ok && pt < vn) {
+    const float* Kf = cam + (size_t)obj * 9;
+    const double f = coord ? Kf[4] : Kf[0];
+    const float* Xf = pts3d + ((size_t)obj * vn + pt) * 3;
+    const double X0 = Xf[0], X1 = Xf[1], X2 = Xf[2];
+    const double rx = R[0] * X0 + R[1] * X1 + R[2] * X2, ry = R[3] * X0 + R[4] * X1 + R[5] * X2,
+                 rz = R[6] * X0 + R[7] * X1 + R[8] * X2;
+    const double z = rz + t[2], iz = 1.0 / z;
+    // d pi_coord / d Xc = (f/z, 0, -f x/z^2) or (0, f/z, -f y/z^2); d Xc / d w = -[RX]x, so the w-part is RX x d
+    const double d0 = coord ? 0.0 : f * iz, d1 = coord ? f * iz : 0.0, d2 = -f * (coord ? ry + t[1] : rx + t[0]) * iz * iz;
+    Jr[0] = ry * d2 - rz * d1;
+    Jr[1] = rz * d0 - rx * d2;
+    Jr[2] = rx * d1 - ry * d0;
+    Jr[3] = d0;
+    Jr[4] = d1;
+    Jr[5] = d2;
+    bool good = z > 0;
+#pragma unroll
+    for (int a = 0; a < 6; ++a) good = good && isfinite(Jr[a]);
+    ok = good;
+  }
+  ok = __all_sync(0xffffffffu, ok);
+  // J^T J (lower triangle, row-major packed) summed over the warp
+  double H[21];
+  {
+    int k = 0;
+#pragma unroll
+    for (int a = 0; a < 6; ++a)
+#pragma unroll
+      for (int b = 0; b <= a; ++b) H[k++] = Jr[a] * Jr[b];
+  }
+#pragma unroll
+  for (int o = 16; o; o >>= 1)
+#pragma unroll
+    for (int k = 0; k < 21; ++k) H[k] += __shfl_xor_sync(0xffffffffu, H[k], o);
+  // Cholesky H = L L^T in place, with the relative pivot test (fixed loop bounds so that H stays in registers)
+#pragma unroll
+  for (int j = 0; j < 6; ++j) {
+    const int jj = j * (j + 1) / 2;
+    double s = H[jj + j];
+#pragma unroll
+    for (int k = 0; k < 6; ++k)
+      if (k < j) s -= H[jj + k] * H[jj + k];
+    ok = ok && s > kPnpPivotRtol * H[jj + j];
+    const double l = sqrt(fmax(s, 1e-300));
+    H[jj + j] = l;
+#pragma unroll
+    for (int i = 0; i < 6; ++i) {
+      if (i <= j) continue;
+      const int ii = i * (i + 1) / 2;
+      double v = H[ii + j];
+#pragma unroll
+      for (int k = 0; k < 6; ++k)
+        if (k < j) v -= H[ii + k] * H[jj + k];
+      H[ii + j] = v / l;
+    }
+  }
+  // s = H^-1 g_y: L u = g, L^T s = u
+  double sv[6] = {gw[0], gw[1], gw[2], gt[0], gt[1], gt[2]};
+#pragma unroll
+  for (int i = 0; i < 6; ++i) {
+    const int ii = i * (i + 1) / 2;
+#pragma unroll
+    for (int k = 0; k < 6; ++k)
+      if (k < i) sv[i] -= H[ii + k] * sv[k];
+    sv[i] /= H[ii + i];
+  }
+#pragma unroll
+  for (int i = 5; i >= 0; --i) {
+#pragma unroll
+    for (int k = 0; k < 6; ++k)
+      if (k > i) sv[i] -= H[k * (k + 1) / 2 + i] * sv[k];
+    sv[i] /= H[i * (i + 1) / 2 + i];
+  }
+  double g = 0;
+#pragma unroll
+  for (int a = 0; a < 6; ++a) g += Jr[a] * sv[a];
+  if (pt < vn) grad2d[(size_t)obj * 2 * vn + lane] = ok ? (float)g : 0.f;
+}
+
 }  // namespace casa

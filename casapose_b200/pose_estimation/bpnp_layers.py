@@ -1,7 +1,11 @@
-"""Forward pass of the reference's BPnP layer (/root/reference/casapose/pose_estimation/bpnp_layers.py:86-135,
-278-359).  Host-side OpenCV like the reference (tf.numpy_function, :322).  The implicit-function-theorem
-backward (:138-277) is a training-only gradient and out of scope."""
+"""The reference's BPnP layer (/root/reference/casapose/pose_estimation/bpnp_layers.py:86-135, 278-359).  The forward
+is host-side OpenCV like the reference (tf.numpy_function, :322).  The implicit-function-theorem backward of BPnP_fast
+(:138-277) is casa_pnp_backward on the GPU: it is routed through torch.autograd when the 2-D points are a CUDA tensor
+that requires grad."""
 import numpy as np
+import torch
+
+from .ransac_voting import PnpGradFn, wants_grad
 
 
 def pnp(points_3d, points_2d, camera_matrix, init_pose=None):
@@ -48,7 +52,11 @@ def rodrigues_batch(rvecs):
 
 
 class BPNP_fast:
-    """Forward-only stand-in for the Keras layer: layer([pts2d, pts3d, K]) -> [n, 6] (rvec, tvec)."""
+    """Stand-in for the Keras layer: layer([pts2d, pts3d, K]) -> [n, 6] (rvec, tvec), or [b, oc, 6] for [b, oc, vn, 2]
+    points.  pts2d as numpy (or a tensor that needs no gradient) gives the numpy result of the host solve.  pts2d as a
+    CUDA tensor that requires grad gives the same values as a float32 torch tensor on that device, whose backward is
+    casa_pnp_backward (pose_form 6, BPnP_fast: bpnp_layers.py:138-277).  The gradient w.r.t. pts3d, K and the initial
+    pose is not computed."""
 
     def __init__(self, name):
         self.name = name
@@ -56,6 +64,12 @@ class BPNP_fast:
     def __call__(self, inputs, **kwargs):
         pts2d, pts3d, K = inputs[:3]
         init = inputs[3] if len(inputs) == 4 else None
+        if wants_grad(pts2d):
+            return self._differentiable(pts2d, pts3d, K, init)
+        return self._solve(pts2d, pts3d, K, init)
+
+    @staticmethod
+    def _solve(pts2d, pts3d, K, init):
         pts2d = np.asarray(pts2d, np.float32)
         pts3d = np.asarray(pts3d, np.float32)
         shape2d = pts2d.shape
@@ -69,3 +83,27 @@ class BPNP_fast:
         if len(shape2d) == 4:
             out = out.reshape(-1, shape2d[1], 6)
         return out
+
+    def _differentiable(self, pts2d, pts3d, K, init):
+        if not pts2d.is_cuda:
+            raise ValueError("BPNP_fast: the gradient runs on the GPU (casa_pnp_backward); pts2d must be a CUDA tensor")
+
+        def host(x):
+            return x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else x
+
+        dev = pts2d.device
+        shape2d = tuple(pts2d.shape)
+        vn = shape2d[-2]
+        q = pts2d.to(torch.float32).reshape(-1, vn, 2)
+        n = q.shape[0]
+        p3 = np.asarray(host(pts3d), np.float32)
+        p3 = np.broadcast_to(p3, (n, vn, 3)) if p3.ndim == 2 else p3.reshape(-1, vn, 3)[:n]
+        p3 = torch.from_numpy(np.ascontiguousarray(p3)).to(dev)
+        cam = torch.from_numpy(np.ascontiguousarray(np.broadcast_to(np.asarray(host(K), np.float32), (n, 3, 3)))).to(dev)
+        init = None if init is None else host(init)
+
+        def solve(d):
+            return torch.from_numpy(self._solve(d.reshape(shape2d).cpu().numpy(), host(pts3d), host(K), init).reshape(n, 6)).to(dev)
+
+        out = PnpGradFn.apply(q, solve, p3, cam, 6)
+        return out.reshape(shape2d[0], shape2d[1], 6) if len(shape2d) == 4 else out

@@ -8,7 +8,7 @@ import numpy as np
 import torch
 
 from .bpnp_layers import BPNP_fast, rodrigues_batch
-from .ransac_voting import _np, estimate_poses, evaluate_poses, ransac_voting_layer_all_masks
+from .ransac_voting import PnpGradFn, _np, estimate_poses, evaluate_poses, ransac_voting_layer_all_masks, wants_grad
 
 
 def _vote_from_scores(output_seg, output_vertex, oc, vc, min_num, **vote_kw):
@@ -75,11 +75,28 @@ def evaluate_pose_estimates(points_estimated, poses, poses_gt, target_seg, objec
              false_positive_pose], poses, points_estimated)
 
 
+def _host_poses(pts, obj3d, cam):
+    """pose_evaluation.py:199-212 before the availability mask: BPNP_fast (OpenCV), Rodrigues, t_z flip -> [n,3,4]."""
+    poses6 = BPNP_fast(name="BPNP")([np.ascontiguousarray(pts), obj3d, cam])  # :199
+    if not np.isfinite(poses6).all():  # :201-206
+        raise FloatingPointError("Tensor had inf or nan values: %r" % (poses6,))
+    R = rodrigues_batch(poses6[:, 0:3])  # :208
+    T = poses6[:, 3:6][..., None]  # :209
+    poses = np.concatenate([R, T], axis=-1)
+    return np.where(T[:, 2:3, :] < 0, -poses, poses)  # :212
+
+
 def poses_pnp(points_estimated, seg_estimated, object_points_3d, camera_data, no_objects, min_num=20, pnp_backend="cv2"):
-    """pose_evaluation.py:164-217: LS-layer output (y,x) -> PnP -> [b,oc,1,3,4].  pnp_backend="cuda": casa_pnp."""
+    """pose_evaluation.py:164-217: LS-layer output (y,x) -> PnP -> [b,oc,1,3,4].  pnp_backend="cuda": casa_pnp.
+    If points_estimated is a CUDA tensor that requires grad, the (CPU) result is differentiable w.r.t. it with either
+    backend: the backward is casa_pnp_backward on the returned [R|t] (BPnP_fast, bpnp_layers.py:138-277).  The forward
+    values are those of the call without grad."""
     b, h, w, _ = seg_estimated.shape
     oc, ic = no_objects, 1
     _, _, _, vc, _ = object_points_3d.shape
+    grad = wants_grad(points_estimated)
+    if grad and not points_estimated.is_cuda:
+        raise ValueError("poses_pnp: the gradient runs on the GPU (casa_pnp_backward); points_estimated must be a CUDA tensor")
     pts = _np(points_estimated, np.float32).reshape(-1, vc, 2)[:, :, ::-1]  # (y,x) -> (x,y) :179
     obj3d = _np(object_points_3d, np.float32).reshape(-1, vc, 3)
     seg = seg_estimated if isinstance(seg_estimated, torch.Tensor) else torch.as_tensor(np.asarray(seg_estimated))
@@ -87,22 +104,30 @@ def poses_pnp(points_estimated, seg_estimated, object_points_3d, camera_data, no
     count = (hot > 0.1).sum(dim=(1, 2))  # :186-188
     available = (count > min_num).to(torch.float32).reshape(-1, 1, 1).cpu().numpy()  # :190-197
     cam = _np(camera_data, np.float32)[0]
+    n = pts.shape[0]
+    if grad:  # the same steps as torch ops on the device, so that autograd can route dL/d poses to points_estimated
+        dev = points_estimated.device
+        q = points_estimated.to(torch.float32).reshape(-1, vc, 2).flip(-1)  # :179
+        av = torch.from_numpy(available).to(dev)
     if pnp_backend == "cuda":
         from .ransac_voting import pnp_cuda
 
-        n = pts.shape[0]
-        poses = pnp_cuda(np.ascontiguousarray(pts), np.broadcast_to(obj3d, (n,) + obj3d.shape[1:]) if obj3d.shape[0] == n
-                         else np.tile(obj3d, (n // obj3d.shape[0], 1, 1)), np.broadcast_to(cam, (n, 3, 3))).cpu().numpy()
+        p3 = np.broadcast_to(obj3d, (n,) + obj3d.shape[1:]) if obj3d.shape[0] == n else np.tile(obj3d, (n // obj3d.shape[0], 1, 1))
+        if grad:
+            return (pnp_cuda(q, p3, np.broadcast_to(cam, (n, 3, 3))) * av).reshape(b, oc, ic, 3, 4).cpu()
+        poses = pnp_cuda(np.ascontiguousarray(pts), p3, np.broadcast_to(cam, (n, 3, 3))).cpu().numpy()
         return torch.from_numpy((poses * available).reshape(b, oc, ic, 3, 4).astype(np.float32))
     if pnp_backend != "cv2":
         raise ValueError("pnp_backend must be 'cv2' or 'cuda'")
-    poses6 = BPNP_fast(name="BPNP")([np.ascontiguousarray(pts), obj3d, cam])  # :199
-    if not np.isfinite(poses6).all():  # :201-206
-        raise FloatingPointError("Tensor had inf or nan values: %r" % (poses6,))
-    R = rodrigues_batch(poses6[:, 0:3])  # :208
-    T = poses6[:, 3:6][..., None]  # :209
-    poses = np.concatenate([R, T], axis=-1)
-    poses = np.where(T[:, 2:3, :] < 0, -poses, poses)  # :212
+    if grad:
+        p3 = torch.from_numpy(np.ascontiguousarray(obj3d[:n])).to(dev)
+        cam_t = torch.from_numpy(np.ascontiguousarray(np.broadcast_to(cam, (n, 3, 3)))).to(dev)
+
+        def solve(d):
+            return torch.from_numpy(np.ascontiguousarray(_host_poses(d.cpu().numpy(), obj3d, cam), np.float32)).to(dev)
+
+        return (PnpGradFn.apply(q, solve, p3, cam_t, 12) * av).reshape(b, oc, ic, 3, 4).cpu()
+    poses = _host_poses(pts, obj3d, cam)
     poses = poses * available  # :213
     return torch.from_numpy(poses.reshape(b, oc, ic, 3, 4).astype(np.float32))
 

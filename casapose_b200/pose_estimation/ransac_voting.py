@@ -281,25 +281,80 @@ def project(xyz, K, RT):
     return xy.astype(f), xyz_proj.astype(f)
 
 
+def wants_grad(x):
+    """True if `x` is a torch tensor that autograd would differentiate here."""
+    return isinstance(x, torch.Tensor) and x.requires_grad and torch.is_grad_enabled()
+
+
+def pnp_backward_cuda(points_3d, camera_matrixes, poses, grad_poses, pose_form):
+    """casa_pnp_backward: dL/d points_2d [n,vn,2] (x,y) for dL/d poses = grad_poses, the BPnP_fast gradient
+    (bpnp_layers.py:138-277).  points_3d [n,vn,3], camera_matrixes [n,3,3], poses / grad_poses [n,3,4] (pose_form 12,
+    [R|t]) or [n,6] (pose_form 6, (rvec, tvec)); all float32 on one CUDA device."""
+    p3 = as_cuda_f32(points_3d, "points_3d")
+    cam = as_cuda_f32(camera_matrixes, "camera_matrixes")
+    poses = as_cuda_f32(poses, "poses")
+    grad_poses = as_cuda_f32(grad_poses.contiguous(), "grad_poses")
+    n, vn = p3.shape[0], p3.shape[1]
+    if tuple(poses.shape) != tuple(grad_poses.shape) or poses.numel() != n * pose_form or tuple(cam.shape) != (n, 3, 3):
+        raise ValueError("pnp_backward_cuda: poses / grad_poses must hold %d x %d floats and camera_matrixes be [%d,3,3]"
+                         % (n, pose_form, n))
+    dev = p3.device
+    out = torch.empty((n, vn, 2), dtype=torch.float32, device=dev)
+    hdl = _lib.handle(dev.index if dev.index is not None else torch.cuda.current_device(), current_stream_ptr(dev))
+    with torch.cuda.device(dev):
+        rc = _lib.lib().casa_pnp_backward(hdl, n, vn, ptr(p3), ptr(cam), ptr(poses), int(pose_form), ptr(grad_poses),
+                                          ptr(out), current_stream_ptr(dev))
+    _lib.check(rc)
+    return out
+
+
+class PnpGradFn(torch.autograd.Function):
+    """torch.autograd carrier of a PnP solve whose backward is casa_pnp_backward.  `solve(points_2d)` runs the forward
+    (the GPU kernel or the host OpenCV sequence) on the detached points and returns the poses on the points' device;
+    PyTorch only routes the gradient."""
+
+    @staticmethod
+    def forward(ctx, points_2d, solve, points_3d, camera_matrixes, pose_form):
+        poses = solve(points_2d.detach())
+        ctx.pose_form = pose_form
+        ctx.save_for_backward(points_3d, camera_matrixes, poses)
+        return poses
+
+    @staticmethod
+    def backward(ctx, grad_poses):
+        p3, cam, poses = ctx.saved_tensors
+        g = pnp_backward_cuda(p3, cam, poses, grad_poses, ctx.pose_form)
+        return g, None, None, None, None
+
+
 def pnp_cuda(points_2d, points_3d, camera_matrixes, offsets=None):
     """Batched GPU PnP (casa_pnp): points_2d [n,vn,2] (x,y), points_3d [n,vn,3], camera_matrixes [n,3,3],
     offsets [n,10] or None -> poses [n,3,4] float32 on the device of points_2d.  Same guards and sign
-    convention as `pnp` / map_offsets / map_pnp (ransac_voting.py:13-57, 487-514)."""
+    convention as `pnp` / map_offsets / map_pnp (ransac_voting.py:13-57, 487-514).
+    If points_2d is a CUDA tensor that requires grad, the poses carry a grad_fn whose backward is casa_pnp_backward
+    (BPnP_fast, bpnp_layers.py:138-277); differentiating through `offsets` is not supported (ValueError)."""
     dev = points_2d.device if isinstance(points_2d, torch.Tensor) and points_2d.is_cuda else torch.device("cuda", torch.cuda.current_device())
 
     def put(x):
         t = x if isinstance(x, torch.Tensor) else torch.as_tensor(np.ascontiguousarray(np.asarray(x, np.float32)))
         return t.to(device=dev, dtype=torch.float32).contiguous()
 
-    p2, p3, cam = put(points_2d), put(points_3d), put(camera_matrixes)
+    grad = wants_grad(points_2d) and points_2d.is_cuda
+    if grad and offsets is not None:
+        raise ValueError("pnp_cuda: no gradient through the offsets un-mapping; pass offsets=None or detached points")
+    p2, p3, cam = put(points_2d), put(points_3d).detach(), put(camera_matrixes).detach()
     off = put(offsets) if offsets is not None else None
-    n, vn = p2.shape[0], p2.shape[1]
-    out = torch.empty((n, 3, 4), dtype=torch.float32, device=dev)
-    hdl = _lib.handle(dev.index if dev.index is not None else torch.cuda.current_device(), current_stream_ptr(dev))
-    with torch.cuda.device(dev):
-        rc = _lib.lib().casa_pnp(hdl, n, vn, ptr(p2), ptr(p3), ptr(cam), ptr(off), ptr(out), current_stream_ptr(dev))
-    _lib.check(rc)
-    return out
+
+    def solve(q):
+        n, vn = q.shape[0], q.shape[1]
+        out = torch.empty((n, 3, 4), dtype=torch.float32, device=dev)
+        hdl = _lib.handle(dev.index if dev.index is not None else torch.cuda.current_device(), current_stream_ptr(dev))
+        with torch.cuda.device(dev):
+            rc = _lib.lib().casa_pnp(hdl, n, vn, ptr(q), ptr(p3), ptr(cam), ptr(off), ptr(out), current_stream_ptr(dev))
+        _lib.check(rc)
+        return out
+
+    return PnpGradFn.apply(p2, solve, p3, cam, 12) if grad else solve(p2)
 
 
 def estimate_poses(points, keypoints, camera_matrixes, valid_points_filter, offsets, pnp_backend="cv2"):

@@ -228,6 +228,23 @@ int casa_pnp(casa_handle* h, int32_t n, int32_t vn, const float* points2d, const
              const float* camera, const float* offsets, float* poses, void* stream);
 
 /*
+ * Backward of PnP w.r.t. the 2-D points — the "fast" implicit-function gradient of the reference's BPnP layer
+ * (/root/reference/casapose/pose_estimation/bpnp_layers.py:138-277, Chen et al., CVPR 2020):
+ * grad_points2d = J (J^T J)^-1 grad_y, J = d projection / d pose at the given pose (Gauss-Newton Hessian, no
+ * residual-curvature terms), so the gradient depends on the pose, the 3-D points and the camera only.
+ *   points3d   device float32 [n,vn,3]           camera device float32 [n,3,3] (zero skew)
+ *   poses      device float32 [n,3,4] [R|t] (pose_form 12: what casa_pnp / poses_pnp write; a t_z < 0 flip, -[R|t],
+ *              is recognised by det(R) < 0) or [n,6] (rvec, tvec) (pose_form 6: what BPNP_fast returns)
+ *   grad_poses device float32, same shape as poses: dL/d poses
+ *   grad_points2d device float32 [n,vn,2] (x,y), written densely
+ * An object gets an exact zero gradient if its pose is all zero, if a point lies at z <= 0 under the (un-flipped)
+ * pose, or if J^T J is numerically singular (e.g. collinear points).  vn in 6..16; n == 0 is a no-op.  One kernel,
+ * no workspace, no synchronisation: asynchronous on `stream` and usable inside a captured graph.
+ */
+int casa_pnp_backward(casa_handle* h, int32_t n, int32_t vn, const float* points3d, const float* camera,
+                      const float* poses, int32_t pose_form, const float* grad_poses, float* grad_points2d, void* stream);
+
+/*
  * ADD / ADD-S / 2-D reprojection errors of a batch of poses (SURVEY.md 8f-3).  Stands in for the reference's
  * map_estimates + evaluate_poses (/root/reference/casapose/pose_estimation/ransac_voting.py:561-625, 628-687):
  * per object one row [err_2d, err_3d, valid_3d, valid_2d, missing, false_positive]; the caller sums rows over
