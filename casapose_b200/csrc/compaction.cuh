@@ -399,21 +399,23 @@ __global__ void __launch_bounds__(256) k_gather_dirs(const float* __restrict__ v
   const int nwarps = gridDim.x * 8;
   for (int base = (blockIdx.x * 8 + warp) * 32; base < tn; base += nwarps * 32) {
     const int t = base + lane;  // lane l owns list position base + l
-    int rowoff = -1;            // float offset of the pixel's row inside the image's field
+    int px = -1;                // the pixel's index in the image (< 2^30)
     if (t < tn) {
       const uint32_t pk = pix[t];
-      rowoff = (int)((pk >> 16) * (uint32_t)d.w + (pk & 0xFFFFu)) * vslots * 2;
+      px = (int)((pk >> 16) * (uint32_t)d.w + (pk & 0xFFFFu));
     }
     // flattened fetch: element e = lane + 32 k of the warp's [32 pixels x rowf floats] block.  Consecutive
     // lanes read consecutive floats of one row and run on into the next pixel's row, which is contiguous in
     // memory whenever the two pixels are neighbours — so most warp-loads are one full 128-byte line, and all
-    // rowf loads of a lane are independent (no per-pixel serialisation).
+    // rowf loads of a lane are independent (no per-pixel serialisation).  The row offset px * vn * vpc * 2 is
+    // formed in 64 bits: it reaches 2^31 from pixel 2^26 on for a shared field with vn = 16, and from pixel 2^21
+    // on for 32 per-class fields with vn = 16.
 #pragma unroll 6
     for (int k = 0; k < rowf; ++k) {
       const int e = k * 32 + lane;
       const int src = e / rowf, f = e - src * rowf;
-      const int ro = __shfl_sync(0xffffffffu, rowoff, src);
-      if (ro >= 0) srow[warp][src][f] = __ldg(vfield + ro + f);
+      const int sp = __shfl_sync(0xffffffffu, px, src);
+      if (sp >= 0) srow[warp][src][f] = __ldg(vfield + (size_t)sp * (vslots * 2) + f);
     }
     __syncwarp();
     if (t < tn)
