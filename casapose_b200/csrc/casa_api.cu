@@ -1947,7 +1947,8 @@ extern "C" int casa_pose_errors(casa_handle* h, int32_t n, int32_t m, int32_t ma
                                                cloud_gt, cloud_est, base, state, out_rows);
   int launches = 1;
   if (may_sym) {
-    k_adds_min<<<dim3(tiles, n), kMetricThreads, 0, st>>>(pp, model_counts, obj_model, state, cloud_gt, cloud_est, partial);
+    k_adds_min<<<dim3(tiles, min(n, kAddsGridY)), kMetricThreads, 0, st>>>(pp, tiles, model_counts, obj_model, state, cloud_gt,
+                                                                          cloud_est, partial);
     ++launches;
   }
   k_pose_finalize<<<(n + 127) / 128, 128, 0, st>>>(pp, tiles, model_counts, obj_model, state, base, partial, diameters, out_rows);

@@ -7,8 +7,8 @@
 // bit for bit; what is reproduced is its structure — a robust initial pose from point subsets, then the
 // Levenberg-Marquardt minimum of the reprojection error over all points, which is what the reference returns:
 //   * candidates: the full point set, every leave-one-out and every leave-two-out subset (46 for 9 points);
-//     each is solved by a normalised DLT (reduced to a 4x4 symmetric eigen-problem), projected on SO(3) by a polar
-//     iteration and polished by 5 LM steps; the candidate with the most points inside 12 px (cv2's
+//     each is solved by a normalised DLT (reduced to a 4x4 symmetric eigen-problem, or 3x3 for coplanar points),
+//     projected on SO(3) by a polar iteration and polished by 5 LM steps; the candidate with the most points inside 12 px (cv2's
 //     reprojectionError), then the smallest inlier cost, wins;
 //   * final: LM over all points from the winner, float64 throughout.
 // One warp per object, lanes = candidates.  oracle/pnp_np.py is the numpy restatement of this algorithm;
@@ -54,8 +54,9 @@ __device__ __forceinline__ void so3_exp(const double* w, double* E) {
   E[6] = -a * y + b * x * z;        E[7] = a * x + b * y * z;         E[8] = 1.0 - b * (x * x + y * y);
 }
 
-// smallest-eigenvalue eigenvector of the symmetric 4x4 matrix A (destroyed), cyclic Jacobi
-__device__ __forceinline__ void jacobi4_smallest(double (&A)[4][4], double (&vec)[4]) {
+// smallest-eigenvalue eigenvector of the symmetric DxD matrix A (destroyed; D = 4 or 3 in the leading block), cyclic Jacobi
+template <int D>
+__device__ __forceinline__ void jacobi_smallest(double (&A)[4][4], double (&vec)[4]) {
   double V[4][4];
 #pragma unroll
   for (int i = 0; i < 4; ++i)
@@ -64,35 +65,35 @@ __device__ __forceinline__ void jacobi4_smallest(double (&A)[4][4], double (&vec
   for (int sweep = 0; sweep < 30; ++sweep) {
     double off = 0.0, diag = 0.0;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < D; ++i) {
       diag += A[i][i] * A[i][i];
 #pragma unroll
-      for (int j = i + 1; j < 4; ++j) off += A[i][j] * A[i][j];
+      for (int j = i + 1; j < D; ++j) off += A[i][j] * A[i][j];
     }
     if (off <= 1e-30 * diag || off == 0.0) break;
 #pragma unroll
-    for (int p = 0; p < 3; ++p)
+    for (int p = 0; p < D - 1; ++p)
 #pragma unroll
-      for (int q = p + 1; q < 4; ++q) {
+      for (int q = p + 1; q < D; ++q) {
         const double apq = A[p][q];
         if (fabs(apq) < 1e-300) continue;
         const double theta = (A[q][q] - A[p][p]) / (2.0 * apq);
         const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
         const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {  // columns p, q
+        for (int k = 0; k < D; ++k) {  // columns p, q
           const double akp = A[k][p], akq = A[k][q];
           A[k][p] = c * akp - s * akq;
           A[k][q] = s * akp + c * akq;
         }
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {  // rows p, q
+        for (int k = 0; k < D; ++k) {  // rows p, q
           const double apk = A[p][k], aqk = A[q][k];
           A[p][k] = c * apk - s * aqk;
           A[q][k] = s * apk + c * aqk;
         }
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
+        for (int k = 0; k < D; ++k) {
           const double vkp = V[k][p], vkq = V[k][q];
           V[k][p] = c * vkp - s * vkq;
           V[k][q] = s * vkp + c * vkq;
@@ -101,17 +102,106 @@ __device__ __forceinline__ void jacobi4_smallest(double (&A)[4][4], double (&vec
   }
   int best = 0;
 #pragma unroll
-  for (int i = 1; i < 4; ++i)
+  for (int i = 1; i < D; ++i)
     if (A[i][i] < A[best][best]) best = i;
 #pragma unroll
   for (int k = 0; k < 4; ++k) vec[k] = best == 0 ? V[k][0] : best == 1 ? V[k][1] : best == 2 ? V[k][2] : V[k][3];
 }
 
+// Schur reduction of the DLT normal equations in the leading DxD block (D = 4: the 3x4 projection of general points,
+// D = 3: the homography of coplanar points).  For fixed last row h3 the optimum is h1 = S^-1 Sx h3, h2 = S^-1 Sy h3,
+// and h3 is the smallest eigenvector of M = Sq - Sx S^-1 Sx - Sy S^-1 Sy.  Rows go to p[0..D), p[4..4+D), p[8..8+D).
+// False when a Cholesky pivot of S is not above 1e-14 times its diagonal entry (S singular for this D).
+template <int D>
+__device__ __forceinline__ bool dlt_reduce(const double (&S)[4][4], const double (&Sx)[4][4], const double (&Sy)[4][4],
+                                           const double (&Sq)[4][4], double (&p)[12]) {
+  double L[4][4];
+#pragma unroll
+  for (int j = 0; j < D; ++j) {
+    double d = S[j][j];
+#pragma unroll
+    for (int k = 0; k < j; ++k) d -= L[j][k] * L[j][k];
+    if (!(d > 1e-14 * S[j][j])) return false;
+    L[j][j] = sqrt(d);
+#pragma unroll
+    for (int i = j + 1; i < D; ++i) {
+      double v = S[i][j];
+#pragma unroll
+      for (int k = 0; k < j; ++k) v -= L[i][k] * L[j][k];
+      L[i][j] = v / L[j][j];
+    }
+  }
+  // Tx = S^-1 Sx, Ty = S^-1 Sy (column by column), M = Sq - Sx Tx - Sy Ty
+  double Tx[4][4], Ty[4][4], M4[4][4];
+#pragma unroll
+  for (int col = 0; col < D; ++col) {
+    double zx[4], zy[4];
+#pragma unroll
+    for (int i = 0; i < D; ++i) {
+      double vx = Sx[i][col], vy = Sy[i][col];
+#pragma unroll
+      for (int k = 0; k < i; ++k) {
+        vx -= L[i][k] * zx[k];
+        vy -= L[i][k] * zy[k];
+      }
+      zx[i] = vx / L[i][i];
+      zy[i] = vy / L[i][i];
+    }
+#pragma unroll
+    for (int i = D - 1; i >= 0; --i) {
+      double vx = zx[i], vy = zy[i];
+#pragma unroll
+      for (int k = i + 1; k < D; ++k) {
+        vx -= L[k][i] * Tx[k][col];
+        vy -= L[k][i] * Ty[k][col];
+      }
+      Tx[i][col] = vx / L[i][i];
+      Ty[i][col] = vy / L[i][i];
+    }
+  }
+#pragma unroll
+  for (int a = 0; a < D; ++a)
+#pragma unroll
+    for (int b = 0; b < D; ++b) {
+      double v = Sq[a][b];
+#pragma unroll
+      for (int k = 0; k < D; ++k) v -= Sx[a][k] * Tx[k][b] + Sy[a][k] * Ty[k][b];
+      M4[a][b] = v;
+    }
+#pragma unroll
+  for (int a = 0; a < D; ++a)
+#pragma unroll
+    for (int b = a + 1; b < D; ++b) M4[a][b] = M4[b][a] = 0.5 * (M4[a][b] + M4[b][a]);
+  double p3[4];
+  jacobi_smallest<D>(M4, p3);
+#pragma unroll
+  for (int a = 0; a < D; ++a) {
+    double v1 = 0, v2 = 0;
+#pragma unroll
+    for (int k = 0; k < D; ++k) {
+      v1 += Tx[a][k] * p3[k];
+      v2 += Ty[a][k] * p3[k];
+    }
+    p[a] = v1;
+    p[4 + a] = v2;
+    p[8 + a] = p3[a];
+  }
+  return true;
+}
+
+constexpr double kPnpPlanarRtol = 1e-10;  // smallest / largest eigenvalue of the centred covariance below which the
+                                          // points are solved as a plane: ~1e-14 from float32 rounding of planar
+                                          // sets, ~1e-9 for +-1 um out of a 120 mm plane
+
 // normalised DLT on the points whose bit is set in `sel`; X [vn][3] object points, xn [vn][2] normalised image points.
-// The 12 unknowns (rows p1, p2, p3 of the 3x4 projection) are reduced to the last row: for fixed p3 the optimum is
-// p1 = S^-1 Sx p3, p2 = S^-1 Sy p3 with S = sum P P^T, Sx = sum x P P^T, Sy = sum y P P^T (P = normalised
-// homogeneous point), and p3 is the smallest eigenvector of the 4x4 Schur complement
-// M = sum (x^2 + y^2) P P^T - Sx S^-1 Sx - Sy S^-1 Sy.
+// The 12 unknowns (rows p1, p2, p3 of the 3x4 projection) are reduced to the last row (dlt_reduce<4>) with
+// S = sum P P^T, Sx = sum x P P^T, Sy = sum y P P^T, Sq = sum (x^2 + y^2) P P^T (P = normalised homogeneous point).
+// Coplanar points make S singular; they are solved as a plane instead, when the centred covariance is flat to
+// kPnpPlanarRtol or a pivot of the general reduction fails: the normal n is the largest cross product of two rows of
+// the centred covariance (a rank-2 matrix), (e1, e2, n) a right-handed basis, and the homography
+// H ~ [r1 r2 t'] on Q = (P.e1, P.e2, 1) reduces the same way (dlt_reduce<3>).  Its sign puts the centroid in front
+// (H_22 > 0); r3 = r1 x r2 and the 3x3 of the projection is [r1 r2 r3] [e1 e2 n]^T.  A candidate fails only when
+// both reductions do (for example collinear points).
 __device__ bool pnp_dlt(const double* X, const double* xn, int vn, unsigned sel, double* R, double* t) {
   double c[3] = {0, 0, 0};
   int m = 0;
@@ -156,83 +246,81 @@ __device__ bool pnp_dlt(const double* X, const double* xn, int vn, unsigned sel,
     for (int b = 0; b < a; ++b) {
       S[a][b] = S[b][a]; Sx[a][b] = Sx[b][a]; Sy[a][b] = Sy[b][a]; Sq[a][b] = Sq[b][a];
     }
-  // Cholesky S = L L^T (S is positive definite for non-coplanar points)
-  double L[4][4];
+  // rows of the centred covariance C = S[0..2][0..2]: the largest cross product of two rows is the plane normal of a
+  // rank-2 C, and det C / (|that cross product| tr C) estimates the smallest eigenvalue over the largest within a factor
+  // of 3 (the cross products are columns of adj C, whose eigenvalues are the pairwise products of C's)
+  double nv[3] = {0, 0, 0}, nq = 0;
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    double d = S[j][j];
+  for (int a = 0; a < 2; ++a)
 #pragma unroll
-    for (int k = 0; k < j; ++k) d -= L[j][k] * L[j][k];
-    if (!(d > 1e-14 * S[j][j])) return false;
-    L[j][j] = sqrt(d);
-#pragma unroll
-    for (int i = j + 1; i < 4; ++i) {
-      double v = S[i][j];
-#pragma unroll
-      for (int k = 0; k < j; ++k) v -= L[i][k] * L[j][k];
-      L[i][j] = v / L[j][j];
-    }
-  }
-  // Tx = S^-1 Sx, Ty = S^-1 Sy (column by column), M = Sq - Sx Tx - Sy Ty
-  double Tx[4][4], Ty[4][4], M4[4][4];
-#pragma unroll
-  for (int col = 0; col < 4; ++col) {
-    double zx[4], zy[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      double vx = Sx[i][col], vy = Sy[i][col];
-#pragma unroll
-      for (int k = 0; k < i; ++k) {
-        vx -= L[i][k] * zx[k];
-        vy -= L[i][k] * zy[k];
+    for (int b = a + 1; b < 3; ++b) {
+      const double v[3] = {S[a][1] * S[b][2] - S[a][2] * S[b][1], S[a][2] * S[b][0] - S[a][0] * S[b][2],
+                           S[a][0] * S[b][1] - S[a][1] * S[b][0]};
+      const double q = v[0] * v[0] + v[1] * v[1] + v[2] * v[2];
+      if (q > nq) {
+        nq = q;
+        nv[0] = v[0]; nv[1] = v[1]; nv[2] = v[2];
       }
-      zx[i] = vx / L[i][i];
-      zy[i] = vy / L[i][i];
+    }
+  const double detC = S[0][0] * (S[1][1] * S[2][2] - S[1][2] * S[2][1]) - S[0][1] * (S[1][0] * S[2][2] - S[1][2] * S[2][0]) +
+                      S[0][2] * (S[1][0] * S[2][1] - S[1][1] * S[2][0]);
+  // coplanar after float32 rounding: the 4x4 system is singular whether or not its pivots fall under 1e-14
+  const bool flat = detC <= kPnpPlanarRtol * sqrt(nq) * (S[0][0] + S[1][1] + S[2][2]);
+  double p[12], M[9], p4[3];
+  if (!flat && dlt_reduce<4>(S, Sx, Sy, Sq, p)) {
+    for (int r = 0; r < 3; ++r) {
+      for (int k = 0; k < 3; ++k) M[3 * r + k] = p[4 * r + k] * s;
+      p4[r] = p[4 * r + 3] - (M[3 * r] * c[0] + M[3 * r + 1] * c[1] + M[3 * r + 2] * c[2]);
+    }
+  } else {  // coplanar points: planar DLT
+    if (!(nq > 0) || !isfinite(nq)) return false;
+    const double in = 1.0 / sqrt(nq);
+    const double n[3] = {nv[0] * in, nv[1] * in, nv[2] * in};
+    const double f0 = fabs(n[0]), f1 = fabs(n[1]), f2 = fabs(n[2]);
+    const int ax = (f0 <= f1 && f0 <= f2) ? 0 : (f1 <= f2 ? 1 : 2);  // the axis least aligned with n
+    double e1[3] = {ax == 0 ? 0.0 : (ax == 1 ? -n[2] : n[1]), ax == 0 ? n[2] : (ax == 1 ? 0.0 : -n[0]),
+                    ax == 0 ? -n[1] : (ax == 1 ? n[0] : 0.0)};  // n x axis
+    const double ie = 1.0 / sqrt(e1[0] * e1[0] + e1[1] * e1[1] + e1[2] * e1[2]);
+    e1[0] *= ie; e1[1] *= ie; e1[2] *= ie;
+    const double e2[3] = {n[1] * e1[2] - n[2] * e1[1], n[2] * e1[0] - n[0] * e1[2], n[0] * e1[1] - n[1] * e1[0]};
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int b = 0; b < 4; ++b) S[a][b] = Sx[a][b] = Sy[a][b] = Sq[a][b] = 0.0;
+    for (int i = 0; i < vn; ++i) {
+      if (!((sel >> i) & 1u)) continue;
+      const double P0 = (X[3 * i] - c[0]) * s, P1 = (X[3 * i + 1] - c[1]) * s, P2 = (X[3 * i + 2] - c[2]) * s;
+      const double Q[3] = {P0 * e1[0] + P1 * e1[1] + P2 * e1[2], P0 * e2[0] + P1 * e2[1] + P2 * e2[2], 1.0};
+      const double x = xn[2 * i], y = xn[2 * i + 1], q = x * x + y * y;
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = a; b < 3; ++b) {
+          const double qq = Q[a] * Q[b];
+          S[a][b] += qq;
+          Sx[a][b] += x * qq;
+          Sy[a][b] += y * qq;
+          Sq[a][b] += q * qq;
+        }
     }
 #pragma unroll
-    for (int i = 3; i >= 0; --i) {
-      double vx = zx[i], vy = zy[i];
+    for (int a = 1; a < 3; ++a)
 #pragma unroll
-      for (int k = i + 1; k < 4; ++k) {
-        vx -= L[k][i] * Tx[k][col];
-        vy -= L[k][i] * Ty[k][col];
+      for (int b = 0; b < a; ++b) {
+        S[a][b] = S[b][a]; Sx[a][b] = Sx[b][a]; Sy[a][b] = Sy[b][a]; Sq[a][b] = Sq[b][a];
       }
-      Tx[i][col] = vx / L[i][i];
-      Ty[i][col] = vy / L[i][i];
+    if (!dlt_reduce<3>(S, Sx, Sy, Sq, p)) return false;
+    const double sg = p[10] < 0 ? -s : s;  // H = rows p[0..3), p[4..7), p[8..11); columns 0, 1 carry the scale s
+    const double a1[3] = {p[0] * sg, p[4] * sg, p[8] * sg}, a2[3] = {p[1] * sg, p[5] * sg, p[9] * sg};
+    const double l1 = sqrt(a1[0] * a1[0] + a1[1] * a1[1] + a1[2] * a1[2]);
+    const double l2 = sqrt(a2[0] * a2[0] + a2[1] * a2[1] + a2[2] * a2[2]);
+    const double il = 1.0 / sqrt(l1 * l2);
+    const double a3[3] = {(a1[1] * a2[2] - a1[2] * a2[1]) * il, (a1[2] * a2[0] - a1[0] * a2[2]) * il,
+                          (a1[0] * a2[1] - a1[1] * a2[0]) * il};
+    for (int r = 0; r < 3; ++r) {
+      for (int k = 0; k < 3; ++k) M[3 * r + k] = a1[r] * e1[k] + a2[r] * e2[k] + a3[r] * n[k];
+      p4[r] = (p[10] < 0 ? -p[4 * r + 2] : p[4 * r + 2]) - (M[3 * r] * c[0] + M[3 * r + 1] * c[1] + M[3 * r + 2] * c[2]);
     }
-  }
-#pragma unroll
-  for (int a = 0; a < 4; ++a)
-#pragma unroll
-    for (int b = 0; b < 4; ++b) {
-      double v = Sq[a][b];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) v -= Sx[a][k] * Tx[k][b] + Sy[a][k] * Ty[k][b];
-      M4[a][b] = v;
-    }
-#pragma unroll
-  for (int a = 0; a < 4; ++a)
-#pragma unroll
-    for (int b = a + 1; b < 4; ++b) M4[a][b] = M4[b][a] = 0.5 * (M4[a][b] + M4[b][a]);
-  double p3[4];
-  jacobi4_smallest(M4, p3);
-  double p[12];
-#pragma unroll
-  for (int a = 0; a < 4; ++a) {
-    double v1 = 0, v2 = 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      v1 += Tx[a][k] * p3[k];
-      v2 += Ty[a][k] * p3[k];
-    }
-    p[a] = v1;
-    p[4 + a] = v2;
-    p[8 + a] = p3[a];
-  }
-  double M[9], p4[3];
-  for (int r = 0; r < 3; ++r) {
-    for (int k = 0; k < 3; ++k) M[3 * r + k] = p[4 * r + k] * s;
-    p4[r] = p[4 * r + 3] - (M[3 * r] * c[0] + M[3 * r + 1] * c[1] + M[3 * r + 2] * c[2]);
   }
   double det = mat3_det(M);
   if (det < 0) {
@@ -395,7 +483,9 @@ __global__ void __launch_bounds__(128) k_pnp(PnpParams pp, const float* __restri
     uv[2 * i + 1] = p.y;
   }
   float* out = poses + (size_t)obj * 12;
-  bool dead = fabsf(sum) < 0.01f;  // map_offsets :489 / map_pnp :510
+  // map_offsets :489 / map_pnp :510; a NaN or inf keypoint (non-finite sum) also gives zeros, as in the reference, where
+  // cv2 returns a NaN translation for it and pnp() returns zeros (:48-50)
+  bool dead = fabsf(sum) < 0.01f || !isfinite(sum);
   if (!dead && offsets) {
     sum = 0.f;
     for (int i = 0; i < vn; ++i) {
@@ -404,7 +494,7 @@ __global__ void __launch_bounds__(128) k_pnp(PnpParams pp, const float* __restri
       uv[2 * i + 1] = q.y;
       sum = __fadd_rn(sum, __fadd_rn(q.x, q.y));
     }
-    dead = fabsf(sum) < 0.01f;
+    dead = fabsf(sum) < 0.01f || !isfinite(sum);
   }
   if (dead) {
     if (lane < 12) out[lane] = 0.f;

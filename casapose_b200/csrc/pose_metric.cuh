@@ -13,7 +13,7 @@
 //
 //   k_pose_project  one block per object: guards, both projections, err_2d, ADD; symmetric objects leave their
 //                   two point clouds (float32 xyz) in scratch;
-//   k_adds_min      (256-row tile, object): every thread owns one ground-truth point and scans the estimated
+//   k_adds_min      (256-row tile, object stride): every thread owns one ground-truth point and scans the estimated
 //                   cloud through shared memory — FP32-issue-bound, 7 instructions per pair;
 //   k_pose_finalize sums the tile partials in order, applies the 0.1*diameter and 2-D thresholds.
 // Output rows are map_estimates' own: [err_2d, err_3d, valid_3d, valid_2d, missing, false_positive].
@@ -24,6 +24,7 @@ namespace casa {
 
 constexpr int kMetricThreads = 256;
 constexpr int kAddsTile = 1024;  // estimated points per shared-memory pass
+constexpr int kAddsGridY = 65535;  // gridDim.y limit: k_adds_min strides over objects beyond it
 
 struct PoseErrParams {
   int n, m, maxp;
@@ -122,47 +123,50 @@ __global__ void __launch_bounds__(kMetricThreads)
   }
 }
 
-// grid (tiles, n): rows = ground-truth points, scan = estimated points (adds_error(target, estimate), :619)
+// grid (tiles, min(n, kAddsGridY)): rows = ground-truth points, scan = estimated points (adds_error(target, estimate),
+// :619).  Objects stride over blockIdx.y, so the object count is not bound by the 65535 limit of gridDim.y; partial
+// sums are indexed [obj][tile] with `tiles` row tiles per object.
 __global__ void __launch_bounds__(kMetricThreads)
-    k_adds_min(PoseErrParams pp, const int* __restrict__ model_cnt, const int* __restrict__ obj_model,
+    k_adds_min(PoseErrParams pp, int tiles, const int* __restrict__ model_cnt, const int* __restrict__ obj_model,
                const int* __restrict__ state, const float4* __restrict__ cloud_gt, const float4* __restrict__ cloud_est,
                double* __restrict__ partial) {
   __shared__ float4 sB[kAddsTile];
   __shared__ double sh[kMetricThreads / 32];
-  const int obj = blockIdx.y;
-  if (state[obj] != 2) return;
-  const int model = obj_model ? obj_model[obj] : obj % pp.m;
-  const int cnt = min(model_cnt[model], pp.maxp);
-  const int row0 = blockIdx.x * kMetricThreads;
-  if (row0 >= cnt) return;
-  const int r = row0 + threadIdx.x;
-  const float4 a = cloud_gt[(size_t)obj * pp.maxp + min(r, cnt - 1)];
-  const float4* B = cloud_est + (size_t)obj * pp.maxp;
-  float best0 = INFINITY, best1 = INFINITY;  // two chains: the minimum is exact in any order
-  for (int t0 = 0; t0 < cnt; t0 += kAddsTile) {
-    const int nt = min(kAddsTile, cnt - t0);
-    __syncthreads();
-    for (int k = threadIdx.x; k < nt; k += kMetricThreads) sB[k] = B[t0 + k];
-    __syncthreads();
-    int k = 0;
+  for (int obj = blockIdx.y; obj < pp.n; obj += gridDim.y) {  // uniform per block: the barriers below stay uniform
+    if (state[obj] != 2) continue;
+    const int model = obj_model ? obj_model[obj] : obj % pp.m;
+    const int cnt = min(model_cnt[model], pp.maxp);
+    const int row0 = blockIdx.x * kMetricThreads;
+    if (row0 >= cnt) continue;
+    const int r = row0 + threadIdx.x;
+    const float4 a = cloud_gt[(size_t)obj * pp.maxp + min(r, cnt - 1)];
+    const float4* B = cloud_est + (size_t)obj * pp.maxp;
+    float best0 = INFINITY, best1 = INFINITY;  // two chains: the minimum is exact in any order
+    for (int t0 = 0; t0 < cnt; t0 += kAddsTile) {
+      const int nt = min(kAddsTile, cnt - t0);
+      __syncthreads();
+      for (int k = threadIdx.x; k < nt; k += kMetricThreads) sB[k] = B[t0 + k];
+      __syncthreads();
+      int k = 0;
 #pragma unroll 4
-    for (; k + 1 < nt; k += 2) {
-      const float4 b0 = sB[k], b1 = sB[k + 1];
-      const float x0 = a.x - b0.x, y0 = a.y - b0.y, z0 = a.z - b0.z;
-      const float x1 = a.x - b1.x, y1 = a.y - b1.y, z1 = a.z - b1.z;
-      best0 = fminf(best0, fmaf(x0, x0, fmaf(y0, y0, z0 * z0)));
-      best1 = fminf(best1, fmaf(x1, x1, fmaf(y1, y1, z1 * z1)));
+      for (; k + 1 < nt; k += 2) {
+        const float4 b0 = sB[k], b1 = sB[k + 1];
+        const float x0 = a.x - b0.x, y0 = a.y - b0.y, z0 = a.z - b0.z;
+        const float x1 = a.x - b1.x, y1 = a.y - b1.y, z1 = a.z - b1.z;
+        best0 = fminf(best0, fmaf(x0, x0, fmaf(y0, y0, z0 * z0)));
+        best1 = fminf(best1, fmaf(x1, x1, fmaf(y1, y1, z1 * z1)));
+      }
+      if (k < nt) {
+        const float4 b0 = sB[k];
+        const float x0 = a.x - b0.x, y0 = a.y - b0.y, z0 = a.z - b0.z;
+        best0 = fminf(best0, fmaf(x0, x0, fmaf(y0, y0, z0 * z0)));
+      }
     }
-    if (k < nt) {
-      const float4 b0 = sB[k];
-      const float x0 = a.x - b0.x, y0 = a.y - b0.y, z0 = a.z - b0.z;
-      best0 = fminf(best0, fmaf(x0, x0, fmaf(y0, y0, z0 * z0)));
-    }
+    const double best = (double)fminf(best0, best1);
+    const double v = r < cnt ? (double)(float)sqrt(fabs(best) + 1e-5) : 0.0;  // :609, cast to float32 per point
+    const double s = block_sum(v, sh);
+    if (threadIdx.x == 0) partial[(size_t)obj * tiles + blockIdx.x] = s;
   }
-  const double best = (double)fminf(best0, best1);
-  const double v = r < cnt ? (double)(float)sqrt(fabs(best) + 1e-5) : 0.0;  // :609, cast to float32 per point
-  const double s = block_sum(v, sh);
-  if (threadIdx.x == 0) partial[(size_t)obj * gridDim.x + blockIdx.x] = s;
 }
 
 __global__ void k_pose_finalize(PoseErrParams pp, int tiles, const int* __restrict__ model_cnt, const int* __restrict__ obj_model,

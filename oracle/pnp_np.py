@@ -22,24 +22,64 @@ def _polar(M):
     return R
 
 
+PLANAR_RTOL = 1e-10  # pnp.cuh kPnpPlanarRtol
+
+
+def _reduce(S, Sx, Sy, Sq):
+    """dlt_reduce<D>: Schur reduction of the DLT normal equations, rows (h1, h2, h3) of the projection (D = 4) or the
+    homography (D = 3); None when a Cholesky pivot of S is not above 1e-14 times its diagonal entry."""
+    D = len(S)
+    L = np.zeros((D, D))
+    for j in range(D):
+        d = S[j, j] - L[j, :j] @ L[j, :j]
+        if not d > 1e-14 * S[j, j]:
+            return None
+        L[j, j] = np.sqrt(d)
+        for i in range(j + 1, D):
+            L[i, j] = (S[i, j] - L[i, :j] @ L[j, :j]) / L[j, j]
+    Tx = np.linalg.solve(L.T, np.linalg.solve(L, Sx))
+    Ty = np.linalg.solve(L.T, np.linalg.solve(L, Sy))
+    M = Sq - Sx @ Tx - Sy @ Ty  # Schur complement on the last row
+    M = 0.5 * (M + M.T)
+    _, v = np.linalg.eigh(M)
+    h3 = v[:, 0]
+    return np.stack([Tx @ h3, Ty @ h3, h3])
+
+
+def _moments(Q, xn):
+    x, y = xn[:, 0], xn[:, 1]
+    QQ = Q[:, :, None] * Q[:, None, :]
+    return QQ.sum(0), (x[:, None, None] * QQ).sum(0), (y[:, None, None] * QQ).sum(0), ((x * x + y * y)[:, None, None] * QQ).sum(0)
+
+
 def dlt(X, xn):
     c = X.mean(0)
     s = 1.0 / np.sqrt(((X - c) ** 2).sum(1).mean())
     Xs = (X - c) * s
-    P = np.concatenate([Xs, np.ones((len(X), 1))], 1)  # [m,4]
-    x, y = xn[:, 0], xn[:, 1]
-    PP = P[:, :, None] * P[:, None, :]
-    S, Sx, Sy = PP.sum(0), (x[:, None, None] * PP).sum(0), (y[:, None, None] * PP).sum(0)
-    Sq = ((x * x + y * y)[:, None, None] * PP).sum(0)
-    np.linalg.cholesky(S)  # positive definite for non-coplanar points (LinAlgError otherwise)
-    Tx, Ty = np.linalg.solve(S, Sx), np.linalg.solve(S, Sy)
-    M4 = Sq - Sx @ Tx - Sy @ Ty  # Schur complement on the last row of the projection
-    M4 = 0.5 * (M4 + M4.T)
-    _, v = np.linalg.eigh(M4)
-    p3 = v[:, 0]
-    p = np.stack([Tx @ p3, Ty @ p3, p3])
-    M = p[:, :3] * s
-    p4 = p[:, 3] - M @ c
+    S = _moments(np.concatenate([Xs, np.ones((len(X), 1))], 1), xn)
+    C = S[0][:3, :3]
+    n = max((np.cross(C[a], C[b]) for a, b in ((0, 1), (0, 2), (1, 2))), key=lambda v: v @ v)
+    flat = C[0] @ np.cross(C[1], C[2]) <= PLANAR_RTOL * np.sqrt(n @ n) * np.trace(C)  # covariance flat to 1e-10
+    p = None if flat else _reduce(*S)
+    if p is not None:
+        M = p[:, :3] * s
+        p4 = p[:, 3] - M @ c
+    else:  # coplanar points: planar DLT (pnp_dlt's second branch)
+        if not (n @ n > 0 and np.isfinite(n @ n)):
+            raise np.linalg.LinAlgError("collinear points")
+        n = n / np.sqrt(n @ n)
+        e1 = np.cross(n, np.eye(3)[int(np.argmin(np.abs(n)))])
+        e1 = e1 / np.sqrt(e1 @ e1)
+        e2 = np.cross(n, e1)
+        h = _reduce(*_moments(np.stack([Xs @ e1, Xs @ e2, np.ones(len(X))], 1), xn))
+        if h is None:
+            raise np.linalg.LinAlgError("collinear points")
+        if h[2, 2] < 0:  # centroid in front of the camera
+            h = -h
+        a1, a2 = h[:, 0] * s, h[:, 1] * s
+        a3 = np.cross(a1, a2) / np.sqrt(np.linalg.norm(a1) * np.linalg.norm(a2))
+        M = np.outer(a1, e1) + np.outer(a2, e2) + np.outer(a3, n)
+        p4 = h[:, 2] - M @ c
     if np.linalg.det(M) < 0:
         M, p4 = -M, -p4
     sc = np.cbrt(np.linalg.det(M))
@@ -102,7 +142,9 @@ def lm(X, uv, K4, R, t, iters):
 def pnp(points_3d, points_2d, camera_matrix, reproj_px=12.0):
     """[vn,3], [vn,2] (x,y), [3,3] -> [3,4] float32, the algorithm of k_pnp."""
     uv32 = np.asarray(points_2d, np.float32)
-    if abs(float(uv32.sum(dtype=np.float32))) < 0.01:
+    total = uv32.sum(dtype=np.float32)
+    # compared in float32 (0.01f), as TensorFlow does; a non-finite keypoint: cv2 returns a NaN translation -> zeros
+    if abs(total) < np.float32(0.01) or not np.isfinite(total):
         return np.zeros((3, 4), np.float32)
     X = np.asarray(points_3d, np.float32).astype(np.float64)
     uv = uv32.astype(np.float64)
