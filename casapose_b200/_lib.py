@@ -69,6 +69,9 @@ EXPORTS = {
                                    C.c_void_p, C.c_void_p, C.POINTER(RansacDebug), C.c_void_p]),
     "casa_ransac_vote_seg": (C.c_int, [C.c_void_p, C.POINTER(RansacParams), C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.POINTER(RansacDebug), C.c_void_p]),
+    "casa_ransac_vote_typed": (C.c_int, [C.c_void_p, C.POINTER(RansacParams), C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RansacDebug),
+                                         C.c_void_p]),
     "casa_ransac_vote_dlpack": (C.c_int, [C.c_void_p, C.POINTER(RansacParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                           C.c_void_p]),
     "casa_ransac_vote_host": (C.c_int, [C.c_void_p, C.POINTER(RansacParams), C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -79,6 +82,10 @@ EXPORTS = {
                                C.POINTER(LsDebug), C.c_void_p]),
     "casa_ls_vote_backward": (C.c_int, [C.c_void_p, C.POINTER(LsParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "casa_ls_vote_typed": (C.c_int, [C.c_void_p, C.POINTER(LsParams), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.POINTER(LsDebug), C.c_void_p]),
+    "casa_ls_vote_backward_typed": (C.c_int, [C.c_void_p, C.POINTER(LsParams), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "casa_pnp": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                            C.c_void_p]),
     "casa_pnp_backward": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,

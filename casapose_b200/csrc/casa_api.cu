@@ -244,8 +244,9 @@ struct casa_handle {
   int64_t rounds_total = 0, launches_total = 0;
   unsigned long long* pinned_stats = nullptr;  // 4 words, page-locked
   int score_occ = 0, score_occ_narrow = 0;  // resident k_score blocks per SM (8 / 4 hypotheses per lane)
-  int fused_occ = 0;              // resident k_ls_fused blocks per SM (persistent grid of the LS forward call)
-  int classify_static_smem[2] = {-1, -1};  // static shared memory of k_ls_classify<9> / <0> (queried once)
+  // per input dtype (casa_dtype): an instantiation for 16-bit inputs may differ in registers and static shared memory
+  int fused_occ[3] = {0, 0, 0};   // resident k_ls_fused blocks per SM (persistent grid of the LS forward call)
+  int classify_static_smem[3][2] = {{-1, -1}, {-1, -1}, {-1, -1}};  // static shared memory of k_ls_classify<9> / <0>
   int use_graph = 1;
   // keypoint all-gather (NCCL, resolved with dlopen: the library itself does not link against it)
   void* comm = nullptr;           // ncclComm_t
@@ -967,16 +968,34 @@ enum class MaskForm {
   kPackedBits  // u32 [b,h,w] membership words packed on the host (casa_ransac_vote_host)
 };
 
+// Instantiation of an input-reading kernel for the element type `t` names: f(Elem<T>()) returns the kernel for T.
+template <typename T>
+struct Elem {
+  using type = T;
+};
+template <class F>
+static const void* by_dtype(casa_dtype t, F f) {
+  return t == CASA_FLOAT16 ? f(Elem<__half>()) : t == CASA_BFLOAT16 ? f(Elem<__nv_bfloat16>()) : f(Elem<float>());
+}
+static const void* gather_dirs_fn(int vn, casa_dtype t) {
+  return vn == 9 ? by_dtype(t, [](auto e) { return (const void*)k_gather_dirs<18, typename decltype(e)::type>; })
+                 : by_dtype(t, [](auto e) { return (const void*)k_gather_dirs<0, typename decltype(e)::type>; });
+}
+static size_t dtype_bytes(casa_dtype t) { return t == CASA_FLOAT32 ? 4 : 2; }
+static bool dtype_ok(int t) { return t == CASA_FLOAT32 || t == CASA_FLOAT16 || t == CASA_BFLOAT16; }
+
 // The inputs and outputs of one vote.
 struct VoteInput {
   const void* mask = nullptr;
   MaskForm form = MaskForm::kOneHot;
-  const float* vertex = nullptr;
+  const void* vertex = nullptr;
   bool vertex_mapped = false;  // the field is mapped host memory: k_gather_dirs reads it over PCIe, not k_place
   int not_binary = 0;          // kPackedBits: the host packer saw a mask value other than 0 / 1
   const int32_t* idxs = nullptr;
   const float* selection = nullptr;
   float* out = nullptr;
+  casa_dtype mask_dtype = CASA_FLOAT32;    // element type of mask (kOneHot, kSeg)
+  casa_dtype vertex_dtype = CASA_FLOAT32;  // element type of vertex
 };
 
 // Builds the launch list of one vote and launches it on `st` with `h`'s workspace, into the next read-back slot of
@@ -1026,7 +1045,8 @@ static int vote_enqueue(casa_handle* h, const casa_ransac_params* p, const VoteI
   const int score_occ = narrow ? h->score_occ_narrow : h->score_occ;
   const int refine_gx = d.max_rtiles < h->sm_count * 4 ? d.max_rtiles : h->sm_count * 4;
   const int gather_gx = (d.cap + 255) / 256 < 24 ? (d.cap + 255) / 256 : 24;
-  const int vec4 = ((((size_t)d.hw * d.oc) & 3) == 0) && ((((uintptr_t)in.mask) & 15) == 0);
+  const size_t per_vec = 16 / dtype_bytes(in.mask_dtype);  // mask elements per 128-bit load of k_mask_bits
+  const int vec_mask = ((((size_t)d.hw * d.oc) % per_vec) == 0) && ((((uintptr_t)in.mask) & 15) == 0);
   const int plan_threads = d.J > 256 ? 1024 : 256;
 
   // The launch list of the whole call.  Round 0 is spelled out (it carries the timing events, which a WHILE body
@@ -1046,22 +1066,25 @@ static int vote_enqueue(casa_handle* h, const casa_ransac_params* p, const VoteI
   if (in.form == MaskForm::kPackedBits)  // bit 30 of the flag: not binary
     steps.push_back(kstep((const void*)k_bits_in, dim3(d.nct, d.b), 256).arg((const uint32_t*)in.mask).arg(ws).arg(d).arg(in.not_binary));
   else if (in.form == MaskForm::kSeg)
-    steps.push_back(kstep((const void*)k_seg_bits, dim3(d.nct, d.b), 256).arg((const float*)in.mask).arg(ws).arg(d));
+    steps.push_back(kstep(by_dtype(in.mask_dtype, [](auto e) { return (const void*)k_seg_bits<typename decltype(e)::type>; }),
+                          dim3(d.nct, d.b), 256).arg(in.mask).arg(ws).arg(d));
   else
-    steps.push_back(kstep((const void*)k_mask_bits, dim3(d.nct, d.b), 256).arg((const float*)in.mask).arg(ws).arg(d).arg(vec4));
+    steps.push_back(kstep(by_dtype(in.mask_dtype, [](auto e) { return (const void*)k_mask_bits<typename decltype(e)::type>; }),
+                          dim3(d.nct, d.b), 256).arg(in.mask).arg(ws).arg(d).arg(vec_mask));
   // k_place gathers the directions while it scatters the pixels, unless the field lives in mapped host memory (the
-  // host entry point: k_gather_dirs reads full lines over PCIe) or is not 8-byte aligned; jobs above max_num are
-  // gathered after the cap filter
-  const int fuse_gather = (!in.vertex_mapped && (((uintptr_t)in.vertex) & 7) == 0) ? 1 : 0;
+  // host entry point: k_gather_dirs reads full lines over PCIe) or is not aligned to one (dy, dx) pair; jobs above
+  // max_num are gathered after the cap filter
+  const int fuse_gather = (!in.vertex_mapped && (((uintptr_t)in.vertex) & (2 * dtype_bytes(in.vertex_dtype) - 1)) == 0) ? 1 : 0;
   const bool may_cap = (float)d.hw > p->max_num;
-  steps.push_back(kstep(d.vn == 9 ? (const void*)k_place<9> : (const void*)k_place<0>, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg(in.vertex).arg(ws).arg(d).arg(fuse_gather));
+  const void* place = d.vn == 9 ? by_dtype(in.vertex_dtype, [](auto e) { return (const void*)k_place<9, typename decltype(e)::type>; })
+                                : by_dtype(in.vertex_dtype, [](auto e) { return (const void*)k_place<0, typename decltype(e)::type>; });
+  steps.push_back(kstep(place, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg(in.vertex).arg(ws).arg(d).arg(fuse_gather));
   if (may_cap) steps.push_back(kstep((const void*)k_cap_filter, d.J, 1024).arg(ws).arg(d).arg(in.selection));
   // round 0's plan (work items, refinement tiles) only needs the job table: it runs beside the direction gather and
   // k_hypgen (side branch in slot 1, joined by k_score)
   steps.push_back(kstep((const void*)k_plan, 1, plan_threads).arg(ws).arg(d).arg((int)0).on_side(1, 1));
   if (!fuse_gather || may_cap)
-    steps.push_back(kstep(d.vn == 9 ? (const void*)k_gather_dirs<18> : (const void*)k_gather_dirs<0>, dim3(gather_gx, d.J), 256)
-                        .arg(in.vertex).arg(ws).arg(d).arg(fuse_gather));
+    steps.push_back(kstep(gather_dirs_fn(d.vn, in.vertex_dtype), dim3(gather_gx, d.J), 256).arg(in.vertex).arg(ws).arg(d).arg(fuse_gather));
   for (int part = 0; part < 2; ++part) {  // part 0: round 0; part 1: the WHILE body (rnd = -1: read ctrl[CTRL_ROUND])
     const int rnd = part == 0 ? 0 : -1;
     if (part == 1) {
@@ -1136,20 +1159,29 @@ static int ransac_vote_route(casa_handle* h, const casa_ransac_params* p, const 
   return rc;
 }
 
+extern "C" int casa_ransac_vote_typed(casa_handle* h, const casa_ransac_params* p, int mask_is_seg, casa_dtype mask_dtype,
+                                      const void* mask, casa_dtype vertex_dtype, const void* vertex, const int32_t* idxs,
+                                      const float* selection, float* out_points, const casa_ransac_debug* debug, void* stream) {
+  if (!dtype_ok(mask_dtype) || !dtype_ok(vertex_dtype))
+    return fail(CASA_ERR_INVALID, "mask / vertex dtype %d / %d is not a casa_dtype", (int)mask_dtype, (int)vertex_dtype);
+  VoteInput in{mask, mask_is_seg ? MaskForm::kSeg : MaskForm::kOneHot, vertex, /*vertex_mapped=*/false, /*not_binary=*/0,
+               idxs, selection, out_points};
+  in.mask_dtype = mask_dtype;
+  in.vertex_dtype = vertex_dtype;
+  cudaStream_t ran_on;
+  return ransac_vote_route(h, p, in, debug, stream, &ran_on);
+}
+
 extern "C" int casa_ransac_vote(casa_handle* h, const casa_ransac_params* p, const float* mask, const float* vertex,
                                 const int32_t* idxs, const float* selection, float* out_points,
                                 const casa_ransac_debug* debug, void* stream) {
-  const VoteInput in{mask, MaskForm::kOneHot, vertex, /*vertex_mapped=*/false, /*not_binary=*/0, idxs, selection, out_points};
-  cudaStream_t ran_on;
-  return ransac_vote_route(h, p, in, debug, stream, &ran_on);
+  return casa_ransac_vote_typed(h, p, 0, CASA_FLOAT32, mask, CASA_FLOAT32, vertex, idxs, selection, out_points, debug, stream);
 }
 
 extern "C" int casa_ransac_vote_seg(casa_handle* h, const casa_ransac_params* p, const float* seg, const float* vertex,
                                     const int32_t* idxs, const float* selection, float* out_points,
                                     const casa_ransac_debug* debug, void* stream) {
-  const VoteInput in{seg, MaskForm::kSeg, vertex, /*vertex_mapped=*/false, /*not_binary=*/0, idxs, selection, out_points};
-  cudaStream_t ran_on;
-  return ransac_vote_route(h, p, in, debug, stream, &ran_on);
+  return casa_ransac_vote_typed(h, p, 1, CASA_FLOAT32, seg, CASA_FLOAT32, vertex, idxs, selection, out_points, debug, stream);
 }
 
 // ------------------------------------------------------------------------------------------------ DLPack shim
@@ -1182,14 +1214,20 @@ struct DLManagedTensor {
   void (*deleter)(DLManagedTensor*);
 };
 
-int check_dl(const DLManagedTensor* m, const char* name, int device, int ndim_a, int ndim_b) {
+// *dtype (NULL: only float32 is accepted): float32, float16 (code 2, 16 bits) or bfloat16 (code 4, 16 bits)
+int check_dl(const DLManagedTensor* m, const char* name, int device, int ndim_a, int ndim_b, casa_dtype* dtype = nullptr) {
   if (!m) return fail(CASA_ERR_INVALID, "%s: DLManagedTensor is NULL", name);
   const DLTensor& t = m->dl_tensor;
   if (t.device.device_type != 2 && t.device.device_type != 13)
     return fail(CASA_ERR_INVALID, "%s: DLPack device type %d is not CUDA", name, t.device.device_type);
   if (t.device.device_id != device) return fail(CASA_ERR_INVALID, "%s lives on CUDA device %d, the handle on %d", name, t.device.device_id, device);
-  if (t.dtype.code != 2 || t.dtype.bits != 32 || t.dtype.lanes != 1)
-    return fail(CASA_ERR_INVALID, "%s must be float32 (DLPack dtype code %d, %d bits, %d lanes)", name, t.dtype.code, t.dtype.bits, t.dtype.lanes);
+  const bool f32 = t.dtype.code == 2 && t.dtype.bits == 32 && t.dtype.lanes == 1;
+  const bool f16 = t.dtype.code == 2 && t.dtype.bits == 16 && t.dtype.lanes == 1;
+  const bool bf16 = t.dtype.code == 4 && t.dtype.bits == 16 && t.dtype.lanes == 1;
+  if (!(f32 || (dtype && (f16 || bf16))))
+    return fail(CASA_ERR_INVALID, "%s must be %s (DLPack dtype code %d, %d bits, %d lanes)", name,
+                dtype ? "float32, float16 or bfloat16" : "float32", t.dtype.code, t.dtype.bits, t.dtype.lanes);
+  if (dtype) *dtype = f32 ? CASA_FLOAT32 : f16 ? CASA_FLOAT16 : CASA_BFLOAT16;
   if (t.ndim != ndim_a && t.ndim != ndim_b) return fail(CASA_ERR_INVALID, "%s has %d dimensions", name, t.ndim);
   if (!t.data || !t.shape) return fail(CASA_ERR_INVALID, "%s: NULL data / shape", name);
   if (t.strides) {  // must be compact row-major (NHWC like the reference's tensors): no silent copies
@@ -1202,7 +1240,7 @@ int check_dl(const DLManagedTensor* m, const char* name, int device, int ndim_a,
   return CASA_OK;
 }
 
-const float* dl_data(const DLManagedTensor* m) { return (const float*)((const char*)m->dl_tensor.data + m->dl_tensor.byte_offset); }
+const void* dl_data(const DLManagedTensor* m) { return (const char*)m->dl_tensor.data + m->dl_tensor.byte_offset; }
 
 struct DeferredDelete {
   DLManagedTensor* m;
@@ -1244,8 +1282,9 @@ extern "C" int casa_ransac_vote_dlpack(casa_handle* h, const casa_ransac_params*
     if (o && o->deleter) o->deleter(o);
     return code;
   };
-  int rc = check_dl(m, mask_is_seg ? "seg" : "mask", h->device, 4, 4);
-  if (!rc) rc = check_dl(v, "vertex", h->device, 5, 6);
+  casa_dtype mdt = CASA_FLOAT32, vdt = CASA_FLOAT32;
+  int rc = check_dl(m, mask_is_seg ? "seg" : "mask", h->device, 4, 4, &mdt);
+  if (!rc) rc = check_dl(v, "vertex", h->device, 5, 6, &vdt);
   if (!rc) rc = check_dl(o, "out", h->device, 4, 4);
   if (rc) return reject(rc);
   casa_ransac_params q = *p;  // shapes come from the tensors themselves
@@ -1261,8 +1300,10 @@ extern "C" int casa_ransac_vote_dlpack(casa_handle* h, const casa_ransac_params*
   if (vs[0] != ms[0] || vs[1] != ms[1] || vs[2] != ms[2] || vs[v->dl_tensor.ndim - 1] != 2 || (q.vertex_per_class && vs[3] != q.oc))
     return reject(fail(CASA_ERR_INVALID, "vertex must be [b,h,w,vn,2] or [b,h,w,oc,vn,2] matching the mask"));
   if (os[0] != q.b || os[1] != q.oc || os[2] != q.vn || os[3] != 2) return reject(fail(CASA_ERR_INVALID, "out must be [b,oc,vn,2]"));
-  const VoteInput in{dl_data(m), mask_is_seg ? MaskForm::kSeg : MaskForm::kOneHot, dl_data(v), false, 0, nullptr, nullptr,
-                     (float*)dl_data(o)};
+  VoteInput in{dl_data(m), mask_is_seg ? MaskForm::kSeg : MaskForm::kOneHot, dl_data(v), false, 0, nullptr, nullptr,
+               (float*)dl_data(o)};
+  in.mask_dtype = mdt;
+  in.vertex_dtype = vdt;
   cudaStream_t ran_on;
   rc = ransac_vote_route(h, &q, in, nullptr, stream, &ran_on);
   // the capsules are consumed either way: their deleters run once the work queued so far where the vote ran has finished
@@ -1681,42 +1722,57 @@ struct LsGrad {
   float* grad_direct = nullptr;        // [b,h,w,2*vn]
   float* grad_conf = nullptr;          // [b,h,w,vn]
 };
-int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct, const float* conf,
+int ls_vote_impl(casa_handle* h, const casa_ls_params* p, casa_dtype dt, const void* seg, const void* direct, const void* conf,
                  float* out_points, const casa_ls_debug* debug, void* stream, const LsGrad* grad, int pix_capacity = 0);
 }  // namespace
 
-extern "C" int casa_ls_vote(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
-                            const float* conf, float* out_points, const casa_ls_debug* debug, void* stream) {
+extern "C" int casa_ls_vote_typed(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg, const void* direct,
+                                  const void* conf, float* out_points, const casa_ls_debug* debug, void* stream) {
   if (!h || !p) return fail(CASA_ERR_INVALID, "handle / params is NULL");
+  if (!dtype_ok(dtype)) return fail(CASA_ERR_INVALID, "dtype %d is not a casa_dtype", (int)dtype);
   if (!seg || !direct || !conf || !out_points) return fail(CASA_ERR_INVALID, "seg / direct / conf / out_points must not be NULL");
   if (h->async_mode >= 2 && !debug && !p->check_finite && !h->is_lane) {  // lanes, as for the votes (check_finite waits for the host)
     casa_handle* sub = nullptr;
     int k = 0;
     int rcl = lane_begin(h, h->async_mode, stream, &sub, &k);
     if (rcl) return rcl;
-    rcl = ls_vote_impl(sub, p, seg, direct, conf, out_points, nullptr, (void*)sub->own_stream, nullptr);
+    rcl = ls_vote_impl(sub, p, dtype, seg, direct, conf, out_points, nullptr, (void*)sub->own_stream, nullptr);
     const int rce = lane_end(h, k, stream);
     h->last_launches = sub->last_launches;
     return rcl ? rcl : rce;
   }
-  return ls_vote_impl(h, p, seg, direct, conf, out_points, debug, stream, nullptr);
+  return ls_vote_impl(h, p, dtype, seg, direct, conf, out_points, debug, stream, nullptr);
 }
 
-extern "C" int casa_ls_vote_backward(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
-                                     const float* conf, const float* grad_points, float* out_points, float* grad_direct,
-                                     float* grad_conf, void* stream) {
+extern "C" int casa_ls_vote(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
+                            const float* conf, float* out_points, const casa_ls_debug* debug, void* stream) {
+  return casa_ls_vote_typed(h, p, CASA_FLOAT32, seg, direct, conf, out_points, debug, stream);
+}
+
+extern "C" int casa_ls_vote_backward_typed(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg,
+                                           const void* direct, const void* conf, const float* grad_points, float* out_points,
+                                           float* grad_direct, float* grad_conf, void* stream) {
   if (!h || !p) return fail(CASA_ERR_INVALID, "handle / params is NULL");
+  if (!dtype_ok(dtype)) return fail(CASA_ERR_INVALID, "dtype %d is not a casa_dtype", (int)dtype);
   if (!seg || !direct || !conf || !grad_points || !grad_direct || !grad_conf)
     return fail(CASA_ERR_INVALID, "casa_ls_vote_backward: only out_points may be NULL");
   LsGrad g;
   g.grad_points = grad_points;
   g.grad_direct = grad_direct;
   g.grad_conf = grad_conf;
-  return ls_vote_impl(h, p, seg, direct, conf, out_points, nullptr, stream, &g);
+  return ls_vote_impl(h, p, dtype, seg, direct, conf, out_points, nullptr, stream, &g);
+}
+
+extern "C" int casa_ls_vote_backward(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
+                                     const float* conf, const float* grad_points, float* out_points, float* grad_direct,
+                                     float* grad_conf, void* stream) {
+  return casa_ls_vote_backward_typed(h, p, CASA_FLOAT32, seg, direct, conf, grad_points, out_points, grad_direct, grad_conf,
+                                     stream);
 }
 
 namespace {
-int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct, const float* conf,
+// dt: element type of seg, direct and conf (the input-reading kernels are instantiated per type; the rest is float32)
+int ls_vote_impl(casa_handle* h, const casa_ls_params* p, casa_dtype dt, const void* seg, const void* direct, const void* conf,
                  float* out_points, const casa_ls_debug* debug, void* stream, const LsGrad* grad, int pix_capacity) {
   if (p->num_classes < 2 || p->num_classes > 33) return fail(CASA_ERR_INVALID, "num_classes=%d outside 2..33", p->num_classes);
   casa_ransac_params rp;
@@ -1787,10 +1843,11 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
   steps.push_back(special(STEP_CLEAR));  // ctrl / stats: one memset node in front of the kernels
   {
     const size_t sm = (size_t)kCountTile * ld.nc * 4;
-    const void* classify = ld.nc == 9 ? (const void*)k_ls_classify<9> : (const void*)k_ls_classify<0>;
+    const void* classify = ld.nc == 9 ? by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<9, typename decltype(e)::type>; })
+                                      : by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<0, typename decltype(e)::type>; });
     // Without the opt-in, static plus dynamic shared memory of a block may not exceed 48 KB: the kernel's own counters
     // (scnt) count too, so nc = 12 (exactly 48 KB of staged logits) needs the attribute as well.
-    int& static_sm = h->classify_static_smem[ld.nc == 9 ? 0 : 1];
+    int& static_sm = h->classify_static_smem[dt][ld.nc == 9 ? 0 : 1];
     if (static_sm < 0) {
       cudaFuncAttributes fa;
       CUDA_TRY(cudaFuncGetAttributes(&fa, classify));
@@ -1799,7 +1856,7 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
     if (sm + (size_t)static_sm > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(classify, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
     steps.push_back(kstep(classify, dim3(d.nct, d.b), 256, sm).arg(seg).arg(ws).arg(d).arg(lw).arg(ld).arg((int)(runs_cc ? 1 : 0)));
   }
-  steps.push_back(kstep((const void*)k_place<0>, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg((const float*)nullptr).arg(ws).arg(d).arg((int)0));
+  steps.push_back(kstep((const void*)k_place<0, float>, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg((const float*)nullptr).arg(ws).arg(d).arg((int)0));
   // topology: the work-item / tile plan only needs the job table and runs beside the component chain (side branch)
   steps.push_back(kstep((const void*)k_plan, 1, d.J > 256 ? 1024 : 256).arg(ws).arg(d).arg((int)0).on_side(1));
   const int gx = (d.cap + 255) / 256 < 24 ? (d.cap + 255) / 256 : 24;
@@ -1814,18 +1871,23 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
   const int grid_x = d.max_rtiles < h->sm_count * 4 ? d.max_rtiles : h->sm_count * 4;
   if (grad) {
     // the backward pass reads the gathered directions / weights / confidences: the three-kernel form fills them
-    steps.push_back(kstep(d.vn == 9 ? (const void*)k_gather_dirs<18> : (const void*)k_gather_dirs<0>, dim3(gx, d.J), 256)
-                        .arg(direct).arg(ws).arg(d).arg((int)0).joins());
-    steps.push_back(kstep((const void*)k_ls_weights, dim3(gx, d.J), 256).arg(ws).arg(d).arg(lw).arg(ld).arg(seg).arg(conf));
+    steps.push_back(kstep(gather_dirs_fn(d.vn, dt), dim3(gx, d.J), 256).arg(direct).arg(ws).arg(d).arg((int)0).joins());
+    steps.push_back(kstep(by_dtype(dt, [](auto e) { return (const void*)k_ls_weights<typename decltype(e)::type>; }), dim3(gx, d.J), 256)
+                        .arg(ws).arg(d).arg(lw).arg(ld).arg(seg).arg(conf));
     steps.push_back(kstep((const void*)k_ls_reduce, dim3(grid_x, d.vn), 256).arg(ws).arg(d).arg(lw).arg(ld));
   } else {
-    if (h->fused_occ == 0) {
-      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->fused_occ, k_ls_fused<true>, 32 * d.vn, 0));
-      if (h->fused_occ < 1) h->fused_occ = 1;
+    int& occ = h->fused_occ[dt];
+    if (occ == 0) {
+      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
+          &occ, by_dtype(dt, [](auto e) { return (const void*)k_ls_fused<true, typename decltype(e)::type>; }), 32 * d.vn, 0));
+      if (occ < 1) occ = 1;
     }
-    const int fused_gx = d.max_rtiles < h->sm_count * h->fused_occ ? d.max_rtiles : h->sm_count * h->fused_occ;
-    // float2 loads of a pixel's (dy, dx) need an 8-byte aligned `direct`; callers may pass any 4-byte aligned buffer
-    const void* fused = (((uintptr_t)direct) & 7) == 0 ? (const void*)k_ls_fused<true> : (const void*)k_ls_fused<false>;
+    const int fused_gx = d.max_rtiles < h->sm_count * occ ? d.max_rtiles : h->sm_count * occ;
+    // one load of a pixel's (dy, dx) needs `direct` aligned to a pair (8 bytes, 4 for 16-bit types); callers may pass
+    // any buffer aligned to one element
+    const void* fused = (((uintptr_t)direct) & (2 * dtype_bytes(dt) - 1)) == 0
+                            ? by_dtype(dt, [](auto e) { return (const void*)k_ls_fused<true, typename decltype(e)::type>; })
+                            : by_dtype(dt, [](auto e) { return (const void*)k_ls_fused<false, typename decltype(e)::type>; });
     steps.push_back(kstep(fused, fused_gx, 32 * d.vn).arg(ws).arg(d).arg(lw).arg(ld).arg(seg).arg(direct).arg(conf)
                         .arg((int)(runs_cc ? 1 : 0)).joins());
   }
@@ -1868,7 +1930,7 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, const float* seg, cons
       CUDA_TRY(cudaMemset(h->sticky, 0, sizeof(uint32_t)));  // the retried call reports for itself
       if (need <= d.cap || need > (1ll << 30))
         return fail(CASA_ERR_WORKSPACE, "CoordLSVotingWeighted: pixel lists overflow (need %lld slots per image)", need);
-      return ls_vote_impl(h, p, seg, direct, conf, out_points == (float*)(base + off_tmp_out) ? nullptr : out_points, debug, stream, grad, (int)need);
+      return ls_vote_impl(h, p, dt, seg, direct, conf, out_points == (float*)(base + off_tmp_out) ? nullptr : out_points, debug, stream, grad, (int)need);
     }
     if (p->check_finite && (h->last_status & CASA_STATUS_LS_NONFINITE))
       return fail(CASA_ERR_INPUT, "CoordLSVotingWeighted: non-finite R / q / p (the reference asserts here, voting_layers_2d.py:109-121)");

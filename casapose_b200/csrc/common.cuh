@@ -1,11 +1,41 @@
 // Shared definitions of the casapose_b200 kernels (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "../../include/casapose_b200.h"
 
 namespace casa {
+
+// Element types of the network outputs the input-reading kernels take (casa_dtype): float, __half, __nv_bfloat16.
+// Every element is widened exactly to float32 at load; everything after the load is the float32 path, so a 16-bit
+// call computes what the float32 call computes on the upcast tensor.
+__device__ __forceinline__ float ld_f32(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_f32(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ float ld_f32(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+// (dy, dx) pairs: Pair<T>::type is the two-element vector of T, ld_pair loads one and widens it
+template <typename T> struct Pair;
+template <> struct Pair<float> { using type = float2; };
+template <> struct Pair<__half> { using type = __half2; };
+template <> struct Pair<__nv_bfloat16> { using type = __nv_bfloat162; };
+__device__ __forceinline__ float2 ld_pair(const float2* p) { return __ldg(p); }
+__device__ __forceinline__ float2 ld_pair(const __half2* p) { return __half22float2(__ldg(p)); }
+__device__ __forceinline__ float2 ld_pair(const __nv_bfloat162* p) { return __bfloat1622float2(__ldg(p)); }
+// element j of a 16-byte vector holding 16 / sizeof(T) elements of T
+__device__ __forceinline__ float vec_elem(const uint4& v, int j, const float*) {
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+  return __uint_as_float(w[j]);
+}
+__device__ __forceinline__ float vec_elem(const uint4& v, int j, const __half*) {
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+  return __half2float(__ushort_as_half((unsigned short)(w[j >> 1] >> (16 * (j & 1)))));
+}
+__device__ __forceinline__ float vec_elem(const uint4& v, int j, const __nv_bfloat16*) {
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+  return __uint_as_float((j & 1) ? (w[j >> 1] & 0xFFFF0000u) : (w[j >> 1] << 16));
+}
 
 constexpr int kCountTile = 1024;   // pixels per block in the mask / scatter kernels (256 thr x 4)
 constexpr int kScoreWarps = 8;     // warps per scoring block

@@ -3,7 +3,7 @@
 // Replaces  coords = reverse(where(mask != 0)) + 0.5 ; direct = boolean_mask(vertex, mask)
 // (/root/reference/casapose/pose_estimation/ransac_voting.py:287-308) for all (image, class)
 // pairs of the batch at once:
-//   k_mask_bits   reads the float mask ONCE (the only pass over [b,h,w,oc]), writes one
+//   k_mask_bits   reads the mask ONCE (float32, float16 or bfloat16; the only pass over [b,h,w,oc]), writes one
 //                 class-membership word per pixel and per-tile class counts (warp ballots);
 //   k_place       job table (class offsets, foreground_num gate :290, down-sampling threshold :298), raster-order
 //                 scatter of packed pixel coordinates (y<<16 | x) — the order is semantically required because
@@ -18,47 +18,50 @@
 
 namespace casa {
 
-// Vectorised path (tile slab 16-byte aligned, i.e. (h*w*oc) % 4 == 0 and an aligned base): the block streams its
-// tile's [1024 x oc] floats as one contiguous run of 128-bit loads — every warp-load is 512 contiguous bytes,
-// all oc loads of a thread are independent and in flight together (this matters when `mask` is mapped pinned
-// host memory: full-line PCIe reads) — and ORs the few non-zero elements into a shared-memory word per pixel.
-__global__ void __launch_bounds__(256) k_mask_bits(const float* __restrict__ mask, WS ws, Dims d, int vec4) {
+// Vectorised path (tile slab 16-byte aligned, i.e. (h*w*oc) % (16 / sizeof(T)) == 0 and an aligned base): the block
+// streams its tile's [1024 x oc] elements as one contiguous run of 128-bit loads (4 floats or 8 16-bit values) — every
+// warp-load is 512 contiguous bytes, all loads of a thread are independent and in flight together (this matters when
+// `mask` is mapped pinned host memory: full-line PCIe reads) — and ORs the few non-zero elements into a shared-memory
+// word per pixel.
+template <typename T>  // float, __half or __nv_bfloat16
+__global__ void __launch_bounds__(256) k_mask_bits(const T* __restrict__ mask, WS ws, Dims d, int vec) {
+  constexpr int kPerVec = 16 / sizeof(T);  // elements per 128-bit load
   const int img = blockIdx.y, tile = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31;
   __shared__ int scnt[32];
   __shared__ unsigned sbits[kCountTile];
   if (tid < 32) scnt[tid] = 0;
-  const float* mimg = mask + (size_t)img * d.hw * d.oc;
+  const T* mimg = mask + (size_t)img * d.hw * d.oc;
   const int p0 = tile * kCountTile;
   const int npx = min(kCountTile, d.hw - p0);
   bool bad = false;
   uint32_t m[4] = {0u, 0u, 0u, 0u};
-  if (vec4) {
+  if (vec) {
 #pragma unroll
     for (int k = 0; k < 4; ++k) sbits[k * 256 + tid] = 0u;
     __syncthreads();
-    const float4* slab = reinterpret_cast<const float4*>(mimg + (size_t)p0 * d.oc);
-    const int n4 = npx * d.oc / 4;  // npx*oc is a multiple of 4 on this path
-    for (int i0 = 0; i0 < n4; i0 += 256 * 8) {
-      float4 v[8];
+    const uint4* slab = reinterpret_cast<const uint4*>(mimg + (size_t)p0 * d.oc);
+    const int nv = npx * d.oc / kPerVec;  // npx*oc is a multiple of kPerVec on this path
+    for (int i0 = 0; i0 < nv; i0 += 256 * 8) {
+      uint4 v[8];
 #pragma unroll
       for (int u = 0; u < 8; ++u) {
         const int i = i0 + u * 256 + tid;
-        v[u] = i < n4 ? __ldg(slab + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[u] = i < nv ? __ldg(slab + i) : make_uint4(0u, 0u, 0u, 0u);
       }
 #pragma unroll
       for (int u = 0; u < 8; ++u) {
-        const float f[4] = {v[u].x, v[u].y, v[u].z, v[u].w};
-        // seven of eight elements of a one-hot mask are +0: test the four bit patterns at once (-0 and NaN are
-        // non-zero patterns and take the per-element path below)
-        if (((__float_as_uint(f[0]) | __float_as_uint(f[1])) | (__float_as_uint(f[2]) | __float_as_uint(f[3]))) == 0u) continue;
-        const int e0 = (i0 + u * 256 + tid) * 4;
+        // most elements of a one-hot mask are +0: test the four 32-bit words at once (-0 and NaN are non-zero
+        // patterns and take the per-element path below)
+        if (((v[u].x | v[u].y) | (v[u].z | v[u].w)) == 0u) continue;
+        const int e0 = (i0 + u * 256 + tid) * kPerVec;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          if (f[j] != 0.f) {  // NaN != 0 is true, like tf.not_equal (:304)
+        for (int j = 0; j < kPerVec; ++j) {
+          const float f = vec_elem(v[u], j, mask);
+          if (f != 0.f) {  // NaN != 0 is true, like tf.not_equal (:304)
             const int e = e0 + j, px = e / d.oc;
             atomicOr(&sbits[px], 1u << (e - px * d.oc));
-            bad |= f[j] != 1.f;
+            bad |= f != 1.f;
           }
         }
       }
@@ -71,9 +74,9 @@ __global__ void __launch_bounds__(256) k_mask_bits(const float* __restrict__ mas
     for (int k = 0; k < 4; ++k) {
       const int p = p0 + k * 256 + tid;
       if (p < d.hw) {
-        const float* row = mimg + (size_t)p * d.oc;
+        const T* row = mimg + (size_t)p * d.oc;
         for (int c = 0; c < d.oc; ++c) {
-          const float v = __ldg(row + c);
+          const float v = ld_f32(row + c);
           m[k] |= (uint32_t)(v != 0.f) << c;
           bad |= (v != 0.f && v != 1.f);
         }
@@ -130,7 +133,8 @@ __global__ void __launch_bounds__(256) k_bits_in(const uint32_t* __restrict__ sr
 
 // Fused pre-step (pose_evaluation.py:36-47): bit c of a pixel is set iff argmax(seg) == c + 1
 // (tf.argmax takes the first maximum; NaN scores never win, like Eigen's comparison-based arg-max).
-__global__ void __launch_bounds__(256) k_seg_bits(const float* __restrict__ seg, WS ws, Dims d) {
+template <typename T>
+__global__ void __launch_bounds__(256) k_seg_bits(const T* __restrict__ seg, WS ws, Dims d) {
   const int img = blockIdx.y, tile = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31;
   const int nc = d.oc + 1;
@@ -142,11 +146,11 @@ __global__ void __launch_bounds__(256) k_seg_bits(const float* __restrict__ seg,
     const int p = tile * kCountTile + k * 256 + tid;
     uint32_t m = 0;
     if (p < d.hw) {
-      const float* row = seg + ((size_t)img * d.hw + p) * nc;
-      float best = __ldg(row);
+      const T* row = seg + ((size_t)img * d.hw + p) * nc;
+      float best = ld_f32(row);
       int arg = 0;
       for (int c = 1; c < nc; ++c) {
-        const float v = __ldg(row + c);
+        const float v = ld_f32(row + c);
         if (v > best) {
           best = v;
           arg = c;
@@ -178,8 +182,9 @@ __global__ void __launch_bounds__(256) k_seg_bits(const float* __restrict__ seg,
 //     keypoint-major direction buffer at the same list position (direct = boolean_mask(vertex, mask), :308).  Jobs
 //     above max_num are gathered after k_cap_filter (k_gather_dirs, only_capped), gated jobs never.
 constexpr int kPlaceSub = 4;  // count tiles per k_place block (4096 pixels, 16 per thread)
-template <int VN>             // keypoints per row when known at compile time (9), 0 = runtime
-__global__ void __launch_bounds__(256, 4) k_place(const float* __restrict__ vertex, WS ws, Dims d, int gather) {
+// T: element type of `vertex`; gather requires it aligned to one (dy, dx) pair.
+template <int VN, typename T>  // keypoints per row when known at compile time (9), 0 = runtime
+__global__ void __launch_bounds__(256, 4) k_place(const T* __restrict__ vertex, WS ws, Dims d, int gather) {
   const int img = blockIdx.y, tile0 = blockIdx.x * kPlaceSub;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int kSlots = kPlaceSub * 4;  // pixels per thread; slot j covers pixels [j*256, (j+1)*256) of the block
@@ -303,7 +308,8 @@ __global__ void __launch_bounds__(256, 4) k_place(const float* __restrict__ vert
     const int tbase = s_pre[c];
     uint32_t* out = ws.pix + (size_t)img * d.cap + s_off[c];
     const bool dirs = gather && !(flags & (JOB_GATED | JOB_NEEDS_CAP));
-    const float2* vfield = reinterpret_cast<const float2*>(vertex) + (size_t)img * d.hw * vslots + (d.vpc > 1 ? c * vn : 0);
+    using P = typename Pair<T>::type;
+    const P* vfield = reinterpret_cast<const P*>(vertex) + (size_t)img * d.hw * vslots + (d.vpc > 1 ? c * vn : 0);
     float2* dst0 = ws.vdir + ((size_t)img * d.cap + s_off[c]) * vn;
 #pragma unroll
     for (int j = 0; j < kSlots; ++j) {
@@ -315,15 +321,15 @@ __global__ void __launch_bounds__(256, 4) k_place(const float* __restrict__ vert
         const int slot = tbase + wcnt[c][j * 8 + warp] + __popc(bal & lanemask_lt());
         out[slot] = ((uint32_t)y << 16) | (uint32_t)x;
         if (dirs) {
-          const float2* row = vfield + (size_t)p * vslots;
+          const P* row = vfield + (size_t)p * vslots;
           if (VN) {
             float2 r[VN ? VN : 1];
 #pragma unroll
-            for (int v = 0; v < VN; ++v) r[v] = __ldg(row + v);
+            for (int v = 0; v < VN; ++v) r[v] = ld_pair(row + v);
 #pragma unroll
             for (int v = 0; v < VN; ++v) dst0[(size_t)v * tn + slot] = r[v];
           } else {
-            for (int v = 0; v < vn; ++v) dst0[(size_t)v * tn + slot] = __ldg(row + v);
+            for (int v = 0; v < vn; ++v) dst0[(size_t)v * tn + slot] = ld_pair(row + v);
           }
         }
       }
@@ -382,16 +388,16 @@ __global__ void __launch_bounds__(1024) k_cap_filter(WS ws, Dims d, const float*
 // the class's own field, pose_evaluation.py:38-45).  One thread per listed pixel: the pixel's 8*vn-byte
 // row is read once (the only access to `vertex`, which may be device memory or mapped pinned host
 // memory — then only masked pixels of the field cross PCIe), the writes are coalesced per keypoint.
-template <int ROWF>  // floats per pixel row when known at compile time (18 for vn = 9), 0 = runtime
-__global__ void __launch_bounds__(256) k_gather_dirs(const float* __restrict__ vertex, WS ws, Dims d, int only_capped) {
+template <int ROWF, typename T>  // elements per pixel row when known at compile time (18 for vn = 9), 0 = runtime
+__global__ void __launch_bounds__(256) k_gather_dirs(const T* __restrict__ vertex, WS ws, Dims d, int only_capped) {
   const int job = blockIdx.y, img = job / d.oc, cls = job - img * d.oc;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int tn = ws.job_tn[job];
   if (tn <= 0 || (ws.job_flags[job] & JOB_GATED)) return;
   if (only_capped && !(ws.job_flags[job] & JOB_NEEDS_CAP)) return;  // the others were gathered by k_place
   const int vslots = d.vn * d.vpc;
-  const int rowf = ROWF ? ROWF : 2 * d.vn;  // floats fetched per pixel (<= 32)
-  const float* vfield = vertex + (size_t)img * d.hw * vslots * 2 + (d.vpc > 1 ? cls * d.vn * 2 : 0);
+  const int rowf = ROWF ? ROWF : 2 * d.vn;  // elements fetched per pixel (<= 32)
+  const T* vfield = vertex + (size_t)img * d.hw * vslots * 2 + (d.vpc > 1 ? cls * d.vn * 2 : 0);
   const int off = ws.job_off[job];
   const uint32_t* pix = ws.pix + (size_t)img * d.cap + off;
   float2* dst0 = ws.vdir + ((size_t)img * d.cap + off) * d.vn;
@@ -404,8 +410,8 @@ __global__ void __launch_bounds__(256) k_gather_dirs(const float* __restrict__ v
       const uint32_t pk = pix[t];
       px = (int)((pk >> 16) * (uint32_t)d.w + (pk & 0xFFFFu));
     }
-    // flattened fetch: element e = lane + 32 k of the warp's [32 pixels x rowf floats] block.  Consecutive
-    // lanes read consecutive floats of one row and run on into the next pixel's row, which is contiguous in
+    // flattened fetch: element e = lane + 32 k of the warp's [32 pixels x rowf elements] block.  Consecutive
+    // lanes read consecutive elements of one row and run on into the next pixel's row, which is contiguous in
     // memory whenever the two pixels are neighbours — so most warp-loads are one full 128-byte line, and all
     // rowf loads of a lane are independent (no per-pixel serialisation).  The row offset px * vn * vpc * 2 is
     // formed in 64 bits: it reaches 2^31 from pixel 2^26 on for a shared field with vn = 16, and from pixel 2^21
@@ -415,7 +421,7 @@ __global__ void __launch_bounds__(256) k_gather_dirs(const float* __restrict__ v
       const int e = k * 32 + lane;
       const int src = e / rowf, f = e - src * rowf;
       const int sp = __shfl_sync(0xffffffffu, px, src);
-      if (sp >= 0) srow[warp][src][f] = __ldg(vfield + (size_t)sp * (vslots * 2) + f);
+      if (sp >= 0) srow[warp][src][f] = ld_f32(vfield + (size_t)sp * (vslots * 2) + f);
     }
     __syncwarp();
     if (t < tn)

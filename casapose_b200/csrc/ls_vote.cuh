@@ -103,11 +103,23 @@ __device__ __forceinline__ float hot_of_row(const float* row, int nc, int cls) {
 // same tiling and outputs as k_mask_bits (compaction.cuh), fed by the segmentation logits: the tile's
 // [1024 x nc] floats are staged in shared memory with coalesced loads, then every thread classifies 4 pixels
 // NC: classes when known at compile time (9: fully unrolled rows, all loads of the tile in flight), 0 = runtime.
+// T: element type of `seg`, widened to float while it is staged (128-bit loads when the slab is 16-byte aligned).
 // flag_onehot (forward call): cls9 bit 7 marks pixels whose softmax is exactly one-hot, so that the reduction need not
 // read their logits again.
 extern __shared__ __align__(16) float ls_smem[];
-template <int NC>
-__global__ void __launch_bounds__(256) k_ls_classify(const float* __restrict__ seg, WS ws, Dims d, LsWS lw, LsDims ld, int flag_onehot) {
+// 16 bytes of T, widened, into the float tile at vector index i (4 floats, or 8 values of a 16-bit type)
+__device__ __forceinline__ void stage16(float4* sm4, int i, const uint4& v, const float*) {
+  sm4[i] = make_float4(__uint_as_float(v.x), __uint_as_float(v.y), __uint_as_float(v.z), __uint_as_float(v.w));
+}
+template <typename T>
+__device__ __forceinline__ void stage16(float4* sm4, int i, const uint4& v, const T* t) {
+  sm4[2 * i] = make_float4(vec_elem(v, 0, t), vec_elem(v, 1, t), vec_elem(v, 2, t), vec_elem(v, 3, t));
+  sm4[2 * i + 1] = make_float4(vec_elem(v, 4, t), vec_elem(v, 5, t), vec_elem(v, 6, t), vec_elem(v, 7, t));
+}
+
+template <int NC, typename T>
+__global__ void __launch_bounds__(256) k_ls_classify(const T* __restrict__ seg, WS ws, Dims d, LsWS lw, LsDims ld, int flag_onehot) {
+  constexpr int kPerVec = 16 / sizeof(T);  // elements per 128-bit load
   const int img = blockIdx.y, tile = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31;
   const int nc = NC ? NC : ld.nc;
@@ -115,22 +127,30 @@ __global__ void __launch_bounds__(256) k_ls_classify(const float* __restrict__ s
   if (tid < 32) scnt[tid] = 0;
   const int p0 = tile * kCountTile;
   const int npx = min(kCountTile, d.hw - p0);
-  const float* slab = seg + ((size_t)img * d.hw + p0) * nc;
+  const T* slab = seg + ((size_t)img * d.hw + p0) * nc;
   const int nfl = npx * nc;
-  if (((nfl | (int)(((size_t)img * d.hw + p0) * nc)) & 3) == 0 && (reinterpret_cast<uintptr_t>(seg) & 15) == 0) {
-    const float4* slab4 = reinterpret_cast<const float4*>(slab);  // 16-byte aligned slab: 128-bit loads
+  if (((nfl | (int)(((size_t)img * d.hw + p0) * nc)) & (kPerVec - 1)) == 0 && (reinterpret_cast<uintptr_t>(seg) & 15) == 0) {
+    const uint4* slab4 = reinterpret_cast<const uint4*>(slab);  // 16-byte aligned slab: 128-bit loads
     float4* sm4 = reinterpret_cast<float4*>(ls_smem);
-    if (NC && npx == kCountTile) {  // NC float4 per thread, all in flight before the first store
-      float4 v[NC ? NC : 1];
+    if (NC && npx == kCountTile) {  // the whole tile per thread in flight before the first store
+      constexpr int kVecs = NC * kCountTile / kPerVec;  // 128-bit loads of the tile
+      constexpr int kU = (kVecs + 255) / 256;
+      uint4 v[NC ? kU : 1];
 #pragma unroll
-      for (int u = 0; u < NC; ++u) v[u] = __ldg(slab4 + u * 256 + tid);
+      for (int u = 0; u < kU; ++u) {
+        const int i = u * 256 + tid;
+        if (kU * 256 == kVecs || i < kVecs) v[u] = __ldg(slab4 + i);
+      }
 #pragma unroll
-      for (int u = 0; u < NC; ++u) sm4[u * 256 + tid] = v[u];
+      for (int u = 0; u < kU; ++u) {
+        const int i = u * 256 + tid;
+        if (kU * 256 == kVecs || i < kVecs) stage16(sm4, i, v[u], seg);
+      }
     } else {
-      for (int i = tid; i < nfl / 4; i += 256) sm4[i] = __ldg(slab4 + i);
+      for (int i = tid; i < nfl / kPerVec; i += 256) stage16(sm4, i, __ldg(slab4 + i), seg);
     }
   } else {
-    for (int i = tid; i < nfl; i += 256) ls_smem[i] = __ldg(slab + i);
+    for (int i = tid; i < nfl; i += 256) ls_smem[i] = ld_f32(slab + i);
   }
   __syncthreads();
 #pragma unroll
@@ -577,8 +597,9 @@ __device__ __forceinline__ float ls_weight(float x, int sigmoid_weights) {
 
 // One thread per listed pixel of a job: weight = hot_seg * component mask (:39-41, :72-79), and the pixel's
 // confidence row turned into softplus / sigmoid weights (:32-35), stored keypoint-major like the directions.
-__global__ void __launch_bounds__(256) k_ls_weights(WS ws, Dims d, LsWS lw, LsDims ld, const float* __restrict__ seg,
-                                                    const float* __restrict__ conf) {
+template <typename T>
+__global__ void __launch_bounds__(256) k_ls_weights(WS ws, Dims d, LsWS lw, LsDims ld, const T* __restrict__ seg,
+                                                    const T* __restrict__ conf) {
   const int job = blockIdx.y, img = job / d.oc, c = job - img * d.oc;
   const int tn = ws.job_tn[job];
   if (tn <= 0) return;
@@ -592,7 +613,7 @@ __global__ void __launch_bounds__(256) k_ls_weights(WS ws, Dims d, LsWS lw, LsDi
     const int x = pk & 0xFFFFu, y = pk >> 16;
     const size_t p = (size_t)img * ld.hw + (size_t)y * ld.w + x;
     float row[33];
-    for (int k = 0; k < ld.nc; ++k) row[k] = __ldg(seg + p * ld.nc + k);
+    for (int k = 0; k < ld.nc; ++k) row[k] = ld_f32(seg + p * ld.nc + k);
     float w = hot_of_row(row, ld.nc, c + 1);  // hot_seg (:39-41)
     if (ld.filter) {                          // copy_components * hot_seg (:72-79)
       const int c9 = lw.cls9[p];
@@ -602,7 +623,7 @@ __global__ void __launch_bounds__(256) k_ls_weights(WS ws, Dims d, LsWS lw, LsDi
     wt[t] = w;
     // dropped pixels (weight 0) get defined zeros: k_ls_reduce loads the entry before it looks at the weight
     for (int v = 0; v < d.vn; ++v)
-      cc[(size_t)v * tn + t] = w != 0.f ? ls_weight(__ldg(conf + p * ld.vn + v), ld.sigmoid_weights) : 0.f;
+      cc[(size_t)v * tn + t] = w != 0.f ? ls_weight(ld_f32(conf + p * ld.vn + v), ld.sigmoid_weights) : 0.f;
   }
 }
 
@@ -685,12 +706,13 @@ __global__ void __launch_bounds__(256) k_ls_reduce(WS ws, Dims d, LsWS lw, LsDim
 //                          go through the reference's float32 element-wise sequence (:89-108) into float64 sums.
 // Replaces k_gather_dirs + k_ls_weights + k_ls_reduce (102 us of launches and 140 MB of intermediates per 16 frames)
 // for the forward call; the backward pass still uses the gathered arrays.
-// VEC (chosen on the host from the pointer): `direct` is 8-byte aligned and a pixel's (dy, dx) is one float2 load;
-// otherwise (e.g. a view 4 bytes into an allocation) two scalar loads of the same floats.
+// VEC (chosen on the host from the pointer): `direct` is aligned to one (dy, dx) pair (8 bytes for float, 4 for the
+// 16-bit types) and a pixel's pair is one load; otherwise (e.g. a view one element into an allocation) two scalar loads.
+// T: element type of seg, direct and conf.
 constexpr int kFusedTile = 512;  // list entries per tile of k_ls_fused (d.rtile of the forward call)
-template <bool VEC>
-__global__ void __launch_bounds__(512, 2) k_ls_fused(WS ws, Dims d, LsWS lw, LsDims ld, const float* __restrict__ seg,
-                                                  const float* __restrict__ direct, const float* __restrict__ conf,
+template <bool VEC, typename T>
+__global__ void __launch_bounds__(512, 2) k_ls_fused(WS ws, Dims d, LsWS lw, LsDims ld, const T* __restrict__ seg,
+                                                  const T* __restrict__ direct, const T* __restrict__ conf,
                                                   int use_keep) {
   const int tid = threadIdx.x, lane = tid & 31, v = tid >> 5;
   const int n_rtiles = ws.rtile_start[d.J];
@@ -719,7 +741,7 @@ __global__ void __launch_bounds__(512, 2) k_ls_fused(WS ws, Dims d, LsWS lw, LsD
         w = c9 == c + 1 ? 1.0f : 0.0f;
       } else {
         float row[33];
-        for (int q = 0; q < ld.nc; ++q) row[q] = __ldg(seg + p * ld.nc + q);
+        for (int q = 0; q < ld.nc; ++q) row[q] = ld_f32(seg + p * ld.nc + q);
         w = hot_of_row(row, ld.nc, c + 1);  // hot_seg (:39-41)
       }
       if (ld.filter) {                          // copy_components * hot_seg (:72-79)
@@ -749,13 +771,13 @@ __global__ void __launch_bounds__(512, 2) k_ls_fused(WS ws, Dims d, LsWS lw, LsD
         bc[j] = 0.f;
         if (bw[j] != 0.f) {
           const size_t p = (size_t)img * ld.hw + (size_t)(bp[j] >> 16) * ld.w + (bp[j] & 0xFFFFu);
-          if (VEC) {
-            bd[j] = __ldg(reinterpret_cast<const float2*>(direct + p * (size_t)(2 * d.vn)) + v);  // (n0, n1) = (dy, dx)
+          if (VEC) {  // (n0, n1) = (dy, dx)
+            bd[j] = ld_pair(reinterpret_cast<const typename Pair<T>::type*>(direct + p * (size_t)(2 * d.vn)) + v);
           } else {
-            const float* dp = direct + p * (size_t)(2 * d.vn) + 2 * v;
-            bd[j] = make_float2(__ldg(dp), __ldg(dp + 1));
+            const T* dp = direct + p * (size_t)(2 * d.vn) + 2 * v;
+            bd[j] = make_float2(ld_f32(dp), ld_f32(dp + 1));
           }
-          bc[j] = __ldg(conf + p * (size_t)d.vn + v);
+          bc[j] = ld_f32(conf + p * (size_t)d.vn + v);
         }
       }
 #pragma unroll

@@ -9,7 +9,7 @@ import ctypes as C
 import torch
 
 from .. import _lib
-from .._carrier import as_cuda, as_cuda_f32, current_stream_ptr, ptr
+from .._carrier import as_cuda, as_cuda_f32, as_cuda_float, current_stream_ptr, ptr
 
 DEBUG_FIELDS = ("tn0", "tn", "rounds", "counts", "win_idx", "hyps", "win_pts", "win_ratio", "ata", "atb",
                 "refined", "pix", "pix_off", "stats")
@@ -46,7 +46,8 @@ def ransac_voting_layer_all_masks(
     out=None,
 ):
     """
-    :param mask:      [b,h,w,oc]   float32 {0,1}
+    :param mask:      [b,h,w,oc]   float32 {0,1}   (mask and vertex may also be float16 or bfloat16, each its own; the
+                      16-bit values are read natively and widened exactly, so the result equals the call on .float())
                       (seg_scores=True: [b,h,w,1+oc] segmentation scores; the one-hot of their arg-max without
                       the background channel is used, pose_evaluation.py:36-51, without materialising it)
     :param vertex:    [b,h,w,vn,2] float32 (dy,dx)   (a [b,h,w,vn*2] tensor is viewed as such;
@@ -55,8 +56,8 @@ def ransac_voting_layer_all_masks(
     :param out:       optional preallocated [b,oc,vn,2] float32 result tensor on the inputs' device
     :return: [b,oc,vn,2] float32 (x,y) — and a dict of intermediates if return_debug
     """
-    mask = as_cuda_f32(mask, "mask")
-    vertex = as_cuda_f32(vertex, "vertex")
+    mask, mask_dt = as_cuda_float(mask, "mask")
+    vertex, vertex_dt = as_cuda_float(vertex, "vertex")
     if mask.dim() != 4:
         raise ValueError("mask must be [b,h,w,oc], got %s" % (tuple(mask.shape),))
     b, h, w, oc = mask.shape
@@ -118,17 +119,18 @@ def ransac_voting_layer_all_masks(
         dbg_struct = _lib.RansacDebug(**{k: ptr(dbg.get(k)) for k in DEBUG_FIELDS})
     hdl = _lib.handle(dev.index if dev.index is not None else torch.cuda.current_device(), current_stream_ptr(dev))
     with torch.cuda.device(dev):
-        fn = _lib.lib().casa_ransac_vote_seg if seg_scores else _lib.lib().casa_ransac_vote
-        rc = fn(
-            hdl, C.byref(p), ptr(mask), ptr(vertex), ptr(idxs), ptr(selection), ptr(out),
-            C.byref(dbg_struct) if dbg_struct is not None else None, current_stream_ptr(dev))
+        def fn(dbg_arg):
+            return _lib.lib().casa_ransac_vote_typed(hdl, C.byref(p), int(bool(seg_scores)), mask_dt, ptr(mask), vertex_dt,
+                                                     ptr(vertex), ptr(idxs), ptr(selection), ptr(out), dbg_arg,
+                                                     current_stream_ptr(dev))
+
+        rc = fn(C.byref(dbg_struct) if dbg_struct is not None else None)
         if rc == -3 and pix_capacity == 0 and not return_debug:
             # CASA_ERR_WORKSPACE: channels that overlap list a pixel more than once and h*w slots per image are not
             # enough.  The reference treats every channel independently (ransac_voting.py:458-470), so the call is
             # repeated with room for every channel (synchronous calls only: an asynchronous one reports at casa_sync).
             p.pix_capacity = oc * h * w
-            rc = fn(hdl, C.byref(p), ptr(mask), ptr(vertex), ptr(idxs), ptr(selection), ptr(out), None,
-                    current_stream_ptr(dev))
+            rc = fn(None)
     _lib.check(rc)
     if return_debug:
         st = C.c_uint32()

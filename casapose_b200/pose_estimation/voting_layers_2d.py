@@ -10,13 +10,18 @@ Same constructor and call convention as the reference Keras layer
 The body is one call into the sm_100a library (casa_ls_vote); there is no CPU / PyTorch fallback.
 The gradient w.r.t. `direct` and `w` (what TensorFlow's autodiff gives the reference in
 train_casapose.py:536-595; `seg` is behind stop_gradient) is casa_ls_vote_backward: `layer.backward(inp,
-grad_out)`, or transparently through torch.autograd when `direct` / `w` are torch tensors that require grad."""
+grad_out)`, or transparently through torch.autograd when `direct` / `w` are torch tensors that require grad.
+
+seg, direct and w may be float32, float16 or bfloat16 (one dtype for all three: they are splits of one network
+output).  16-bit inputs are read natively and widened exactly, so outputs equal the call on the .float() tensors.
+`layer.backward` returns float32 gradients for every input dtype; through autograd a 16-bit leaf receives its
+gradient in its own dtype (the float32 gradient rounded once)."""
 import ctypes as C
 
 import torch
 
 from .. import _lib
-from .._carrier import as_cuda_f32, current_stream_ptr, ptr
+from .._carrier import as_cuda_f32, as_cuda_float, current_stream_ptr, ptr
 
 
 class _LsVoteFn(torch.autograd.Function):
@@ -32,7 +37,7 @@ class _LsVoteFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         seg, direct, w = ctx.saved_tensors
         gd, gw = ctx.layer.backward([seg, direct, w], grad_out)
-        return None, None, gd.reshape(direct.shape), gw
+        return None, None, gd.reshape(direct.shape).to(direct.dtype), gw.to(w.dtype)
 
 
 class CoordLSVotingWeighted:
@@ -62,9 +67,11 @@ class CoordLSVotingWeighted:
         return self._forward(seg, direct, w, return_debug, check_finite)
 
     def _prepare(self, seg, direct, w):
-        seg = as_cuda_f32(seg, "seg")
-        direct = as_cuda_f32(direct, "direct")
-        w = as_cuda_f32(w, "w")
+        seg, dt = as_cuda_float(seg, "seg")
+        direct, dt_direct = as_cuda_float(direct, "direct")
+        w, dt_w = as_cuda_float(w, "w")
+        if not dt == dt_direct == dt_w:
+            raise TypeError("seg, direct and w must share one dtype, got %s, %s, %s" % (seg.dtype, direct.dtype, w.dtype))
         if seg.dim() != 4:
             raise ValueError("seg must be [b,h,w,num_classes], got %s" % (tuple(seg.shape),))
         b, h, wd, nc = seg.shape
@@ -77,7 +84,7 @@ class CoordLSVotingWeighted:
             direct = direct.reshape(b, h, wd, 2 * vn)
         if tuple(direct.shape) != (b, h, wd, 2 * vn) or tuple(w.shape) != (b, h, wd, vn):
             raise ValueError("direct must be [b,h,w,%d] and w [b,h,w,%d]" % (2 * vn, vn))
-        return seg, direct, w, (b, h, wd, nc, vn)
+        return seg, direct, w, (b, h, wd, nc, vn), dt
 
     def _params(self, b, h, wd, nc, vn, check_finite):
         return _lib.LsParams(b=b, h=h, w=wd, num_classes=nc, vn=vn, sigmoid_weights=int(bool(self.sigmoid_weights)),
@@ -86,8 +93,9 @@ class CoordLSVotingWeighted:
                              check_finite=int(bool(check_finite)))
 
     def backward(self, inp, grad_out):
-        """(dL/d direct [b,h,w,2*vn], dL/d w [b,h,w,vn]) for dL/d output = grad_out [b,oc,vn,2] — casa_ls_vote_backward."""
-        seg, direct, w, (b, h, wd, nc, vn) = self._prepare(*[t.detach() if isinstance(t, torch.Tensor) else t for t in inp])
+        """(dL/d direct [b,h,w,2*vn], dL/d w [b,h,w,vn]) for dL/d output = grad_out [b,oc,vn,2] — casa_ls_vote_backward.
+        Both are float32 whatever the inputs' dtype."""
+        seg, direct, w, (b, h, wd, nc, vn), dt = self._prepare(*[t.detach() if isinstance(t, torch.Tensor) else t for t in inp])
         grad_out = as_cuda_f32(grad_out.contiguous() if isinstance(grad_out, torch.Tensor) else grad_out, "grad_out")
         if tuple(grad_out.shape) != (b, nc - 1, vn, 2):
             raise ValueError("grad_out must be [b,%d,%d,2]" % (nc - 1, vn))
@@ -97,13 +105,13 @@ class CoordLSVotingWeighted:
         p = self._params(b, h, wd, nc, vn, False)
         hdl = _lib.handle(dev.index if dev.index is not None else torch.cuda.current_device(), current_stream_ptr(dev))
         with torch.cuda.device(dev):
-            rc = _lib.lib().casa_ls_vote_backward(hdl, C.byref(p), ptr(seg), ptr(direct), ptr(w), ptr(grad_out), None, ptr(gd),
-                                                  ptr(gw), current_stream_ptr(dev))
+            rc = _lib.lib().casa_ls_vote_backward_typed(hdl, C.byref(p), dt, ptr(seg), ptr(direct), ptr(w), ptr(grad_out), None,
+                                                        ptr(gd), ptr(gw), current_stream_ptr(dev))
         _lib.check(rc)
         return gd, gw
 
     def _forward(self, seg, direct, w, return_debug, check_finite):
-        seg, direct, w, (b, h, wd, nc, vn) = self._prepare(seg, direct, w)
+        seg, direct, w, (b, h, wd, nc, vn), dt = self._prepare(seg, direct, w)
         dev = seg.device
         out = torch.empty((b, nc - 1, vn, 2), dtype=torch.float32, device=dev)
         p = self._params(b, h, wd, nc, vn, check_finite)
@@ -120,7 +128,7 @@ class CoordLSVotingWeighted:
             dbg_struct = _lib.LsDebug(**{k: ptr(v) for k, v in dbg.items()})
         hdl = _lib.handle(dev.index if dev.index is not None else torch.cuda.current_device(), current_stream_ptr(dev))
         with torch.cuda.device(dev):
-            rc = _lib.lib().casa_ls_vote(hdl, C.byref(p), ptr(seg), ptr(direct), ptr(w), ptr(out),
-                                         C.byref(dbg_struct) if dbg_struct is not None else None, current_stream_ptr(dev))
+            rc = _lib.lib().casa_ls_vote_typed(hdl, C.byref(p), dt, ptr(seg), ptr(direct), ptr(w), ptr(out),
+                                               C.byref(dbg_struct) if dbg_struct is not None else None, current_stream_ptr(dev))
         _lib.check(rc)
         return (out, dbg) if return_debug else out

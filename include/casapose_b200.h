@@ -13,6 +13,8 @@
  *     last failure on the calling thread is casa_last_error().  No exception crosses.
  *   - all tensors are dense, C-contiguous, float32 NHWC exactly like the reference's
  *     tensors; the caller owns inputs and outputs, the library never frees them.
+ *     The *_typed entry points also read the network outputs (mask / seg, vertex, direct,
+ *     conf) as float16 or bfloat16 (casa_dtype); outputs and gradients stay float32.
  *   - `stream` is a cudaStream_t passed as void* (0 = legacy default stream).
  *   - a handle is bound to one device, owns the workspace, and is not thread-safe;
  *     use one handle per stream / thread.
@@ -46,6 +48,13 @@ typedef enum casa_status {
 #define CASA_STATUS_LS_NONFINITE 16u    /* CoordLSVotingWeighted produced a non-finite R/q/p  */
 
 typedef struct casa_handle casa_handle;
+
+/*
+ * Element type of a network output read by the *_typed entry points.  Each 16-bit element is widened exactly to
+ * float32 when it is loaded and everything after the load is the float32 path, so every output (keypoints, debug
+ * intermediates, status bits, gradients) is bit-identical to the float32 call on the upcast tensor.
+ */
+typedef enum casa_dtype { CASA_FLOAT32 = 0, CASA_FLOAT16 = 1, CASA_BFLOAT16 = 2 } casa_dtype;
 
 int casa_version(void);
 const char* casa_last_error(void);
@@ -131,6 +140,17 @@ int casa_ransac_vote_seg(casa_handle* h, const casa_ransac_params* p, const floa
                          float* out_points, const casa_ransac_debug* debug, void* stream);
 
 /*
+ * casa_ransac_vote (mask_is_seg == 0) or casa_ransac_vote_seg (mask_is_seg != 0) with the mask / seg scores and the
+ * vector field in any casa_dtype, each with its own (a float32 one-hot mask with a bfloat16 field is fine).
+ * casa_ransac_vote and casa_ransac_vote_seg are the CASA_FLOAT32 case of this call.  idxs, selection and out_points
+ * keep their types.  Alignment only picks the load width: the mask's 128-bit loads need a 16-byte aligned base and
+ * (h*w*oc) % (16 / element size) == 0, the fused direction gather a vertex aligned to one (dy, dx) pair.
+ */
+int casa_ransac_vote_typed(casa_handle* h, const casa_ransac_params* p, int mask_is_seg, casa_dtype mask_dtype,
+                           const void* mask, casa_dtype vertex_dtype, const void* vertex, const int32_t* idxs,
+                           const float* selection, float* out_points, const casa_ransac_debug* debug, void* stream);
+
+/*
  * Same call with HOST buffers; returns after out_points is on the host.
  * Pinned (page-locked, device-mapped) buffers take the fast path: the mask is DMA-copied in up to 4 image
  * ranges on a copy stream while the previous range is voted on, and the vector field is NOT copied — the
@@ -169,7 +189,8 @@ int casa_host_wait(casa_handle* h, int64_t ticket);
  * casa_ls_vote and casa_ls_vote_backward accept any 4-byte-aligned float buffer for seg, direct, conf, out,
  * grad_points, grad_direct and grad_conf (e.g. a contiguous view that starts one float into an allocation, or a
  * DLPack export with a byte offset); wider vector loads are used only where the pointer allows them.  The
- * debug buffers (casa_ls_debug) need their element type's natural alignment.
+ * debug buffers (casa_ls_debug) need their element type's natural alignment.  The *_typed variants take seg,
+ * direct and conf in one casa_dtype (they are splits of one network output), each aligned to one element.
  */
 typedef struct casa_ls_params {
   int32_t b, h, w;
@@ -196,6 +217,8 @@ typedef struct casa_ls_debug {
 
 int casa_ls_vote(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
                  const float* conf, float* out_points, const casa_ls_debug* debug, void* stream);
+int casa_ls_vote_typed(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg, const void* direct,
+                       const void* conf, float* out_points, const casa_ls_debug* debug, void* stream);
 
 /*
  * Backward of CoordLSVotingWeighted w.r.t. `direct` and the confidence logits (SURVEY.md 8f-4) — what TF's
@@ -211,6 +234,10 @@ int casa_ls_vote(casa_handle* h, const casa_ls_params* p, const float* seg, cons
 int casa_ls_vote_backward(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
                           const float* conf, const float* grad_points, float* out_points, float* grad_direct,
                           float* grad_conf, void* stream);
+/* The same with seg, direct and conf in `dtype`; grad_direct and grad_conf are written as float32 all the same. */
+int casa_ls_vote_backward_typed(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg,
+                                const void* direct, const void* conf, const float* grad_points, float* out_points,
+                                float* grad_direct, float* grad_conf, void* stream);
 
 /*
  * Batched PnP on the GPU — the step right after the voting path (SURVEY.md 8f-2).  Stands in for the
@@ -293,12 +320,14 @@ int casa_join(casa_handle* h, void* stream);
  * DLPack entry point: the same vote with the tensors handed over as DLManagedTensor* (the pointer inside a "dltensor"
  * PyCapsule produced by any framework's __dlpack__: TensorFlow's tf.experimental.dlpack.to_dlpack, CuPy, JAX, PyTorch).
  * This is the drop-in's counterpart of the reference's only foreign-code seam, tf.numpy_function
- * (ransac_voting.py:513, bpnp_layers.py:322).  Device type, device id, float32 dtype, dimensions and C-contiguous
+ * (ransac_voting.py:513, bpnp_layers.py:322).  Device type, device id, dtype, dimensions and C-contiguous
  * strides are validated here, in C; b, h, w, oc, vn and vertex_per_class are taken from the tensors (the other fields of
  * `p` are used as given); `out` is a caller-allocated [b,oc,vn,2] tensor of the same device.  The three capsules are
  * CONSUMED in every case: their deleters are called exactly once — at once if the call is rejected, otherwise when the
  * GPU work queued on `stream` by this call has finished (polled at later calls on the handle, casa_sync, casa_destroy).
- * mask_is_seg != 0: `mask` holds [b,h,w,1+oc] segmentation scores (casa_ransac_vote_seg).
+ * mask_is_seg != 0: `mask` holds [b,h,w,1+oc] segmentation scores (casa_ransac_vote_seg).  `mask` and `vertex` may be
+ * float32 (DLPack code 2, 32 bits), float16 (code 2, 16 bits) or bfloat16 (code 4, 16 bits), as in
+ * casa_ransac_vote_typed; `out` is float32.
  */
 int casa_ransac_vote_dlpack(casa_handle* h, const casa_ransac_params* p, void* mask_dlm, void* vertex_dlm, void* out_dlm,
                             int mask_is_seg, void* stream);
