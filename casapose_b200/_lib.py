@@ -84,6 +84,8 @@ EXPORTS = {
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "casa_ls_vote_typed": (C.c_int, [C.c_void_p, C.POINTER(LsParams), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.POINTER(LsDebug), C.c_void_p]),
+    "casa_ls_vote_counts": (C.c_int, [C.c_void_p, C.POINTER(LsParams), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.POINTER(LsDebug), C.c_void_p]),
     "casa_ls_vote_backward_typed": (C.c_int, [C.c_void_p, C.POINTER(LsParams), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "casa_pnp": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

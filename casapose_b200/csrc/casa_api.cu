@@ -246,7 +246,8 @@ struct casa_handle {
   int score_occ = 0, score_occ_narrow = 0;  // resident k_score blocks per SM (8 / 4 hypotheses per lane)
   // per input dtype (casa_dtype): an instantiation for 16-bit inputs may differ in registers and static shared memory
   int fused_occ[3] = {0, 0, 0};   // resident k_ls_fused blocks per SM (persistent grid of the LS forward call)
-  int classify_static_smem[3][2] = {{-1, -1}, {-1, -1}, {-1, -1}};  // static shared memory of k_ls_classify<9> / <0>
+  int classify_static_smem[3][2][2] = {{{-1, -1}, {-1, -1}}, {{-1, -1}, {-1, -1}}, {{-1, -1}, {-1, -1}}};  // static shared
+                                  // memory of k_ls_classify<9> / <0>, without / with the hot_counts (COUNT) ballots
   int use_graph = 1;
   // keypoint all-gather (NCCL, resolved with dlopen: the library itself does not link against it)
   void* comm = nullptr;           // ncclComm_t
@@ -297,6 +298,8 @@ struct casa_graph {
   std::vector<cudaGraphNode_t> knodes;  // kernel nodes in list order (top level and WHILE body alike)
   cudaGraphConditionalHandle cond = 0;  // condition of the graph's WHILE node (0: the list has no loop)
   cudaGraphNode_t ev0_node = nullptr, ev1_node = nullptr, evr_node = nullptr, ctrl_node = nullptr, stats_node = nullptr;
+  cudaGraphNode_t zero_node = nullptr;  // STEP_ZERO: memset node of a caller's buffer
+  void* zero_dst = nullptr;             // address it currently clears
   std::vector<std::vector<char>> last_args;  // argument bytes each kernel node currently holds: unchanged nodes are not patched
   const void* last_slot = nullptr;           // read-back slot the event / copy nodes currently point at
 };
@@ -586,7 +589,8 @@ extern "C" size_t casa_ransac_workspace_bytes(const casa_ransac_params* p) {
 // ---- as a CUDA graph whose kernel-node parameters are patched per call (CUDA graphs instead of launch gaps).
 namespace {
 
-enum StepKind { STEP_KERNEL, STEP_EV0, STEP_EV1, STEP_READBACK, STEP_CLEAR, STEP_WHILE_BEGIN, STEP_WHILE_END };
+// STEP_ZERO: zero-fills `zero_bytes` (a multiple of 4) at `zero_dst`, a caller's buffer (at most one per list)
+enum StepKind { STEP_KERNEL, STEP_EV0, STEP_EV1, STEP_READBACK, STEP_CLEAR, STEP_WHILE_BEGIN, STEP_WHILE_END, STEP_ZERO };
 
 struct Step {
   StepKind kind = STEP_KERNEL;
@@ -598,6 +602,8 @@ struct Step {
   size_t used = 0;
   int n = 0;
   int cond_arg = -1;  // index of the argument that receives the graph's WHILE condition handle (k_update)
+  void* zero_dst = nullptr;  // STEP_ZERO
+  size_t zero_bytes = 0;
   // graph topology: 0 = main chain; 1 = opens a side branch off the main chain's last node; 2 = continues the side
   // branch.  join: this main-chain step also waits for the side branch (which ends there).
   // Two side branches can be open at a time (slot 0 and slot 1).
@@ -649,6 +655,13 @@ Step special(StepKind k, int side = 0) {
   return s;
 }
 
+Step zero_step(void* dst, size_t bytes) {
+  Step s = special(STEP_ZERO);
+  s.zero_dst = dst;
+  s.zero_bytes = bytes;
+  return s;
+}
+
 uint64_t fnv(uint64_t hsh, const void* p, size_t n) {
   const unsigned char* b = (const unsigned char*)p;
   for (size_t i = 0; i < n; ++i) hsh = (hsh ^ b[i]) * 1099511628211ull;
@@ -679,6 +692,7 @@ static int run_direct(casa_handle* h, std::vector<Step>& steps, const WS& ws, cu
         CUDA_TRY(cudaMemsetAsync(ws.ctrl, 0, CTRL_WORDS * sizeof(int), st));
         CUDA_TRY(cudaMemsetAsync(ws.stats, 0, 4 * sizeof(unsigned long long), st));
         break;
+      case STEP_ZERO: CUDA_TRY(cudaMemsetAsync(s.zero_dst, 0, s.zero_bytes, st)); break;
       case STEP_EV0: CUDA_TRY(cudaEventRecord(slot->ev0, st)); break;
       case STEP_EV1: CUDA_TRY(cudaEventRecord(slot->ev1, st)); break;
       case STEP_READBACK:
@@ -719,6 +733,7 @@ static int run_graph(casa_handle* h, std::vector<Step>& steps, const WS& ws, cud
     key = fnv(key, &s.grid, sizeof(s.grid));
     key = fnv(key, &s.block, sizeof(s.block));
     key = fnv(key, &s.smem, sizeof(s.smem));
+    if (s.kind == STEP_ZERO) key = fnv(key, &s.zero_bytes, sizeof(s.zero_bytes));
   }
   key = fnv(key, &ws.ctrl, sizeof(ws.ctrl));  // the clear / read-back nodes carry workspace addresses
   casa_graph* g = nullptr;
@@ -779,6 +794,19 @@ static int run_graph(casa_handle* h, std::vector<Step>& steps, const WS& ws, cud
           mp.height = 1;
           mp.value = 0;
           CUDA_TRY(cudaGraphAddMemsetNode(&node, cur, dep, nd, &mp));
+          break;
+        }
+        case STEP_ZERO: {
+          cudaMemsetParams mp;
+          memset(&mp, 0, sizeof(mp));
+          mp.dst = s.zero_dst;
+          mp.elementSize = 4;
+          mp.width = s.zero_bytes / 4;
+          mp.height = 1;
+          mp.value = 0;
+          CUDA_TRY(cudaGraphAddMemsetNode(&node, cur, dep, nd, &mp));
+          g->zero_node = node;
+          g->zero_dst = s.zero_dst;
           break;
         }
         case STEP_READBACK: {
@@ -842,6 +870,18 @@ static int run_graph(casa_handle* h, std::vector<Step>& steps, const WS& ws, cud
       cudaKernelNodeParams kp;
       kparams(s, args, kp);
       CUDA_TRY(cudaGraphExecKernelNodeSetParams(g->exec, g->knodes[k++], &kp));
+    }
+    for (const Step& s : steps) {
+      if (s.kind != STEP_ZERO || s.zero_dst == g->zero_dst) continue;
+      cudaMemsetParams mp;  // same size (part of the key), this call's buffer
+      memset(&mp, 0, sizeof(mp));
+      mp.dst = s.zero_dst;
+      mp.elementSize = 4;
+      mp.width = s.zero_bytes / 4;
+      mp.height = 1;
+      mp.value = 0;
+      CUDA_TRY(cudaGraphExecMemsetNodeSetParams(g->exec, g->zero_node, &mp));
+      g->zero_dst = s.zero_dst;
     }
     if (slot && g->last_slot != (const void*)slot) {  // this call's read-back slot
       g->last_slot = slot;
@@ -1723,7 +1763,23 @@ struct LsGrad {
   float* grad_conf = nullptr;          // [b,h,w,vn]
 };
 int ls_vote_impl(casa_handle* h, const casa_ls_params* p, casa_dtype dt, const void* seg, const void* direct, const void* conf,
-                 float* out_points, const casa_ls_debug* debug, void* stream, const LsGrad* grad, int pix_capacity = 0);
+                 float* out_points, const casa_ls_debug* debug, void* stream, const LsGrad* grad, int32_t* hot_counts,
+                 int pix_capacity = 0);
+
+int ls_vote_entry(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg, const void* direct,
+                  const void* conf, float* out_points, int32_t* hot_counts, const casa_ls_debug* debug, void* stream) {
+  if (h->async_mode >= 2 && !debug && !p->check_finite && !h->is_lane) {  // lanes, as for the votes (check_finite waits for the host)
+    casa_handle* sub = nullptr;
+    int k = 0;
+    int rcl = lane_begin(h, h->async_mode, stream, &sub, &k);
+    if (rcl) return rcl;
+    rcl = ls_vote_impl(sub, p, dtype, seg, direct, conf, out_points, nullptr, (void*)sub->own_stream, nullptr, hot_counts);
+    const int rce = lane_end(h, k, stream);
+    h->last_launches = sub->last_launches;
+    return rcl ? rcl : rce;
+  }
+  return ls_vote_impl(h, p, dtype, seg, direct, conf, out_points, debug, stream, nullptr, hot_counts);
+}
 }  // namespace
 
 extern "C" int casa_ls_vote_typed(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg, const void* direct,
@@ -1731,17 +1787,18 @@ extern "C" int casa_ls_vote_typed(casa_handle* h, const casa_ls_params* p, casa_
   if (!h || !p) return fail(CASA_ERR_INVALID, "handle / params is NULL");
   if (!dtype_ok(dtype)) return fail(CASA_ERR_INVALID, "dtype %d is not a casa_dtype", (int)dtype);
   if (!seg || !direct || !conf || !out_points) return fail(CASA_ERR_INVALID, "seg / direct / conf / out_points must not be NULL");
-  if (h->async_mode >= 2 && !debug && !p->check_finite && !h->is_lane) {  // lanes, as for the votes (check_finite waits for the host)
-    casa_handle* sub = nullptr;
-    int k = 0;
-    int rcl = lane_begin(h, h->async_mode, stream, &sub, &k);
-    if (rcl) return rcl;
-    rcl = ls_vote_impl(sub, p, dtype, seg, direct, conf, out_points, nullptr, (void*)sub->own_stream, nullptr);
-    const int rce = lane_end(h, k, stream);
-    h->last_launches = sub->last_launches;
-    return rcl ? rcl : rce;
-  }
-  return ls_vote_impl(h, p, dtype, seg, direct, conf, out_points, debug, stream, nullptr);
+  return ls_vote_entry(h, p, dtype, seg, direct, conf, out_points, nullptr, debug, stream);
+}
+
+extern "C" int casa_ls_vote_counts(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg, const void* direct,
+                                   const void* conf, float* out_points, int32_t* hot_counts, const casa_ls_debug* debug,
+                                   void* stream) {
+  if (!h || !p) return fail(CASA_ERR_INVALID, "handle / params is NULL");
+  if (!dtype_ok(dtype)) return fail(CASA_ERR_INVALID, "dtype %d is not a casa_dtype", (int)dtype);
+  if (!seg || !direct || !conf || !out_points || !hot_counts)
+    return fail(CASA_ERR_INVALID, "seg / direct / conf / out_points / hot_counts must not be NULL");
+  if (((uintptr_t)hot_counts & 3) != 0) return fail(CASA_ERR_INVALID, "hot_counts must be 4-byte aligned");
+  return ls_vote_entry(h, p, dtype, seg, direct, conf, out_points, hot_counts, debug, stream);
 }
 
 extern "C" int casa_ls_vote(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
@@ -1760,7 +1817,7 @@ extern "C" int casa_ls_vote_backward_typed(casa_handle* h, const casa_ls_params*
   g.grad_points = grad_points;
   g.grad_direct = grad_direct;
   g.grad_conf = grad_conf;
-  return ls_vote_impl(h, p, dtype, seg, direct, conf, out_points, nullptr, stream, &g);
+  return ls_vote_impl(h, p, dtype, seg, direct, conf, out_points, nullptr, stream, &g, nullptr);
 }
 
 extern "C" int casa_ls_vote_backward(casa_handle* h, const casa_ls_params* p, const float* seg, const float* direct,
@@ -1772,8 +1829,10 @@ extern "C" int casa_ls_vote_backward(casa_handle* h, const casa_ls_params* p, co
 
 namespace {
 // dt: element type of seg, direct and conf (the input-reading kernels are instantiated per type; the rest is float32)
+// hot_counts (casa_ls_vote_counts) or NULL: k_ls_classify's COUNT instantiation, behind a memset of the counts
 int ls_vote_impl(casa_handle* h, const casa_ls_params* p, casa_dtype dt, const void* seg, const void* direct, const void* conf,
-                 float* out_points, const casa_ls_debug* debug, void* stream, const LsGrad* grad, int pix_capacity) {
+                 float* out_points, const casa_ls_debug* debug, void* stream, const LsGrad* grad, int32_t* hot_counts,
+                 int pix_capacity) {
   if (p->num_classes < 2 || p->num_classes > 33) return fail(CASA_ERR_INVALID, "num_classes=%d outside 2..33", p->num_classes);
   casa_ransac_params rp;
   memset(&rp, 0, sizeof(rp));
@@ -1841,20 +1900,25 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, casa_dtype dt, const v
   std::vector<Step> steps;
   steps.reserve(16);
   steps.push_back(special(STEP_CLEAR));  // ctrl / stats: one memset node in front of the kernels
+  if (hot_counts) steps.push_back(zero_step(hot_counts, (size_t)d.J * sizeof(int32_t)));
   {
     const size_t sm = (size_t)kCountTile * ld.nc * 4;
-    const void* classify = ld.nc == 9 ? by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<9, typename decltype(e)::type>; })
-                                      : by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<0, typename decltype(e)::type>; });
+    const void* classify =
+        hot_counts ? (ld.nc == 9 ? by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<9, typename decltype(e)::type, true>; })
+                                 : by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<0, typename decltype(e)::type, true>; }))
+                   : (ld.nc == 9 ? by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<9, typename decltype(e)::type, false>; })
+                                 : by_dtype(dt, [](auto e) { return (const void*)k_ls_classify<0, typename decltype(e)::type, false>; }));
     // Without the opt-in, static plus dynamic shared memory of a block may not exceed 48 KB: the kernel's own counters
     // (scnt) count too, so nc = 12 (exactly 48 KB of staged logits) needs the attribute as well.
-    int& static_sm = h->classify_static_smem[dt][ld.nc == 9 ? 0 : 1];
+    int& static_sm = h->classify_static_smem[dt][ld.nc == 9 ? 0 : 1][hot_counts ? 1 : 0];
     if (static_sm < 0) {
       cudaFuncAttributes fa;
       CUDA_TRY(cudaFuncGetAttributes(&fa, classify));
       static_sm = (int)fa.sharedSizeBytes;
     }
     if (sm + (size_t)static_sm > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(classify, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    steps.push_back(kstep(classify, dim3(d.nct, d.b), 256, sm).arg(seg).arg(ws).arg(d).arg(lw).arg(ld).arg((int)(runs_cc ? 1 : 0)));
+    steps.push_back(kstep(classify, dim3(d.nct, d.b), 256, sm).arg(seg).arg(ws).arg(d).arg(lw).arg(ld).arg((int)(runs_cc ? 1 : 0))
+                        .arg((int*)hot_counts));
   }
   steps.push_back(kstep((const void*)k_place<0, float>, dim3((d.nct + kPlaceSub - 1) / kPlaceSub, d.b), 256).arg((const float*)nullptr).arg(ws).arg(d).arg((int)0));
   // topology: the work-item / tile plan only needs the job table and runs beside the component chain (side branch)
@@ -1930,7 +1994,8 @@ int ls_vote_impl(casa_handle* h, const casa_ls_params* p, casa_dtype dt, const v
       CUDA_TRY(cudaMemset(h->sticky, 0, sizeof(uint32_t)));  // the retried call reports for itself
       if (need <= d.cap || need > (1ll << 30))
         return fail(CASA_ERR_WORKSPACE, "CoordLSVotingWeighted: pixel lists overflow (need %lld slots per image)", need);
-      return ls_vote_impl(h, p, dt, seg, direct, conf, out_points == (float*)(base + off_tmp_out) ? nullptr : out_points, debug, stream, grad, (int)need);
+      return ls_vote_impl(h, p, dt, seg, direct, conf, out_points == (float*)(base + off_tmp_out) ? nullptr : out_points, debug, stream, grad,
+                          hot_counts, (int)need);
     }
     if (p->check_finite && (h->last_status & CASA_STATUS_LS_NONFINITE))
       return fail(CASA_ERR_INPUT, "CoordLSVotingWeighted: non-finite R / q / p (the reference asserts here, voting_layers_2d.py:109-121)");

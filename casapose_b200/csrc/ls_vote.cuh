@@ -106,6 +106,9 @@ __device__ __forceinline__ float hot_of_row(const float* row, int nc, int cls) {
 // T: element type of `seg`, widened to float while it is staged (128-bit loads when the slab is 16-byte aligned).
 // flag_onehot (forward call): cls9 bit 7 marks pixels whose softmax is exactly one-hot, so that the reduction need not
 // read their logits again.
+// COUNT: also counts, per image and class c >= 1, the pixels with hot > 0.1f into hot_counts[b][oc] (zeroed by the
+// caller) — poses_pnp's object availability (/root/reference/casapose/pose_estimation/pose_evaluation.py:183-190).
+// Instantiations without it never touch hot_counts and compile to the kernel as it was before the flag.
 extern __shared__ __align__(16) float ls_smem[];
 // 16 bytes of T, widened, into the float tile at vector index i (4 floats, or 8 values of a 16-bit type)
 __device__ __forceinline__ void stage16(float4* sm4, int i, const uint4& v, const float*) {
@@ -117,14 +120,15 @@ __device__ __forceinline__ void stage16(float4* sm4, int i, const uint4& v, cons
   sm4[2 * i + 1] = make_float4(vec_elem(v, 4, t), vec_elem(v, 5, t), vec_elem(v, 6, t), vec_elem(v, 7, t));
 }
 
-template <int NC, typename T>
-__global__ void __launch_bounds__(256) k_ls_classify(const T* __restrict__ seg, WS ws, Dims d, LsWS lw, LsDims ld, int flag_onehot) {
+template <int NC, typename T, bool COUNT>
+__global__ void __launch_bounds__(256) k_ls_classify(const T* __restrict__ seg, WS ws, Dims d, LsWS lw, LsDims ld, int flag_onehot,
+                                                     int* __restrict__ hot_counts) {
   constexpr int kPerVec = 16 / sizeof(T);  // elements per 128-bit load
   const int img = blockIdx.y, tile = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31;
   const int nc = NC ? NC : ld.nc;
-  __shared__ int scnt[32];
-  if (tid < 32) scnt[tid] = 0;
+  __shared__ int scnt[COUNT ? 64 : 32];  // [0, 32): hot != 0 per class; [32, 64): hot > 0.1f (COUNT)
+  if (tid < (COUNT ? 64 : 32)) scnt[tid] = 0;
   const int p0 = tile * kCountTile;
   const int npx = min(kCountTile, d.hw - p0);
   const T* slab = seg + ((size_t)img * d.hw + p0) * nc;
@@ -156,7 +160,7 @@ __global__ void __launch_bounds__(256) k_ls_classify(const T* __restrict__ seg, 
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
     const int q = k * 256 + tid;
-    uint32_t m = 0;
+    uint32_t m = 0, m1 = 0;  // m1 (COUNT): classes with hot > 0.1f, a subset of m
     if (q < npx) {
       const float* row = ls_smem + q * nc;
       float mx = -3.4e38f, m2 = -3.4e38f;
@@ -176,6 +180,7 @@ __global__ void __launch_bounds__(256) k_ls_classify(const T* __restrict__ seg, 
       if (mx - m2 > 110.f) {  // exactly one-hot
         if (arg > 0) {
           m = 1u << (arg - 1);
+          if (COUNT) m1 = m;  // hot = 1 for the arg class
           c9 = arg | (flag_onehot ? kOneHotFlag : 0);
         }
       } else {
@@ -184,6 +189,7 @@ __global__ void __launch_bounds__(256) k_ls_classify(const T* __restrict__ seg, 
         for (int c = 1; c < nc; ++c) {
           const float hv = __fdiv_rn(expf(__fsub_rn(__fmul_rn(row[c], 1.0e6f), mx)), sum);
           m |= (uint32_t)(hv != 0.f) << (c - 1);
+          if (COUNT) m1 |= (uint32_t)(hv > 0.1f) << (c - 1);  // pose_evaluation.py:186
           if ((int)__fadd_rn(hv, 0.1f) == 1) c9 = c;  // :44 (at most one class can reach 0.9)
         }
       }
@@ -191,14 +197,21 @@ __global__ void __launch_bounds__(256) k_ls_classify(const T* __restrict__ seg, 
       lw.cls9[(size_t)img * d.hw + p0 + q] = (unsigned char)c9;
     }
     if (__any_sync(0xffffffffu, m != 0u)) {
+      // m1 differs from m only at near-tie pixels: elsewhere its ballots are m's
+      const bool same = COUNT ? __all_sync(0xffffffffu, m1 == m) : true;
       for (int c = 0; c < d.oc; ++c) {
         const unsigned bal = __ballot_sync(0xffffffffu, (m >> c) & 1u);
         if (lane == 0 && bal) atomicAdd(&scnt[c], __popc(bal));
+        if (COUNT) {
+          const unsigned bal1 = same ? bal : __ballot_sync(0xffffffffu, (m1 >> c) & 1u);
+          if (lane == 0 && bal1) atomicAdd(&scnt[32 + c], __popc(bal1));
+        }
       }
     }
   }
   __syncthreads();
   if (tid < d.oc) ws.tile_cnt[((size_t)img * d.oc + tid) * d.nct + tile] = scnt[tid];
+  if (COUNT && tid < d.oc && scnt[32 + tid]) atomicAdd(&hot_counts[(size_t)img * d.oc + tid], scnt[32 + tid]);
 }
 
 // ---------------------------------------------------------------------------------- connected components

@@ -15,7 +15,11 @@ grad_out)`, or transparently through torch.autograd when `direct` / `w` are torc
 seg, direct and w may be float32, float16 or bfloat16 (one dtype for all three: they are splits of one network
 output).  16-bit inputs are read natively and widened exactly, so outputs equal the call on the .float() tensors.
 `layer.backward` returns float32 gradients for every input dtype; through autograd a 16-bit leaf receives its
-gradient in its own dtype (the float32 gradient rounded once)."""
+gradient in its own dtype (the float32 gradient rounded once).
+
+`layer(inp, return_counts=True)` also returns poses_pnp's object availability counts from the same pass over `seg`
+(casa_ls_vote_counts): [b, num_classes-1] int32 on the device, the pixels whose softmax(1e6 seg) exceeds 0.1
+(/root/reference/casapose/pose_estimation/pose_evaluation.py:183-188)."""
 import ctypes as C
 
 import torch
@@ -28,16 +32,19 @@ class _LsVoteFn(torch.autograd.Function):
     """torch.autograd carrier of casa_ls_vote / casa_ls_vote_backward (PyTorch only routes the gradient)."""
 
     @staticmethod
-    def forward(ctx, layer, seg, direct, w):
+    def forward(ctx, layer, seg, direct, w, return_counts=False, check_finite=True):
         ctx.layer = layer
         ctx.save_for_backward(seg, direct, w)
-        return layer._forward(seg, direct, w, False, True)
+        res = layer._forward(seg, direct, w, False, check_finite, return_counts)
+        if return_counts:
+            ctx.mark_non_differentiable(res[1])
+        return res
 
     @staticmethod
-    def backward(ctx, grad_out):
+    def backward(ctx, grad_out, *grad_counts):
         seg, direct, w = ctx.saved_tensors
         gd, gw = ctx.layer.backward([seg, direct, w], grad_out)
-        return None, None, gd.reshape(direct.shape).to(direct.dtype), gw.to(w.dtype)
+        return None, None, gd.reshape(direct.shape).to(direct.dtype), gw.to(w.dtype), None, None
 
 
 class CoordLSVotingWeighted:
@@ -60,11 +67,13 @@ class CoordLSVotingWeighted:
     def __call__(self, inp, **kwargs):
         return self.call(inp, **kwargs)
 
-    def call(self, inp, return_debug=False, check_finite=True, **kwargs):
+    def call(self, inp, return_debug=False, check_finite=True, *, return_counts=False, **kwargs):
+        """coords [b, oc, vn, 2]; with return_counts (coords, counts [b, oc] int32); with return_debug the debug dict
+        comes last.  On the autograd path the counts are a non-differentiable output."""
         seg, direct, w = inp
         if not return_debug and torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (direct, w)):
-            return _LsVoteFn.apply(self, seg.detach() if isinstance(seg, torch.Tensor) else seg, direct, w)
-        return self._forward(seg, direct, w, return_debug, check_finite)
+            return _LsVoteFn.apply(self, seg.detach() if isinstance(seg, torch.Tensor) else seg, direct, w, return_counts)
+        return self._forward(seg, direct, w, return_debug, check_finite, return_counts)
 
     def _prepare(self, seg, direct, w):
         seg, dt = as_cuda_float(seg, "seg")
@@ -110,10 +119,11 @@ class CoordLSVotingWeighted:
         _lib.check(rc)
         return gd, gw
 
-    def _forward(self, seg, direct, w, return_debug, check_finite):
+    def _forward(self, seg, direct, w, return_debug, check_finite, return_counts=False):
         seg, direct, w, (b, h, wd, nc, vn), dt = self._prepare(seg, direct, w)
         dev = seg.device
         out = torch.empty((b, nc - 1, vn, 2), dtype=torch.float32, device=dev)
+        counts = torch.empty((b, nc - 1), dtype=torch.int32, device=dev) if return_counts else None
         p = self._params(b, h, wd, nc, vn, check_finite)
         dbg = None
         dbg_struct = None
@@ -127,8 +137,14 @@ class CoordLSVotingWeighted:
             }
             dbg_struct = _lib.LsDebug(**{k: ptr(v) for k, v in dbg.items()})
         hdl = _lib.handle(dev.index if dev.index is not None else torch.cuda.current_device(), current_stream_ptr(dev))
+        dbg_arg = C.byref(dbg_struct) if dbg_struct is not None else None
         with torch.cuda.device(dev):
-            rc = _lib.lib().casa_ls_vote_typed(hdl, C.byref(p), dt, ptr(seg), ptr(direct), ptr(w), ptr(out),
-                                               C.byref(dbg_struct) if dbg_struct is not None else None, current_stream_ptr(dev))
+            if return_counts:
+                rc = _lib.lib().casa_ls_vote_counts(hdl, C.byref(p), dt, ptr(seg), ptr(direct), ptr(w), ptr(out), ptr(counts),
+                                                    dbg_arg, current_stream_ptr(dev))
+            else:
+                rc = _lib.lib().casa_ls_vote_typed(hdl, C.byref(p), dt, ptr(seg), ptr(direct), ptr(w), ptr(out), dbg_arg,
+                                                   current_stream_ptr(dev))
         _lib.check(rc)
-        return (out, dbg) if return_debug else out
+        res = (out,) + ((counts,) if return_counts else ()) + ((dbg,) if return_debug else ())
+        return res if len(res) > 1 else out

@@ -219,6 +219,16 @@ int casa_ls_vote(casa_handle* h, const casa_ls_params* p, const float* seg, cons
                  const float* conf, float* out_points, const casa_ls_debug* debug, void* stream);
 int casa_ls_vote_typed(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg, const void* direct,
                        const void* conf, float* out_points, const casa_ls_debug* debug, void* stream);
+/*
+ * casa_ls_vote_typed, and the object availability count of poses_pnp taken from the same softmax
+ * (/root/reference/casapose/pose_estimation/pose_evaluation.py:183-190):
+ *   hot_counts  device int32 [b,num_classes-1]  pixels with softmax(1e6 seg)[..., c] > 0.1 (float32), c >= 1
+ * must not be NULL.  out_points and the debug outputs are those of casa_ls_vote_typed, bit for bit.
+ * hot_counts is zeroed and written inside the call, ordered like out_points: on `stream`, or on the lanes of
+ * casa_set_async(h, n), after casa_join / casa_sync.
+ */
+int casa_ls_vote_counts(casa_handle* h, const casa_ls_params* p, casa_dtype dtype, const void* seg, const void* direct,
+                        const void* conf, float* out_points, int32_t* hot_counts, const casa_ls_debug* debug, void* stream);
 
 /*
  * Backward of CoordLSVotingWeighted w.r.t. `direct` and the confidence logits (SURVEY.md 8f-4) — what TF's
